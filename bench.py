@@ -20,6 +20,7 @@ N=10 on the lane-group K1 (the top of north_star's "n <= 8" range), 2e6 samples 
   python bench.py --impl reference ...                         the CPU arm: the numpy oracle port on all host cores
   python bench.py --workload cfg-synth-32-8-30|cfg-sweep-f|probe-8-2-10   one of the others as the headline line
   python bench.py --scaling strong                             configs[3] with 1e8 samples in total as the headline line
+  python bench.py --dump-outputs DIR ...                       also write the headline's last timed step to DIR/*.npy
 
 One JSON line on stdout (rank 0).
 """
@@ -56,6 +57,10 @@ PIPE_ACTIVE_NCU = {"cfg-synth-4-2-10": ("profiles/r02f_k1_eval_4x2_metrics.csv",
 
 
 POWER_WARM_S = 0.75          # see measure_synth step (0)
+# --dump-outputs: per-sample tables are written at a fixed, seeded subset of at most DUMP_SAMPLES samples, fewer when
+# their H horizons would not fit DUMP_TABLE_BYTES (the rest of a dump is a few KB of statistics, so the whole stays under
+# 64 MB); the headline workload (12.5e6 samples, H = 1) dumps ~20 MB, and two builds stay comparable sample for sample
+DUMP_SAMPLES, DUMP_SEED, DUMP_TABLE_BYTES = 1 << 19, 7, 48 << 20
 
 
 def flops_per_eval(n, m, N, lyap_iters=8):
@@ -220,6 +225,29 @@ def _json_field(rel, key):
         return json.load(open(os.path.join(ROOT, rel))).get(key)
     except (OSError, ValueError):
         return None
+
+
+def step_outputs(r, moments, first):
+    """What one K1 / K4 step hands its caller, as host arrays: the J / rho / ratio / flags tables [H][S] at a fixed,
+    seeded subset of the shard's samples (all of them when they fit, see DUMP_SAMPLES), the global indices of those
+    samples, and the per-shard column moments [world][cols][6]."""
+    import numpy as np
+    import torch
+    H, S = r["J"].shape
+    k = min(DUMP_SAMPLES, DUMP_TABLE_BYTES // (8 * (4 * H + 1)))      # 4 tables of H rows + the index, float64
+    idx = np.arange(S) if S <= k else np.sort(np.random.default_rng(DUMP_SEED).choice(S, k, replace=False))
+    sel = torch.from_numpy(idx).to(r["J"].device)
+    out = {k: r[k].index_select(1, sel).cpu().numpy() for k in ("J", "rho", "ratio", "flags")}
+    out.update(sample_index=first + idx, moments=moments.cpu().numpy())
+    return out
+
+
+def dump_outputs(path, arrays):
+    """DIR/<name>.npy for every array, in float64 (flags and indices are exact in it)."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), np.asarray(v, dtype=np.float64))
 
 
 def workload_config(wl, n_gpus, scaling="weak"):
@@ -422,9 +450,10 @@ def link_ceiling(cx, h_in, d_in, d_out_bytes, steps=3):
                     "all %d ranks concurrently, no kernels" % cx.world}
 
 
-def measure_synth(cx, wl, steps, warmup, scaling="weak", full=True):
+def measure_synth(cx, wl, steps, warmup, scaling="weak", full=True, outputs=None):
     """One synthetic workload (K1 or K4): device-resident value, kernel-alone roofline, end-to-end through the host-buffer
-    entry point. `full=False` (sub-records) skips the nested-horizon and link-ceiling legs."""
+    entry point. `full=False` (sub-records) skips the nested-horizon and link-ceiling legs. A dict `outputs` receives
+    step_outputs() of the last timed step."""
     import numpy as np
     torch, dist, eng = cx.torch, cx.dist, cx.eng
     from lq_mpc_b200 import sampling as sp
@@ -510,6 +539,8 @@ def measure_synth(cx, wl, steps, warmup, scaling="weak", full=True):
                                 "between launches: full clocks, no throttle reason, every single launch at its "
                                 "median duration)", "first_attempt": first}
     stats = merge_moments(st.cpu().numpy())
+    if outputs is not None:
+        outputs.update(step_outputs(r, st, rank * S))
     # ---- (2b) supplementary: every horizon 1..N from ONE nested Riccati recursion per sample (K1 only)
     ms_nested = None
     if full and not tiled:
@@ -617,9 +648,10 @@ def measure_synth(cx, wl, steps, warmup, scaling="weak", full=True):
     return rec
 
 
-def measure_strong(cx, steps):
+def measure_strong(cx, steps, outputs=None):
     """BASELINE configs[3] as written: 1e8 samples in TOTAL, sharded over the ranks (strong scaling). Inputs are drawn
-    on the device (seeded torch generator, U[-0.01, 0.01] / N(0, I)): this leg times the device-resident path only."""
+    on the device (seeded torch generator, U[-0.01, 0.01] / N(0, I)): this leg times the device-resident path only.
+    A dict `outputs` receives step_outputs() of the last timed step."""
     torch, eng = cx.torch, cx.eng
     from lq_mpc_b200 import sampling as sp
     from lq_mpc_b200.stats import column_moments_device
@@ -638,8 +670,10 @@ def measure_strong(cx, steps):
         return r, column_moments_device(eng, r["table"])
     for _ in range(3):
         step()
-    ms, _ = cx.timed(step, steps)
-    del dA, dB, x0
+    ms, (r, mom) = cx.timed(step, steps)
+    if outputs is not None:
+        outputs.update(step_outputs(r, mom, cx.rank * S))
+    del dA, dB, x0, r
     torch.cuda.empty_cache()
     if cx.rank != 0:
         return None
@@ -649,9 +683,10 @@ def measure_strong(cx, steps):
             "config": workload_config(dict(wl, S=S), cx.world, "strong")}
 
 
-def measure_sweep(cx, wl, reps=1):
+def measure_sweep(cx, wl, reps=1, outputs=None):
     """cfg-sweep (BASELINE configs[2]): error-level x horizon grid on the 2-state example with the input box active.
-    One 'step' = the whole sweep (n_err x nmax cells, per_level perturbations each) on device-resident grids."""
+    One 'step' = the whole sweep (n_err x nmax cells, per_level perturbations each) on device-resident grids. A dict
+    `outputs` receives every array and scalar of the last sweep's result except its timings."""
     import numpy as np
     torch, eng = cx.torch, cx.eng
     from lq_mpc_b200 import sampling as sp
@@ -674,16 +709,17 @@ def measure_sweep(cx, wl, reps=1):
     error_horizon_sweep(eng, wA, wB, error_vec, [1, 7, wl["nmax"]], F_u, Q)                  # warm-up (3 horizons)
     error_horizon_sweep(eng, eA, eB, error_vec, [wl["nmax"]], F_u, Q)
     launches0 = eng.launch_count
-    best = None
+    secs, phases = [], []
     for _ in range(reps):
         cx.barrier()
         r = error_horizon_sweep(eng, eA, eB, error_vec, horizons, F_u, Q, phase_times=True)
-        sec = cx.max_over_ranks(r["seconds"])
-        if best is None or sec < best[0]:
-            best = (sec, r)
+        secs.append(cx.max_over_ranks(r["seconds"]))
+        phases.append(r["phase_seconds"])
+    if outputs is not None:
+        outputs.update({k: v for k, v in r.items() if k not in ("seconds", "wall_seconds", "phase_seconds")})
     launches = eng.launch_count - launches0
     clocks = cx.sampler.take()
-    sec, r = best
+    sec = sum(secs) / reps                      # every timed sweep counts, as the timed steps of the K1 / K4 legs do
     del eA, eB
     torch.cuda.empty_cache()
     if cx.rank != 0:
@@ -691,7 +727,7 @@ def measure_sweep(cx, wl, reps=1):
     evals_gpu = wl["per_level"] * wl["n_err"] * len(horizons)
     evals = evals_gpu * cx.world
     n_void = float(r["n_invalid"].sum())
-    ph = r["phase_seconds"]
+    ph = {k: sum(p[k] for p in phases) / reps for k in phases[0]}
     peak_fp64, peak_dmma = cx.fp64_peaks()
     peak = max(peak_fp64, peak_dmma)
     k3_flops = sum(k3_flops_per_eval(2, 1, N) for N in horizons) * wl["per_level"] * wl["n_err"]
@@ -699,6 +735,8 @@ def measure_sweep(cx, wl, reps=1):
     return {
         "metric": "mpc_evals_per_sec", "value": evals / sec, "unit": "evals/s", "n_gpus": cx.world, "steps": reps,
         "warmup": 2, "ms_per_step": sec * 1e3, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
+        "sweep_seconds": {"mean": sec, "min": min(secs), "max": max(secs), "sweeps": reps,
+                          "what": "value, ms_per_step and phase_seconds are means over the timed sweeps"},
         "dtype": "f64", "data": "synthetic (K6 device sampler, Philox4x32-10, seed 20240522)",
         "config": workload_config(wl, cx.world),
         "evals": evals, "evals_valid_bound": evals - n_void, "evals_void_bound": n_void,
@@ -738,14 +776,15 @@ def run_ours(args, wl):
     gc.disable()             # 100 ms host stall; it must not fall between two launches of a timed region
     steps = args.steps
     line = None
+    outputs = {} if args.dump_outputs else None
     if wl.get("sweep"):
-        line = measure_sweep(cx, wl, reps=max(1, min(3, steps)))
+        line = measure_sweep(cx, wl, reps=steps, outputs=outputs)
     elif args.scaling == "strong":
-        line = measure_strong(cx, steps)
+        line = measure_strong(cx, steps, outputs=outputs)
         if line is not None:
             line.update({"metric": "mpc_evals_per_sec", "higher_is_better": True, "vs_baseline": None, "dtype": "f64"})
     else:
-        line = measure_synth(cx, wl, steps, args.warmup, full=True)
+        line = measure_synth(cx, wl, steps, args.warmup, full=True, outputs=outputs)
     subs = {}
     if args.workload == "cfg-synth-4-2-10" and args.scaling == "weak" and not args.headline_only:
         strong = measure_strong(cx, max(3, min(10, steps)))
@@ -771,6 +810,8 @@ def run_ours(args, wl):
                 subs["cfg-synth-32-8-30"]["cpu_baseline"] = _synth_cpu_record(k4, 8_000)
             if "cfg-sweep-f" in subs:
                 subs["cfg-sweep-f"]["cpu_baseline"] = _sweep_cpu_record()
+        if outputs is not None:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(line))
     if cx.world > 1:
         cx.dist.barrier()
@@ -804,7 +845,13 @@ def main():
     ap.add_argument("--headline-only", action="store_true", help="skip the strong-scaling / cfg-5 / cfg-sweep sub-records")
     ap.add_argument("--scaling", default="weak", choices=["weak", "strong"])
     ap.add_argument("--workload", default="cfg-synth-4-2-10", choices=sorted(WORKLOADS))
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the headline's last timed step computed as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's outputs; the CPU arm has none to write")
     wl = dict(WORKLOADS[args.workload], name=args.workload)
     if args.impl == "reference":
         return run_reference(args, wl)
