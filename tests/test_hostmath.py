@@ -13,6 +13,8 @@ from tests.conftest import relerr
 
 hm = pytest.importorskip("tests.hostmath.api")
 TOL = 1e-9
+# every (n, m) the engine instantiates its templates for (LQ_FOR_EACH_DIM in lq_mpc_b200/csrc/engine.h)
+COMPILED_DIMS = [(1, 1), (2, 1), (2, 2), (3, 1), (3, 2), (3, 3), (4, 1), (4, 2), (4, 4), (6, 2), (8, 2)]
 
 
 @pytest.mark.parametrize("n", [1, 2, 3, 4, 6, 8])
@@ -394,3 +396,60 @@ def test_k2_math_long_horizon_late_saturation_vs_dense_qp():
         x = A @ x + B @ u
         J += float(x @ Q @ x + u @ R @ u)
     assert abs(sim["J_T"][0] - J) < TOL * J
+
+
+def _scale_to_saturation(Ah, Bh, Q, R, N, lo, hi, X, t):
+    """Columns of X rescaled so that the unconstrained plan of model s from column s peaks at t[s] times the input box:
+    t > 1 makes the box active, t < 1 leaves the plan feasible (the plan is linear in the initial state)."""
+    out = X.copy()
+    for s in range(X.shape[1]):
+        K, _ = o.riccati(Ah[s], Bh[s], Q, R, Q, N)
+        x, r = X[:, s], 0.0
+        for k in range(N):
+            u = K[k] @ x
+            r = max(r, float(np.max(np.maximum(u / hi, u / lo))))
+            x = Ah[s] @ x + Bh[s] @ u
+        out[:, s] *= t[s] / r
+    return out
+
+
+@pytest.mark.parametrize("n,m", COMPILED_DIMS)
+def test_k2_math_every_compiled_pair_vs_dense_qp(n, m):
+    """Box solve and closed loop of every compiled (n, m) — (1, 1), (3, 3) and (4, 4) included, the last two being the
+    n <= 4 pairs that re-read the stage-0 gain from scratch on the certificate path — vs the dense Cholesky + BVLS
+    oracle: a short horizon (the whole cost-to-go stored) and a long one (20..40 stages) with general SPD weights, model
+    != plant, most initial states saturating and some not; the closed loop runs until the certificate takes over."""
+    rng = np.random.default_rng(40 + 10 * n + m)
+    S, T = 6, 30
+    for N, general in ((int(rng.integers(3, 12)), False), (int(rng.integers(20, min(40, 256 // m) + 1)), True)):
+        A = rng.normal(size=(n, n)); A *= rng.uniform(0.6, 1.0) / np.max(np.abs(np.linalg.eigvals(A)))
+        B = rng.normal(size=(n, m))
+        if general:
+            Mq, Mr = rng.normal(size=(n, n)), rng.normal(size=(m, m))
+            Q, R = Mq @ Mq.T / n + 0.5 * np.eye(n), Mr @ Mr.T / m + 0.3 * np.eye(m)
+        else:
+            Q, R = rng.uniform(0.5, 3) * np.eye(n), rng.uniform(0.1, 2) * np.eye(m)
+        lo, hi = -rng.uniform(0.05, 0.4, size=m), rng.uniform(0.05, 0.4, size=m)
+        dA = rng.uniform(-0.01, 0.01, size=(n * n, S)); dB = rng.uniform(-0.01, 0.01, size=(n * m, S))
+        Ah = [A + dA[:, s].reshape(n, n) for s in range(S)]
+        Bh = [B + dB[:, s].reshape(n, m) for s in range(S)]
+        t = np.r_[rng.uniform(0.2, 0.8, 2), rng.uniform(1.2, 3.0, S - 2)]
+        x0 = _scale_to_saturation(Ah, Bh, Q, R, N, lo, hi, rng.normal(size=(n, S)), t)
+        sol = hm.mpc(0, A, B, Q, R, Q, lo, hi, dA, dB, N, x0_soa=x0)
+        sim = hm.mpc(1, A, B, Q, R, Q, lo, hi, dA, dB, N, T=T, x0_soa=x0)
+        assert not np.any(sol["flags"] & ~2) and not np.any(sim["flags"] & ~2)
+        certified = 0
+        for s in range(S):
+            ur, Vr, act = o.mpc_solve(N, Ah[s], Bh[s], Q, R, Q, lo, hi, x0[:, s])
+            assert act == (t[s] > 1) and bool(sol["flags"][0, s] & 2) == act, (n, m, N, s)
+            if not act:
+                ur, Vr, _ = o.mpc_solve(N, Ah[s], Bh[s], Q, R, Q, lo, hi, x0[:, s], exact_fast=False)
+            assert abs(sol["V"][0, s] - Vr) < TOL * abs(Vr), (n, m, N, s)
+            assert np.max(np.abs(sol["u0"][0, :, s] - ur)) < TOL, (n, m, N, s)
+            so = o.simulate(T, N, Ah[s], Bh[s], Q, R, Q, lo, hi, x0[:, s], A, B)
+            assert abs(sim["J_T"][s] - so["J_T"]) < TOL * so["J_T"], (n, m, N, s)
+            assert np.max(np.abs(sim["U"][:, :, s].T - so["U"])) < TOL, (n, m, N, s)
+            assert np.max(np.abs(sim["X"][:, :, s].T - so["X"])) < TOL * max(1.0, np.max(np.abs(so["X"])))
+            assert sim["n_active"][s] == so["n_active"], (n, m, N, s)
+            certified += int(so["n_active"] < T - 5)
+        assert certified >= S // 2, (n, m, N)          # the later steps of most closed loops are unconstrained
