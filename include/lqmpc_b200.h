@@ -186,6 +186,38 @@ int lqmpc_bounds_batch(lqmpc_ctx* ctx, int64_t S, const double* dA, const double
                        int strict_reference, double* alpha, double* beta, double* xi, double* eta, double* bound,
                        double* detail, double* K_out, double* P_out, int32_t* flags);
 
+/* Horizon-range forms of K2a and K3: the same computation as lqmpc_mpc_solve_batch / lqmpc_bounds_batch for every
+ * horizon N_min..N_max (H = N_max - N_min + 1), in one call, results stacked on a leading [H] axis (slot h = N - N_min).
+ *   lqmpc_mpc_solve_range: V [H][P][S], u0 [H][P][m][S], M_V [H][S], flags [H][P][S]; any output may be NULL.
+ *     Fused for the compiled (n, m) pairs with the input box and zero references: ONE unconstrained Riccati sweep of
+ *     N_max stages per sample serves every horizon (the law of horizon N at stage k is the sweep's stage
+ *     k + N_max - N), and the results are bit-identical to H single-horizon calls.
+ *   lqmpc_bounds_range: the arguments of lqmpc_bounds_batch with N_min, N_max for N; M_V [H][S] (or NULL ->
+ *     M_V_scalar); alpha, beta, xi, eta, bound, flags [H][S]; detail [H][lqmpc_bounds_fields()][S] (each horizon's
+ *     block has the single-horizon layout); K_out [m*n][S] and P_out [n*n][S] once (they do not depend on N).
+ *     Fused for the compiled (n, m) pairs with n <= 6 on the matrix-free route (scalar weights or
+ *     strict_reference = 0, with or without an input polytope, K_in / K_shared or the in-kernel DARE): the
+ *     horizon-independent part once per sample, the Gram-spectrum bisections of all horizons sharing their probes,
+ *     the error-consistent sums extended term by term. ||Gamma||^2 and lambda_min(H^) agree with
+ *     lqmpc_bounds_batch to the bisection tolerance 2^-42 of both searches, the fields computed from them to a few
+ *     times that; the others are the same formulas, which the compiler may contract into FMAs differently in the two
+ *     kernels (last-bit differences). bound = (alpha V_expert + beta) / (1 - xi - eta) magnifies these by
+ *     1 / |1 - xi - eta| where that denominator is near 0 (a bound at the edge of validity). Flags, K_out and P_out
+ *     are equal.
+ * Every other case — the run-time-dimension route, an installed input polytope or references (solve), the dense
+ * route of K3 (literal kron with non-scalar weights, LQMPC_K3_DENSE), K3 at n = 8 (measured faster per horizon) — is
+ * answered by one single-horizon call per N
+ * writing into the [h] slices. */
+int lqmpc_mpc_solve_range(lqmpc_ctx* ctx, int64_t S, const double* dA, const double* dB, int N_min, int N_max,
+                          int npts, const double* pts, const double* x0, double* V, double* u0, double* M_V,
+                          int32_t* flags);
+int lqmpc_bounds_range(lqmpc_ctx* ctx, int64_t S, const double* dA, const double* dB, int N_min, int N_max,
+                       const double* e_A, const double* e_B, double e_A_scalar, double e_B_scalar, const double* M_V,
+                       double M_V_scalar, const double* x_shared, const double* x, const double* K_in,
+                       const double* K_shared, const double* p3_host, double V_expert, double bar_u, double bar_d_u,
+                       int strict_reference, double* alpha, double* beta, double* xi, double* eta, double* bound,
+                       double* detail, double* K_out, double* P_out, int32_t* flags);
+
 /* Batched control.dlqr (utils_class.py:761,840,923): stabilising DARE solution P and K = (R+B'PB)^-1 B'PA
  * (convention u = -Kx) of (A+dA_s, B+dB_s); dA/dB NULL = the true model. K_out [m*n][S], P_out [n*n][S], flags [S]. */
 int lqmpc_dlqr_batch(lqmpc_ctx* ctx, int64_t S, const double* dA, const double* dB, double* K_out, double* P_out,

@@ -289,8 +289,58 @@ struct BoundsNorms {
   double nx2;               // ||x||^2
 };
 
+// Error-consistent sums of fc_ec_g_x / fc_ec_g_u (utils.py:78-117, 186-223, 296-305) over i = 0..N (bgu: i < N).
+struct EcSums {
+  double s_in, s_out, bgx, bgu;
+};
+
+LQ_HD EcSums ec_sums(int N, double fA, double fB, double e_A, double e_B, double nx, double bu) {
+  const double eAfA = e_A + fA, eBfB = e_B + fB;
+  double s_in = 0.0, s_out = 0.0, bgx = 0.0, bgu = 0.0, bgu_in = 0.0;
+  for (int i = 0; i <= N; ++i) {
+    const double fpi = pow(fA, (double)i);
+    const double gx1 = pow(eAfA, (double)i) - fpi;
+    const double gu1 = eBfB * gx1 + e_B * fpi;
+    s_out += (s_in + gx1 * gx1) * (nx * nx + i * bu);
+    s_in += gu1 * gu1;
+    if (i >= 1) bgx += gx1;
+    if (i < N) { bgu_in += gu1; bgu += bgu_in; }
+  }
+  EcSums r;
+  r.s_in = s_in; r.s_out = s_out; r.bgx = bgx; r.bgu = bgu;
+  return r;
+}
+
+// The same sums extended one horizon at a time (horizon range): each new term is computed exactly as ec_sums computes
+// it (pow, not running products: (e_A + fA)^i - fA^i cancels, and running products would carry their accumulated
+// rounding into the difference) and accumulated in the same order, so every horizon's sums equal ec_sums(N).
+// at(N) must be called with N = N_min, N_min + 1, ...
+struct EcRunning {
+  double fA, fB, e_A, e_B, nx, bu;
+  double s_in = 0.0, s_out = 0.0, bgx = 0.0, bgu = 0.0, bgu_in = 0.0, gu_pend = 0.0;
+  int i = 0;
+  bool pend = false;                     // gu_pend: the term i - 1 of bgu, owed once the horizon exceeds i - 1
+  LQ_HD EcSums at(int N) {
+    const double eAfA = e_A + fA, eBfB = e_B + fB;
+    if (pend && i - 1 < N) { bgu_in += gu_pend; bgu += bgu_in; pend = false; }
+    for (; i <= N; ++i) {
+      const double fpi = pow(fA, (double)i);
+      const double gx1 = pow(eAfA, (double)i) - fpi;
+      const double gu1 = eBfB * gx1 + e_B * fpi;
+      s_out += (s_in + gx1 * gx1) * (nx * nx + i * bu);
+      s_in += gu1 * gu1;
+      if (i >= 1) bgx += gx1;
+      if (i < N) { bgu_in += gu1; bgu += bgu_in; } else { gu_pend = gu1; pend = true; }
+    }
+    EcSums r;
+    r.s_in = s_in; r.s_out = s_out; r.bgx = bgx; r.bgu = bgu;
+    return r;
+  }
+};
+
+// es: the error-consistent sums of horizon sc.N when the caller carries them (horizon range), else computed here.
 LQ_HD int bounds_formulas(double maxQ, double minQ, double maxR, double minR, const BoundsScalars& sc,
-                          const BoundsNorms& q, double* out) {
+                          const BoundsNorms& q, double* out, const EcSums* es = nullptr) {
   int flags = 0;
   const int N = sc.N;
   const double fA = q.fA, fB = q.fB, nK = q.nK, eps_K = q.eps_K, rho_cl = q.rho_cl, bu = q.bu, bdu = q.bdu;
@@ -340,17 +390,8 @@ LQ_HD int bounds_formulas(double maxQ, double minQ, double maxR, double minR, co
   out[BF_H] = h; out[BF_XI] = xi;
   // ---------------- error-consistent sums (utils.py:78-117, 186-223, 296-305)
   const double nx = sqrt(nx2);
-  const double eAfA = sc.e_A + fA, eBfB = sc.e_B + fB;
-  double s_in = 0.0, s_out = 0.0, bgx = 0.0, bgu = 0.0, bgu_in = 0.0;
-  for (int i = 0; i <= N; ++i) {
-    const double fpi = pow(fA, (double)i);
-    const double gx1 = pow(eAfA, (double)i) - fpi;
-    const double gu1 = eBfB * gx1 + sc.e_B * fpi;
-    s_out += (s_in + gx1 * gx1) * (nx * nx + i * bu);
-    s_in += gu1 * gu1;
-    if (i >= 1) bgx += gx1;
-    if (i < N) { bgu_in += gu1; bgu += bgu_in; }
-  }
+  const EcSums ec = es ? *es : ec_sums(N, fA, fB, sc.e_A, sc.e_B, nx, bu);
+  const double s_out = ec.s_out, bgx = ec.bgx, bgu = ec.bgu;
   const double E_psi = maxQ * s_out;
   const double theta_u = maxQ * (2.0 * nG * bgu + bgu * bgu);
   const double theta_xu = maxQ * (nG * bgx + out[BF_NORM_PHI] * bgu + bgx * bgu);
@@ -378,16 +419,21 @@ LQ_HD double gamma_entry(const WsView& ws, const BoundsLayout<n, m>& L, int t, i
   return (t > j) ? ws[L.oG + (int64_t)(t - 1 - j) * (n * m) + r * m + s] : 0.0;
 }
 
-// Per-sample bound computation. K is the terminal gain in the u = +Kx convention (callers pass -K_dlqr).
-// out[BF_COUNT] receives every intermediate the reference's helper functions return.
+// ---- the horizon-independent part of the per-sample bound computation: input-set constants, ||A^||, ||B^||, ||K||,
+// local_radius and rho(A^ + B^ K). K is the terminal gain in the u = +Kx convention (callers pass -K_dlqr).
+struct BoundsPrefix {
+  double bu, bdu;           // max ||u||^2, max ||u1 - u2||^2 over the input set
+  double fA, fB, nK;        // ||A^||_2, ||B^||_2, ||K||_2
+  double eps_K;             // local_radius (utils.py:548-564)
+  double rho_cl;            // rho(A^ + B^ K)
+  int flags;
+};
+
 template <int n, int m>
-LQ_HD int bounds_sample(const Problem<n, m>& pb, const double* Ah, const double* Bh, const double* K,
-                        const double* x, const BoundsScalars& sc, const WsView& ws, double* out) {
-  const BoundsLayout<n, m> L(sc.N);
-  const int N = sc.N, k = L.k;
-  const bool matrix_free = bounds_matrix_free(pb.qr_scalar, sc.strict_reference, sc.force_dense);
-  int flags = 0;
-  LQ_UNROLL for (int i = 0; i < BF_COUNT; ++i) out[i] = 0.0;
+LQ_HD BoundsPrefix bounds_prefix(const Problem<n, m>& pb, const double* Ah, const double* Bh, const double* K,
+                                 const BoundsScalars& sc) {
+  BoundsPrefix pr;
+  pr.flags = 0;
   // ---------------- input-set constants (utils.py:592-650 for a box: attained at vertices)
   double bu = sc.bar_u, bdu = sc.bar_d_u;
   if (bu < 0.0) {
@@ -398,13 +444,10 @@ LQ_HD int bounds_sample(const Problem<n, m>& pb, const double* Ah, const double*
     bdu = 0.0;
     LQ_UNROLL for (int j = 0; j < m; ++j) bdu += (pb.uhi[j] - pb.ulo[j]) * (pb.uhi[j] - pb.ulo[j]);
   }
-  out[BF_BAR_U] = bu;
-  out[BF_BAR_D_U] = bdu;
+  pr.bu = bu;
+  pr.bdu = bdu;
   // ---------------- norms
-  const double fA = norm2<n, n>(Ah), fB = norm2<n, m>(Bh), nK = norm2<m, n>(K);
-  out[BF_NORM_A] = fA; out[BF_NORM_B] = fB; out[BF_NORM_K] = nK;
-  const double maxQ = pb.maxQ, minQ = pb.minQ, maxR = pb.maxR, minR = pb.minR;
-  const double ratioQ = maxQ / minQ;
+  pr.fA = norm2<n, n>(Ah); pr.fB = norm2<n, m>(Bh); pr.nK = norm2<m, n>(K);
   // ---------------- local_radius (utils.py:548-564): max_i ||(F_u K)_i||^2 in the Q^-1 metric — box rows, or the
   //                  rows of a general polytope
   double amax = 0.0;
@@ -425,8 +468,7 @@ LQ_HD int bounds_sample(const Problem<n, m>& pb, const double* Ah, const double*
       if (pb.uhi[j] < 1e300) amax = dmax(amax, kq / (pb.uhi[j] * pb.uhi[j]));
     }
   }
-  const double eps_K = 1.0 / amax;
-  out[BF_EPSILON_K] = eps_K;
+  pr.eps_K = 1.0 / amax;
   // ---------------- ex_stability_lq (utils.py:343-380)
   double Acl[n * n];
   LQ_UNROLL for (int i = 0; i < n; ++i)
@@ -436,33 +478,91 @@ LQ_HD int bounds_sample(const Problem<n, m>& pb, const double* Ah, const double*
       Acl[i * n + j] = acc;
     }
   bool eig_ok;
-  const double rho_cl = spectral_radius<n>(Acl, &eig_ok);
-  if (!eig_ok) flags |= FLAG_EIG_NOCONV;
-  out[BF_RHO_CL] = rho_cl;
-  // ---------------- G_d = A^d B, ||Phi||_2
-  double nPhi;
-  {
-    double Gd[n * m], Mt[n * n], acc[n * n];
-    LQ_UNROLL for (int i = 0; i < n * m; ++i) Gd[i] = Bh[i];
-    if (!matrix_free)
-      for (int d = 0; d < N; ++d) {
-        LQ_UNROLL for (int e = 0; e < n * m; ++e) ws[L.oG + (int64_t)d * (n * m) + e] = Gd[e];
-        double Gn[n * m];
-        mm<n, n, m>(Ah, Gd, Gn);
-        LQ_UNROLL for (int i = 0; i < n * m; ++i) Gd[i] = Gn[i];
-      }
+  pr.rho_cl = spectral_radius<n>(Acl, &eig_ok);
+  if (!eig_ok) pr.flags |= FLAG_EIG_NOCONV;
+  return pr;
+}
+
+// ||Phi||_2 of utils.py:126-144: Phi'Phi = sum_{t=0..N} (A^t)'A^t, one term per horizon. Extending the sum from N to
+// N + 1 adds the next term to the same accumulator, so every horizon of a range gets the single-horizon value exactly.
+template <int n>
+struct PhiGram {
+  double Mt[n * n], acc[n * n];
+  int t;
+  LQ_HD PhiGram() : t(0) {
     LQ_UNROLL for (int i = 0; i < n; ++i)
       LQ_UNROLL for (int j = 0; j < n; ++j) { Mt[i * n + j] = (i == j) ? 1.0 : 0.0; acc[i * n + j] = Mt[i * n + j]; }
-    for (int t = 1; t <= N; ++t) {
+  }
+  LQ_HD void extend_to(const double* Ah, int N) {
+    for (; t < N; ++t) {
       double Mn[n * n];
       mm<n, n, n>(Ah, Mt, Mn);
       LQ_UNROLL for (int i = 0; i < n * n; ++i) Mt[i] = Mn[i];
       sym_add_mtm<n, n>(acc, Mt, Mt, Mn);
       LQ_UNROLL for (int i = 0; i < n * n; ++i) acc[i] = Mn[i];
     }
+  }
+  LQ_HD double norm() const {
     double lo, hi;
     sym_eig_minmax<n>(acc, &lo, &hi);
-    nPhi = sqrt(dmax(hi, 0.0));
+    return sqrt(dmax(hi, 0.0));
+  }
+};
+
+// running error-consistent sums of one sample (horizon range): the constants of bounds_formulas
+template <int n>
+LQ_HD EcRunning ec_running(const BoundsPrefix& pr, const BoundsScalars& sc, const double* x) {
+  EcRunning r;
+  double nx2 = 0.0;
+  LQ_UNROLL for (int i = 0; i < n; ++i) nx2 = fma(x[i], x[i], nx2);
+  r.fA = pr.fA; r.fB = pr.fB; r.e_A = sc.e_A; r.e_B = sc.e_B; r.nx = sqrt(nx2); r.bu = pr.bu;
+  return r;
+}
+
+// ---- the per-horizon part: the scalar formulas on the prefix, ||Phi|| and the two Gram-spectrum extremes of horizon
+// sc.N. out[BF_COUNT] receives every intermediate the reference's helper functions return.
+template <int n, int m>
+LQ_HD int bounds_horizon(const Problem<n, m>& pb, const BoundsPrefix& pr, double nPhi, double cmax, double min_H,
+                         const double* x, const BoundsScalars& sc, double* out, const EcSums* es = nullptr) {
+  BoundsNorms q;
+  q.fA = pr.fA; q.fB = pr.fB; q.nK = pr.nK; q.eps_K = pr.eps_K; q.rho_cl = pr.rho_cl; q.nPhi = nPhi; q.cmax = cmax;
+  q.min_H = min_H;
+  q.bu = pr.bu; q.bdu = pr.bdu;
+  q.nx2 = 0.0;
+  LQ_UNROLL for (int i = 0; i < n; ++i) q.nx2 = fma(x[i], x[i], q.nx2);
+  int flags = pr.flags | bounds_formulas(pb.maxQ, pb.minQ, pb.maxR, pb.minR, sc, q, out, es);
+  LQ_UNROLL for (int i = 0; i < BF_COUNT; ++i)
+    if (!(fabs(out[i]) <= 1.79e308)) flags |= FLAG_NONFINITE;
+  return flags;
+}
+
+// Per-sample bound computation of one horizon: bounds_prefix + bounds_horizon with ||Gamma||, lambda_min(H^) from
+// the matrix-free bisection (or the dense route).
+template <int n, int m>
+LQ_HD int bounds_sample(const Problem<n, m>& pb, const double* Ah, const double* Bh, const double* K,
+                        const double* x, const BoundsScalars& sc, const WsView& ws, double* out) {
+  const BoundsLayout<n, m> L(sc.N);
+  const int N = sc.N, k = L.k;
+  const bool matrix_free = bounds_matrix_free(pb.qr_scalar, sc.strict_reference, sc.force_dense);
+  LQ_UNROLL for (int i = 0; i < BF_COUNT; ++i) out[i] = 0.0;
+  const BoundsPrefix pr = bounds_prefix<n, m>(pb, Ah, Bh, K, sc);
+  const double minR = pb.minR;
+  // ---------------- G_d = A^d B (dense route), ||Phi||_2
+  if (!matrix_free) {
+    double Gd[n * m];
+    LQ_UNROLL for (int i = 0; i < n * m; ++i) Gd[i] = Bh[i];
+    for (int d = 0; d < N; ++d) {
+      LQ_UNROLL for (int e = 0; e < n * m; ++e) ws[L.oG + (int64_t)d * (n * m) + e] = Gd[e];
+      double Gn[n * m];
+      mm<n, n, m>(Ah, Gd, Gn);
+      LQ_UNROLL for (int i = 0; i < n * m; ++i) Gd[i] = Gn[i];
+    }
+  }
+  double nPhi;
+  {
+    PhiGram<n> phi;
+    phi.extend_to(Ah, N);
+    nPhi = phi.norm();
   }
   double cmin = 0.0, cmax = 0.0, min_H;
   if (matrix_free) {
@@ -529,15 +629,7 @@ LQ_HD int bounds_sample(const Problem<n, m>& pb, const double* Ah, const double*
   }
   }
   // ---------------- scalar formulas (shared with the run-time-dimension route)
-  BoundsNorms q;
-  q.fA = fA; q.fB = fB; q.nK = nK; q.eps_K = eps_K; q.rho_cl = rho_cl; q.nPhi = nPhi; q.cmax = cmax; q.min_H = min_H;
-  q.bu = bu; q.bdu = bdu;
-  q.nx2 = 0.0;
-  LQ_UNROLL for (int i = 0; i < n; ++i) q.nx2 = fma(x[i], x[i], q.nx2);
-  flags |= bounds_formulas(maxQ, minQ, maxR, minR, sc, q, out);
-  LQ_UNROLL for (int i = 0; i < BF_COUNT; ++i)
-    if (!(fabs(out[i]) <= 1.79e308)) flags |= FLAG_NONFINITE;
-  return flags;
+  return bounds_horizon<n, m>(pb, pr, nPhi, cmax, min_H, x, sc, out);
 }
 
 }  // namespace lq

@@ -629,6 +629,76 @@ int lqmpc_bounds_batch(lqmpc_ctx* ctx, int64_t S, const double* dA, const double
   return ctx->dyn ? lq_dyn_bounds(ctx, a) : lq_launch_bounds(ctx, a);
 }
 
+int lqmpc_mpc_solve_range(lqmpc_ctx* ctx, int64_t S, const double* dA, const double* dB, int N_min, int N_max,
+                          int npts, const double* pts, const double* x0, double* V, double* u0, double* M_V,
+                          int32_t* flags) {
+  if (!ctx) return LQMPC_EINVAL;
+  if (!ctx->has_problem) return lq_set_error(ctx, LQMPC_ESTATE, "problem not set");
+  if (S < 0 || N_min < 1 || N_max < N_min) return lq_set_error(ctx, LQMPC_EINVAL, "bad S/N_min/N_max");
+  if (S == 0) return LQMPC_OK;
+  if ((pts == nullptr) == (x0 == nullptr)) return lq_set_error(ctx, LQMPC_EINVAL, "give exactly one of pts / x0");
+  if (pts && npts < 1) return lq_set_error(ctx, LQMPC_EINVAL, "npts < 1");
+  cudaSetDevice(ctx->device);
+  if (ctx->dyn || ctx->poly_p > 0 || ctx->ref_ld > 0) {
+    // no fused kernel (run-time dimensions, input polytope, references): one single-horizon launch per N
+    const int64_t P = pts ? npts : 1;
+    for (int N = N_min; N <= N_max; ++N) {
+      const int64_t h = N - N_min;
+      const int rc = lqmpc_mpc_solve_batch(ctx, S, dA, dB, N, npts, pts, x0, V ? V + h * P * S : nullptr,
+                                           u0 ? u0 + h * P * ctx->m * S : nullptr, M_V ? M_V + h * S : nullptr,
+                                           flags ? flags + h * P * S : nullptr);
+      if (rc) return rc;
+    }
+    return LQMPC_OK;
+  }
+  MpcArgs a{};
+  a.S = S; a.dA = dA; a.dB = dB; a.N_min = N_min; a.N = N_max; a.T = 0; a.npts = npts; a.pts = pts; a.x0 = x0;
+  a.V = V; a.u0 = u0; a.M_V = M_V; a.flags = flags;
+  return lq_launch_mpc_range(ctx, a);
+}
+
+int lqmpc_bounds_range(lqmpc_ctx* ctx, int64_t S, const double* dA, const double* dB, int N_min, int N_max,
+                       const double* e_A, const double* e_B, double e_A_scalar, double e_B_scalar, const double* M_V,
+                       double M_V_scalar, const double* x_shared, const double* x, const double* K_in,
+                       const double* K_shared, const double* p3_host, double V_expert, double bar_u, double bar_d_u,
+                       int strict_reference, double* alpha, double* beta, double* xi, double* eta, double* bound,
+                       double* detail, double* K_out, double* P_out, int32_t* flags) {
+  if (!ctx) return LQMPC_EINVAL;
+  if (!ctx->has_problem) return lq_set_error(ctx, LQMPC_ESTATE, "problem not set");
+  if (S < 0 || N_min < 1 || N_max < N_min) return lq_set_error(ctx, LQMPC_EINVAL, "bad S/N_min/N_max");
+  if (S == 0) return LQMPC_OK;
+  if ((x_shared == nullptr) == (x == nullptr)) return lq_set_error(ctx, LQMPC_EINVAL, "give exactly one of x_shared / x");
+  if (K_in && K_shared) return lq_set_error(ctx, LQMPC_EINVAL, "give at most one of K_in / K_shared");
+  if (!p3_host) return lq_set_error(ctx, LQMPC_EINVAL, "null p");
+  if (ctx->poly_p > 0 && (bar_u < 0.0 || bar_d_u < 0.0))
+    return lq_set_error(ctx, LQMPC_EINVAL, "with an input polytope installed bar_u / bar_d_u must be supplied (>= 0)");
+  cudaSetDevice(ctx->device);
+  BoundsArgs a{};
+  a.S = S; a.dA = dA; a.dB = dB; a.N_min = N_min; a.N = N_max; a.eA = e_A; a.eB = e_B; a.eA_s = e_A_scalar;
+  a.eB_s = e_B_scalar; a.MV = M_V; a.MV_s = M_V_scalar; a.x_shared = x_shared; a.x = x; a.K_in = K_in;
+  a.K_shared = K_shared; a.p[0] = p3_host[0]; a.p[1] = p3_host[1]; a.p[2] = p3_host[2];
+  a.V_expert = V_expert; a.bar_u = bar_u; a.bar_d_u = bar_d_u; a.strict = strict_reference;
+  a.alpha = alpha; a.beta = beta; a.xi = xi; a.eta = eta; a.bound = bound; a.detail = detail; a.K_out = K_out;
+  a.P_out = P_out; a.flags = flags;
+  if (ctx->poly_p > 0) { a.polyF = ctx->poly_dev; a.polyP = ctx->poly_p; }
+  if (!lq_bounds_range_fused(ctx, a)) {
+    // run-time dimensions or the dense route: one single-horizon launch per N (K_out / P_out from the first)
+    const int NF = (int)lq::BF_COUNT;
+    for (int N = N_min; N <= N_max; ++N) {
+      const int64_t h = N - N_min;
+      const int rc = lqmpc_bounds_batch(
+          ctx, S, dA, dB, N, e_A, e_B, e_A_scalar, e_B_scalar, M_V ? M_V + h * S : nullptr, M_V_scalar, x_shared, x,
+          K_in, K_shared, p3_host, V_expert, bar_u, bar_d_u, strict_reference, alpha ? alpha + h * S : nullptr,
+          beta ? beta + h * S : nullptr, xi ? xi + h * S : nullptr, eta ? eta + h * S : nullptr,
+          bound ? bound + h * S : nullptr, detail ? detail + h * NF * S : nullptr, h == 0 ? K_out : nullptr,
+          h == 0 ? P_out : nullptr, flags ? flags + h * S : nullptr);
+      if (rc) return rc;
+    }
+    return LQMPC_OK;
+  }
+  return lq_launch_bounds_range(ctx, a);
+}
+
 int lqmpc_dlqr_batch(lqmpc_ctx* ctx, int64_t S, const double* dA, const double* dB, double* K_out, double* P_out,
                      int32_t* flags) {
   if (!ctx) return LQMPC_EINVAL;

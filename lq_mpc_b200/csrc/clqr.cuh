@@ -147,6 +147,14 @@ LQ_HD int64_t clqr_ws_doubles(int N) {
   return ClqrLayout<n, m>(N).total;
 }
 
+// Horizon-range workspace (plan_prepare_range): the layout of an N_max-stage solve with the cost-to-go of EVERY stage
+// stored, so that each horizon N <= N_max finds its S_{klast+1} at stage klast + 1 + (N_max - N).
+template <int n, int m>
+LQ_HD int64_t clqr_range_ws_doubles(int N_max) {
+  const ClqrLayout<n, m> L(N_max);
+  return L.oP + (int64_t)N_max * L.np;
+}
+
 // Per-sample model of the controller (estimated system) + weights, in registers.
 template <int n, int m>
 struct Plan {
@@ -246,6 +254,50 @@ LQ_HD int plan_prepare(const Problem<n, m>& pb, Plan<n, m>& pl, int N, const WsV
   return flags;
 }
 
+// Unconstrained sweep of N_max stages for a whole horizon range. The law of horizon N at stage k is the Riccati iterate
+// with N - k stages to go, i.e. stage k + (N_max - N) of this sweep: one sweep holds the gains and cost-to-go of every
+// N <= N_max, computed by the same operations in the same order as plan_prepare(N). Stores every gain and every S_k
+// (the workspace of clqr_range_ws_doubles) and returns the stages-to-go of the first failed factorisation (N_max + 1:
+// none), so that horizon N carries FLAG_CHOL_FAIL iff that number is <= N. No certificate (the ring solves skip it).
+template <int n, int m>
+LQ_HD int plan_prepare_range(const Problem<n, m>& pb, Plan<n, m>& pl, int N_max, const WsView& ws) {
+  const ClqrLayout<n, m> L(N_max);
+  double P[n * n];
+  LQ_UNROLL for (int i = 0; i < n * n; ++i) P[i] = pb.Pt[i];
+  RicStage<n, m> st;
+  int first_fail = N_max + 1;
+  for (int k = N_max - 1; k >= 0; --k) {
+    riccati_factor<n, m>(P, pl.Bh, pb.R, st);
+    if (!st.ok && first_fail > N_max) first_fail = N_max - k;
+    double K[m * n];
+    riccati_gain<n, m>(st, pl.Ah, K);
+    LQ_UNROLL for (int e = 0; e < m * n; ++e) ws[L.oKu + (int64_t)k * (m * n) + e] = K[e];
+    riccati_update<n, m>(st, pl.Ah, pb.Q, P);
+    int e = 0;
+    LQ_UNROLL for (int i = 0; i < n; ++i)
+      LQ_UNROLL for (int j = i; j < n; ++j) { ws[L.oP + (int64_t)k * L.np + e] = P[i * n + j]; ++e; }
+  }
+  pl.cstar = pb.has_bounds ? -1.0 : HUGE_VAL;
+  return first_fail;
+}
+
+// Plan of horizon N inside a range sweep of N_max stages (koff = N_max - N): P0 is the stored cost-to-go with N stages
+// to go (riccati_update leaves P exactly symmetric, so the packed copy restores it bit for bit), K0 the gain there.
+template <int n, int m>
+LQ_HD void plan_select_horizon(Plan<n, m>& pl, int N_max, int koff, const WsView& ws) {
+  const ClqrLayout<n, m> L(N_max);
+  int e = 0;
+  LQ_UNROLL for (int i = 0; i < n; ++i)
+    LQ_UNROLL for (int j = i; j < n; ++j) {
+      const double v = ws[L.oP + (int64_t)koff * L.np + e];
+      pl.P0[i * n + j] = v; pl.P0[j * n + i] = v; ++e;
+    }
+  if (Plan<n, m>::kHoldK0) {
+    LQ_UNROLL for (int e2 = 0; e2 < m * n; ++e2)
+      pl.K0[Plan<n, m>::kHoldK0 ? e2 : 0] = ws[L.oKu + (int64_t)koff * (m * n) + e2];
+  }
+}
+
 template <int n, int m>
 LQ_HD void step_model(const double* A, const double* B, const double* x, const double* u, double* xn) {
   LQ_UNROLL for (int i = 0; i < n; ++i) {
@@ -261,10 +313,12 @@ LQ_HD void step_model(const double* A, const double* B, const double* x, const d
 // unconstrained with a purely quadratic cost-to-go, so their law IS the unconstrained one (ws.Ku, zero offset) and the
 // sweep starts at klast from the stored S_{klast+1} — O(klast) stages instead of N per active-set iteration (in the
 // sweeps of utils_class.py:802-833 the inputs saturate at the first steps only). Pass N - 1 for a full sweep.
+// `koff`: stage offset of the stored unconstrained gains and cost-to-go — horizon N inside a range sweep of N + koff
+// stages (plan_prepare_range) reads its stage k at k + koff; 0 for a single-horizon plan.
 template <int n, int m>
 LQ_HD bool clqr_backward(const Problem<n, m>& pb, const Plan<n, m>& pl, int N, const Mask128& fixed, const Mask128& athi,
-                         const WsView& ws, const Refs& rf = Refs(), int klast = -2) {
-  const ClqrLayout<n, m> L(N);
+                         const WsView& ws, const Refs& rf = Refs(), int klast = -2, int koff = 0) {
+  const ClqrLayout<n, m> L(N + koff);
   if (klast < -1 || klast > N - 1) klast = N - 1;
   // cost-to-go INCLUDING the state's own stage term: Phi_k(x) = x'S x + 2 s'x + const; Phi_N = (x - r_{N-1})'P(x - r_{N-1})
   double S[n * n], s[n];
@@ -279,7 +333,7 @@ LQ_HD bool clqr_backward(const Problem<n, m>& pb, const Plan<n, m>& pl, int N, c
     int e = 0;
     LQ_UNROLL for (int i = 0; i < n; ++i)
       LQ_UNROLL for (int j = i; j < n; ++j) {
-        const double v = ws[L.oP + (int64_t)(klast + 1) * L.np + e];
+        const double v = ws[L.oP + (int64_t)(klast + 1 + koff) * L.np + e];
         S[i * n + j] = v; S[j * n + i] = v; ++e;
       }
     LQ_UNROLL for (int i = 0; i < n; ++i) s[i] = 0.0;
@@ -377,8 +431,9 @@ LQ_HD bool clqr_backward(const Problem<n, m>& pb, const Plan<n, m>& pl, int N, c
 // n = 8: 32 registers and 55 kB of spills per thread).
 template <int n, int m>
 LQ_HD_NOINLINE_T bool clqr_backward_call(const Problem<n, m>& pb, const Plan<n, m>& pl, int N, const Mask128& fixed,
-                                         const Mask128& athi, const WsView& ws, const Refs& rf, int klast) {
-  return clqr_backward<n, m>(pb, pl, N, fixed, athi, ws, rf, klast);
+                                         const Mask128& athi, const WsView& ws, const Refs& rf, int klast,
+                                         int koff = 0) {
+  return clqr_backward<n, m>(pb, pl, N, fixed, athi, ws, rf, klast, koff);
 }
 
 // Exact constrained solve from state x0. Returns flags; writes u0[m] and V (= optimum + x0'Qx0).
@@ -387,19 +442,23 @@ LQ_HD_NOINLINE_T bool clqr_backward_call(const Problem<n, m>& pb, const Plan<n, 
 //   per active-set iteration: a backward sweep over the stages up to the last clamped one, ONE forward sweep that
 //   also accumulates the objective of its candidate, and a costate sweep over the clamped stages only — the tail
 //   beyond them is unconstrained with cost-to-go x'S x, so its costate is 2 S x without a sweep.
+// `koff` (see clqr_backward): horizon N of a range sweep reads the stored unconstrained gains / cost-to-go at stage
+// k + koff; which working sets restart from a stored S is decided by the stored-stage count of horizon N itself.
 template <int n, int m>
 LQ_HD int clqr_solve(const Problem<n, m>& pb, const Plan<n, m>& pl, int N, const double* x0, const WsView& ws,
-                     double* u0, double* V, const Refs& rf = Refs()) {
-  const ClqrLayout<n, m> L(N);
+                     double* u0, double* V, const Refs& rf = Refs(), int koff = 0) {
+  const ClqrLayout<n, m> L(N + koff);
+  const int kp = (N < kStoredCostToGo) ? N : kStoredCostToGo;   // == ClqrLayout(N).kp
+  const int64_t oKu = L.oKu + (int64_t)koff * (m * n);
   double x[n], xn[n], u[m];
   const bool trk = rf.any();
   int flags = 0;
   // ---- 1. unconstrained plan, clipped into the box as it is rolled out: no clip => it is the QP minimiser. With
   //         references the plan is affine: gains AND offsets come from the affine sweep with an empty working set.
-  if (trk && !((n <= 4) ? clqr_backward<n, m>(pb, pl, N, Mask128(), Mask128(), ws, rf, N - 1)
-                        : clqr_backward_call<n, m>(pb, pl, N, Mask128(), Mask128(), ws, rf, N - 1)))
+  if (trk && !((n <= 4) ? clqr_backward<n, m>(pb, pl, N, Mask128(), Mask128(), ws, rf, N - 1, koff)
+                        : clqr_backward_call<n, m>(pb, pl, N, Mask128(), Mask128(), ws, rf, N - 1, koff)))
     flags |= FLAG_CHOL_FAIL;
-  const int64_t oK = trk ? L.oKc : L.oKu;
+  const int64_t oK = trk ? L.oKc : oKu;
   if (!trk) {
     // ---- 0. regulation: inside the certificate ellipsoid the unconstrained plan is feasible, hence optimal
     const double V0 = quad<n>(x0, pl.P0, x0);
@@ -408,7 +467,7 @@ LQ_HD int clqr_solve(const Problem<n, m>& pb, const Plan<n, m>& pl, int N, const
         mv<m, n>(pl.K0, x0, u0);
       } else {
         double K[m * n];
-        LQ_UNROLL for (int e = 0; e < m * n; ++e) K[e] = ws[L.oKu + e];
+        LQ_UNROLL for (int e = 0; e < m * n; ++e) K[e] = ws[oKu + e];
         mv<m, n>(K, x0, u0);
       }
       *V = V0;
@@ -484,9 +543,9 @@ LQ_HD int clqr_solve(const Problem<n, m>& pb, const Plan<n, m>& pl, int N, const
     // regulation: stages beyond the last clamped one keep the unconstrained law — the sweep covers 0..klast only
     const int top = fixed.top_bit();
     int klast = trk ? N - 1 : (top < 0 ? -1 : top / m);
-    if (klast + 1 >= L.kp) klast = N - 1;                  // S_{klast+1} is not stored that far out: full sweep
-    if (!((n <= 4) ? clqr_backward<n, m>(pb, pl, N, fixed, athi, ws, rf, klast)
-                   : clqr_backward_call<n, m>(pb, pl, N, fixed, athi, ws, rf, klast)))
+    if (klast + 1 >= kp) klast = N - 1;                    // S_{klast+1} is not stored that far out: full sweep
+    if (!((n <= 4) ? clqr_backward<n, m>(pb, pl, N, fixed, athi, ws, rf, klast, koff)
+                   : clqr_backward_call<n, m>(pb, pl, N, fixed, athi, ws, rf, klast, koff)))
       flags |= FLAG_CHOL_FAIL;
     // forward sweep: candidate z*, its trajectory (kept up to stage klast + 1: all the costate sweep reads), its
     // objective, and the largest feasible step along z* - z
@@ -498,7 +557,7 @@ LQ_HD int clqr_solve(const Problem<n, m>& pb, const Plan<n, m>& pl, int N, const
     // per stage: the gain, its offset (zero beyond klast: unconstrained law) and the current iterate z_k
     staged_loop<m * n + 2 * m, StagePrefetch<n, m>::depth>(N, [&](int k, double* v) {
       const bool tl = (k > klast);
-      const int64_t og = tl ? L.oKu : L.oKc;
+      const int64_t og = tl ? oKu : L.oKc;
       LQ_UNROLL for (int e = 0; e < m * n; ++e) v[e] = ws[og + (int64_t)k * (m * n) + e];
       LQ_UNROLL for (int j = 0; j < m; ++j) {
         v[m * n + j] = tl ? 0.0 : ws[L.okc + (int64_t)k * m + j];
@@ -564,7 +623,7 @@ LQ_HD int clqr_solve(const Problem<n, m>& pb, const Plan<n, m>& pl, int N, const
       int e = 0;
       LQ_UNROLL for (int i = 0; i < n; ++i)
         LQ_UNROLL for (int j = i; j < n; ++j) {
-          const double v = ws[L.oP + (int64_t)(klast + 1) * L.np + e];
+          const double v = ws[L.oP + (int64_t)(klast + 1 + koff) * L.np + e];
           Sk[i * n + j] = v; Sk[j * n + i] = v; ++e;
         }
       LQ_UNROLL for (int i = 0; i < n; ++i) xe[i] = ws[L.oxs + (int64_t)(klast + 1) * n + i];

@@ -79,6 +79,7 @@ struct MpcArgs {
   const double* dA;   // [n*n][S] or NULL (zero perturbation)
   const double* dB;   // [n*m][S] or NULL
   int N, T;
+  int N_min = 0;      // range launch (lq_launch_mpc_range): horizons N_min..N, outputs with a leading [H] axis
   int npts;
   const double* pts;  // shared initial states [npts][n] (device) or NULL
   const double* x0;   // per-sample initial states [n][S] (device), used when pts == NULL
@@ -103,6 +104,7 @@ struct BoundsArgs {
   const double* dA;
   const double* dB;
   int N;
+  int N_min = 0;          // range launch (lq_launch_bounds_range): horizons N_min..N, outputs with a leading [H] axis
   const double* eA;       // [S] or NULL -> eA_s
   const double* eB;
   double eA_s, eB_s;
@@ -156,7 +158,10 @@ int lq_launch_fp64_peak(lqmpc_ctx* ctx, double* tflops);
 int lq_launch_dmma_peak(lqmpc_ctx* ctx, double* tflops);
 int lq_launch_mpc(lqmpc_ctx* ctx, const MpcArgs& a, bool simulate);
 int lq_launch_mpc_poly(lqmpc_ctx* ctx, const MpcArgs& a, bool simulate);
+int lq_launch_mpc_range(lqmpc_ctx* ctx, const MpcArgs& a);
 int lq_launch_bounds(lqmpc_ctx* ctx, const BoundsArgs& a);
+bool lq_bounds_range_fused(lqmpc_ctx* ctx, const BoundsArgs& a);
+int lq_launch_bounds_range(lqmpc_ctx* ctx, const BoundsArgs& a);
 int lq_launch_stats(lqmpc_ctx* ctx, const double* table, int cols, int64_t S, int64_t ld, double* stats);
 int lq_launch_moments(lqmpc_ctx* ctx, const double* table, int cols, int64_t S, int64_t ld, double* out);
 int lq_launch_sqdev(lqmpc_ctx* ctx, const double* table, int cols, int64_t S, int64_t ld, const double* mean,

@@ -257,4 +257,219 @@ LQ_HD GramSpectrum gram_spectrum(const double* Ah, const double* Bh, const doubl
   return out;
 }
 
+// Stopping rule of the bisections: the bracket is narrower than kGramSpectrumTol relative, or its midpoint no longer
+// separates the ends.
+LQ_HD bool gs_live(double lo, double hi) {
+  const double mid = 0.5 * (lo + hi);
+  return (hi - lo > kGramSpectrumTol * hi) && (mid > lo) && (mid < hi);
+}
+
+// Both extremes for every horizon N_min..N_max; emit(N, GramSpectrum) is called for each N in increasing order, with
+// `probes` = the bisection passes spent on that horizon. Returns the elimination stages run in total.
+//
+// The elimination runs from the last stage (PH starts at Q, PC at I), so the pivot at s stages to go is the same for
+// every horizon: "H^_N - x I > 0" iff G_1..G_N(x) are positive, and likewise for x I - Gamma_N'Gamma_N. Hence
+//   * a probe that runs one stage beyond N also answers the predicate of horizon N + 1 — bit for bit the probe a
+//     search of horizon N + 1 would make at that shift — and the probes of horizon N leave N + 1 a bracket;
+//   * lambda_min(H^_N) is non-increasing and lambda_max(Gamma_N'Gamma_N) non-decreasing in N: the fail side of
+//     horizon N (a shift whose pivots fail within N stages) is a fail side of N + 1;
+//   * a horizon whose inherited bracket is already converged spends one probe at its pass side, which certifies that
+//     side for N + 1 (where the extremes have converged in N, every later horizon costs this one probe);
+//   * otherwise the first two probes certify a guess: the extreme extrapolated from the previous horizons (a polynomial
+//     in N for lambda_min(H^), which settles to a limit; through the ratio of successive values for
+//     lambda_max(Gamma'Gamma), which grows like rho(A^)^2N when A^ is unstable; second order from three horizons,
+//     first order from two), +- a relative margin of twice the previous extrapolation error (2^-40 .. 2^-6). Both probes
+//     inside the bracket shrink it to twice the margin; a miss still moves one end.
+// Each horizon then bisects with the one-sided predicates and the stopping rule of gram_spectrum. The first searched
+// horizon starts from gram_spectrum's brackets, so N_min == N_max IS gram_spectrum(N_max).
+// State of the range search between horizons; next() searches the next horizon. The n >= 5 kernels call it through
+// the non-inlined gram_range_next_call (as gram_spectrum_call: inlined there, the register allocator gives up).
+template <int n, int m>
+struct GramRange {
+  const double *Ah, *Bh, *Q, *R;
+  int N, N_max;                                  // N: the last horizon searched (or N_min - 1)
+  double colsq[m], sumF, Gd[n * m], loH0, hiH0, M3[9];
+  // what the probes so far say about the NEXT horizon: H pass / fail sides, C fail / pass sides
+  double nLoH, nHiH, nLoC, nHiC;
+  bool inhH, inhC;
+  double vH1, vH2, vH3, vC1, vC2, vC3;           // results of the previous horizons
+  double errH, errC;                             // relative errors of their guesses
+  int hist;                                      // consecutive searched horizons behind N (for the extrapolation)
+  int stages;
+
+  LQ_HD void init(const double* Ah_, const double* Bh_, const double* Q_, const double* R_, double minR, int N_min,
+                  int N_max_) {
+    Ah = Ah_; Bh = Bh_; Q = Q_; R = R_; N_max = N_max_; N = 0;
+    // brackets of gram_spectrum: the impulse-response sums colsq / sumF grow by one term per horizon; the H side does
+    // not depend on N
+    sumF = 0.0;
+    LQ_UNROLL for (int j = 0; j < m; ++j) colsq[j] = 0.0;
+    LQ_UNROLL for (int e = 0; e < n * m; ++e) Gd[e] = Bh[e];
+    loH0 = minR * (1.0 - 1e-15);
+    hiH0 = HUGE_VAL;
+    {
+      double QB[n * m];
+      mm<n, n, m>(Q, Bh, QB);
+      LQ_UNROLL for (int j = 0; j < m; ++j) {
+        double acc = R[j * m + j];
+        LQ_UNROLL for (int k = 0; k < n; ++k) acc = fma(Bh[k * m + j], QB[k * m + j], acc);
+        hiH0 = dmin(hiH0, acc);
+      }
+      hiH0 *= (1.0 + 1e-14);
+    }
+    if (n == 2) gs_congruence2(Ah, M3);
+    nLoH = -HUGE_VAL; nHiH = HUGE_VAL; nLoC = -HUGE_VAL; nHiC = HUGE_VAL;
+    inhH = inhC = false;
+    vH1 = vH2 = vH3 = vC1 = vC2 = vC3 = 0.0;
+    errH = errC = 0x1p-6;
+    hist = 0;
+    stages = 0;
+    while (N + 1 < N_min) extend();
+  }
+
+  LQ_HD void extend() {                          // impulse-response term of horizon N + 1
+    ++N;
+    double fro = 0.0;
+    LQ_UNROLL for (int r = 0; r < n; ++r)
+      LQ_UNROLL for (int j = 0; j < m; ++j) {
+        const double g = Gd[r * m + j];
+        colsq[j] = fma(g, g, colsq[j]);
+        fro = fma(g, g, fro);
+      }
+    sumF += sqrt(fro);
+    double Gn[n * m];
+    mm<n, n, m>(Ah, Gd, Gn);
+    LQ_UNROLL for (int e = 0; e < n * m; ++e) Gd[e] = Gn[e];
+  }
+
+  LQ_HD GramSpectrum next() {
+    extend();
+    double eye[n * n];
+    LQ_UNROLL for (int i = 0; i < n; ++i)
+      LQ_UNROLL for (int j = 0; j < n; ++j) eye[i * n + j] = (i == j) ? 1.0 : 0.0;
+    double loC = 0.0;
+    LQ_UNROLL for (int j = 0; j < m; ++j) loC = dmax(loC, colsq[j]);
+    loC *= (1.0 - 1e-14);
+    double hiC = sumF * sumF * (1.0 + 1e-14);
+    double loH = loH0, hiH = hiH0;
+    bool liveH = (hiH > loH), liveC = (hiC > loC) && (hiC == hiC) && (hiC < 1.7e308);
+    if (!(hiC == hiC) || !(hiC < 1.7e308)) { loC = hiC = sumF * sumF; }      // overflow / NaN operands: propagate
+    const bool srchH = liveH, srchC = liveC;     // valid brackets: their probes inform horizon N + 1
+    if (inhH && liveH) { loH = dmax(loH, nLoH); hiH = dmin(hiH, nHiH); liveH = gs_live(loH, hiH); }
+    if (inhC && liveC) { loC = dmax(loC, nLoC); hiC = dmin(hiC, nHiC); liveC = gs_live(loC, hiC); }
+    const int L = (N < N_max) ? N + 1 : N;      // probes look one stage ahead
+    nLoH = -HUGE_VAL; nHiH = HUGE_VAL; nLoC = -HUGE_VAL; nHiC = HUGE_VAL;
+    bool cert = !liveH && !liveC && (L > N) && (srchH || srchC);
+    double gH[2] = {0.0, 0.0}, gC[2] = {0.0, 0.0}, guessH = 0.0, guessC = 0.0;
+    int kH = 2, kC = 2;                          // next certification point of the guess (2: none left)
+    if (hist >= 2 && liveH && vH2 > 0.0) {
+      guessH = (hist >= 3) ? fma(3.0, vH1 - vH2, vH3) : 2.0 * vH1 - vH2;
+      const double d = dmin(dmax(2.0 * errH, 0x1p-40), 0x1p-6);
+      gH[0] = guessH * (1.0 - d); gH[1] = guessH * (1.0 + d); kH = 0;   // pass side (lo) first
+    }
+    if (hist >= 2 && liveC && vC2 > 0.0) {
+      const double r1 = vC1 / vC2;
+      guessC = vC1 * ((hist >= 3 && vC3 > 0.0) ? 2.0 * r1 - vC2 / vC3 : r1);
+      const double d = dmin(dmax(2.0 * errC, 0x1p-40), 0x1p-6);
+      gC[0] = guessC * (1.0 + d); gC[1] = guessC * (1.0 - d); kC = 0;   // pass side (hi) first
+    }
+    int pass = 0;
+    for (; pass < 128 && (liveH || liveC || cert); ++pass) {
+      double xH = cert ? loH : 0.5 * (loH + hiH), xC = cert ? hiC : 0.5 * (loC + hiC);
+      while (kH < 2 && !(gH[kH] > loH && gH[kH] < hiH)) ++kH;
+      if (kH < 2 && liveH) xH = gH[kH++];
+      while (kC < 2 && !(gC[kC] > loC && gC[kC] < hiC)) ++kC;
+      if (kC < 2 && liveC) xC = gC[kC++];
+      double RdH[m * m], RdC[m * m], PH[n * n], PC[n * n];
+      LQ_UNROLL for (int i = 0; i < m; ++i)
+        LQ_UNROLL for (int j = 0; j < m; ++j) {
+          RdH[i * m + j] = R[i * m + j] - ((i == j) ? xH : 0.0);
+          RdC[i * m + j] = (i == j) ? xC : 0.0;
+        }
+      LQ_UNROLL for (int e = 0; e < n * n; ++e) { PH[e] = Q[e]; PC[e] = eye[e]; }
+      bool okH = true, okC = true, hN = false, cN = false;   // ok*: pivots 1..s positive; *N: pivots 1..N positive
+      if (n <= 4) {                       // the two recursions interleaved, as in gram_spectrum
+        for (int s = 1; s < L; ++s) {
+          if (n == 2) {
+            okH = gs_stage2<m, false>(M3, Bh, Q, RdH, 1.0, PH) && okH;
+            okC = gs_stage2<m, false>(M3, Bh, eye, RdC, -1.0, PC) && okC;
+          } else {
+            okH = gs_stage<n, m>(Ah, Bh, Q, RdH, 1.0, false, PH) && okH;
+            okC = gs_stage<n, m>(Ah, Bh, eye, RdC, -1.0, false, PC) && okC;
+          }
+          ++stages;
+          if (s == N) { hN = okH; cN = okC; }
+          if (!okH && !okC) break;
+        }
+        if (okH || okC) {                 // stage L (peeled): pivots only
+          if (n == 2) {
+            okH = gs_stage2<m, true>(M3, Bh, Q, RdH, 1.0, PH) && okH;
+            okC = gs_stage2<m, true>(M3, Bh, eye, RdC, -1.0, PC) && okC;
+          } else {
+            okH = gs_stage<n, m>(Ah, Bh, Q, RdH, 1.0, true, PH) && okH;
+            okC = gs_stage<n, m>(Ah, Bh, eye, RdC, -1.0, true, PC) && okC;
+          }
+          ++stages;
+        }
+        if (L == N) { hN = okH; cN = okC; }
+      } else {                            // n >= 5: one recursion at a time
+        for (int s = 1; s <= L && okH; ++s) {
+          okH = gs_stage<n, m>(Ah, Bh, Q, RdH, 1.0, s == L, PH);
+          ++stages;
+          if (s == N) hN = okH;
+        }
+        for (int s = 1; s <= L && okC; ++s) {
+          okC = gs_stage<n, m>(Ah, Bh, eye, RdC, -1.0, s == L, PC);
+          ++stages;
+          if (s == N) cN = okC;
+        }
+      }
+      if (liveH) {
+        if (hN) loH = xH; else hiH = xH;
+        liveH = gs_live(loH, hiH);
+      }
+      if (liveC) {
+        if (cN) hiC = xC; else loC = xC;
+        liveC = gs_live(loC, hiC);
+      }
+      if (L > N) {                        // pivots 1..N+1: the predicate of horizon N + 1 at these shifts
+        if (srchH) { if (okH) nLoH = dmax(nLoH, xH); else nHiH = dmin(nHiH, xH); }
+        if (srchC) { if (okC) nHiC = dmin(nHiC, xC); else nLoC = dmax(nLoC, xC); }
+      }
+      cert = false;
+    }
+    GramSpectrum out;
+    out.min_H = 0.5 * (loH + hiH);
+    out.cmax = 0.5 * (loC + hiC);
+    out.probes = pass;
+    // the fail sides of horizon N fail within N stages, hence for N + 1 as well
+    nHiH = dmin(nHiH, hiH);
+    nLoC = dmax(nLoC, loC);
+    inhH = srchH;
+    inhC = srchC;
+    if (guessH > 0.0) errH = fabs(guessH - out.min_H) / out.min_H;
+    if (guessC > 0.0) errC = fabs(guessC - out.cmax) / out.cmax;
+    if (!(errH < 0x1p-6)) errH = 0x1p-6;
+    if (!(errC < 0x1p-6)) errC = 0x1p-6;
+    vH3 = vH2; vH2 = vH1; vH1 = out.min_H;
+    vC3 = vC2; vC2 = vC1; vC1 = out.cmax;
+    hist = (srchH && srchC) ? hist + 1 : 0;
+    return out;
+  }
+};
+
+template <int n, int m>
+LQ_HD_NOINLINE_T GramSpectrum gram_range_next_call(GramRange<n, m>& g) {
+  return g.next();
+}
+
+template <int n, int m, class Emit>
+LQ_HD int gram_spectrum_range(const double* Ah, const double* Bh, const double* Q, const double* R, double minR,
+                              int N_min, int N_max, Emit emit) {
+  GramRange<n, m> g;
+  g.init(Ah, Bh, Q, R, minR, N_min, N_max);
+  for (int N = N_min; N <= N_max; ++N) emit(N, (n <= 4) ? g.next() : gram_range_next_call<n, m>(g));
+  return g.stages;
+}
+
 }  // namespace lq

@@ -10,3 +10,12 @@ int lq_launch_mpc(lqmpc_ctx* ctx, const MpcArgs& a, bool sim) {
 #undef X
   return lq_set_error(ctx, LQMPC_EINVAL, "unsupported (n, m); see lqmpc_supported_dims()");
 }
+
+// Horizon range with the input box and zero references (the caller routes every other case to per-horizon launches).
+int lq_launch_mpc_range(lqmpc_ctx* ctx, const MpcArgs& a) {
+#define X(N_, M_) \
+  if (ctx->n == N_ && ctx->m == M_) return launch_mpc_range_t<N_, M_>(ctx, a);
+  LQ_FOR_EACH_DIM(X)
+#undef X
+  return lq_set_error(ctx, LQMPC_EINVAL, "unsupported (n, m); see lqmpc_supported_dims()");
+}

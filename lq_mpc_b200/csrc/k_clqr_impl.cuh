@@ -69,6 +69,45 @@ __global__ void __launch_bounds__(128, K2Occupancy<n, m>::min_blocks) mpc_solve_
   }
 }
 
+// Horizon range N_min..N_max (box, zero references): ONE unconstrained sweep of N_max stages per sample
+// (plan_prepare_range), then the ring solves of every horizon through the stage-offset view of that sweep. Outputs
+// V [H][P][S], u0 [H][P][m][S], M_V [H][S], flags [H][P][S]; bit-identical to H single-horizon launches.
+template <int n, int m>
+__global__ void __launch_bounds__(128, K2Occupancy<n, m>::min_blocks) mpc_solve_range_kernel(
+    const __grid_constant__ lq::Problem<n, m> pb, const __grid_constant__ MpcArgs a) {
+  const int64_t tid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  const int64_t nthreads = (int64_t)gridDim.x * blockDim.x;
+  const lq::WsView ws{a.ws + tid, nthreads};
+  const int P = a.pts ? a.npts : 1;
+  for (int64_t s = tid; s < a.S; s += nthreads) {
+    lq::Plan<n, m> pl;
+    load_plan<n, m>(a, pb, s, pl);
+    const int first_fail = lq::plan_prepare_range<n, m>(pb, pl, a.N, ws);
+    for (int N = a.N_min; N <= a.N; ++N) {
+      const int koff = a.N - N;
+      const int64_t h = N - a.N_min;
+      lq::plan_select_horizon<n, m>(pl, a.N, koff, ws);
+      const int pf = (first_fail <= N) ? lq::FLAG_CHOL_FAIL : 0;   // only the N stages of this horizon count
+      double mv = -HUGE_VAL;
+      for (int p = 0; p < P; ++p) {
+        double x0[n], u0[m], V;
+#pragma unroll
+        for (int i = 0; i < n; ++i) x0[i] = a.pts ? a.pts[p * n + i] : a.x0[(int64_t)i * a.S + s];
+        const int f = pf | lq::clqr_solve<n, m>(pb, pl, N, x0, ws, u0, &V, lq::Refs(), koff);
+        mv = lq::dmax(mv, V);
+        const int64_t hp = h * P + p;
+        if (a.V) a.V[hp * a.S + s] = V;
+        if (a.u0) {
+#pragma unroll
+          for (int j = 0; j < m; ++j) a.u0[(hp * m + j) * a.S + s] = u0[j];
+        }
+        if (a.flags) a.flags[hp * a.S + s] = f;
+      }
+      if (a.M_V) a.M_V[h * a.S + s] = mv;
+    }
+  }
+}
+
 template <int n, int m>
 struct DevTraj {
   const MpcArgs& a;
@@ -147,6 +186,30 @@ int launch_mpc_t(lqmpc_ctx* ctx, MpcArgs a, bool sim) {
     mpc_solve_kernel<n, m, POLY><<<(unsigned)blocks, threads, 0, ctx->stream>>>(pb, a);
   ctx->launches++;
   return lq_check_cuda(ctx, cudaGetLastError(), sim ? "simulate_kernel launch" : "mpc_solve_kernel launch");
+}
+
+template <int n, int m>
+int launch_mpc_range_t(lqmpc_ctx* ctx, MpcArgs a) {
+  const lq::Problem<n, m>& pb = *reinterpret_cast<const lq::Problem<n, m>*>(ctx->pb);
+  int sms = 148;
+  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, ctx->device);
+  const int threads = 128;
+  int64_t blocks = (a.S + threads - 1) / threads;
+  int occ = 0;
+  cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, mpc_solve_range_kernel<n, m>, threads, 0);
+  if (occ < 1) occ = 1;
+  int waves = (a.N >= 20) ? 1 : 3;                       // the grid cap of launch_mpc_t, at the longest horizon
+  if (const char* wv = getenv("LQMPC_K2_WAVES")) { if (atoi(wv) > 0) waves = atoi(wv); }
+  const int64_t cap = (int64_t)sms * occ * waves;
+  if (blocks > cap) blocks = cap;
+  const int64_t nthreads = blocks * threads;
+  const int64_t per = lq::clqr_range_ws_doubles<n, m>(a.N);
+  int rc = lq_reserve_ws(ctx, (size_t)(per * nthreads) * sizeof(double));
+  if (rc) return rc;
+  a.ws = reinterpret_cast<double*>(ctx->ws);
+  mpc_solve_range_kernel<n, m><<<(unsigned)blocks, threads, 0, ctx->stream>>>(pb, a);
+  ctx->launches++;
+  return lq_check_cuda(ctx, cudaGetLastError(), "mpc_solve_range_kernel launch");
 }
 
 }  // namespace

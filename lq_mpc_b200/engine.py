@@ -57,6 +57,10 @@ ABI = {
     "lqmpc_bounds_batch": (_int, [_vp, _i64, _vp, _vp, _int, _vp, _vp, ctypes.c_double, ctypes.c_double, _vp,
                                   ctypes.c_double, _vp, _vp, _vp, _vp, _vp, ctypes.c_double, ctypes.c_double,
                                   ctypes.c_double, _int] + [_vp] * 9),
+    "lqmpc_mpc_solve_range": (_int, [_vp, _i64, _vp, _vp, _int, _int, _int] + [_vp] * 6),
+    "lqmpc_bounds_range": (_int, [_vp, _i64, _vp, _vp, _int, _int, _vp, _vp, ctypes.c_double, ctypes.c_double, _vp,
+                                  ctypes.c_double, _vp, _vp, _vp, _vp, _vp, ctypes.c_double, ctypes.c_double,
+                                  ctypes.c_double, _int] + [_vp] * 9),
     "lqmpc_dlqr_batch": (_int, [_vp, _i64, _vp, _vp, _vp, _vp, _vp]),
     "lqmpc_column_stats": (_int, [_vp, _vp, _int, _i64, _i64, _vp]),
     "lqmpc_column_sqdev": (_int, [_vp, _vp, _int, _i64, _i64, _vp, _vp]),
@@ -439,6 +443,43 @@ class Engine:
         return out
 
     @_streamed
+    def mpc_solve_range(self, dA, dB, N_min: int, N_max: int, pts=None, x0=None, S: Optional[int] = None,
+                        want=("V", "u0", "M_V", "flags")):
+        """mpc_solve_batch for every horizon N_min..N_max in one call: V [H][P][S], u0 [H][P][m][S], M_V [H][S],
+        flags [H][P][S] (slot h = N - N_min), bit-identical to H calls of mpc_solve_batch."""
+        torch = self.torch
+        n, m = self.n, self.m
+        dA, dB = self._opt_dev(dA), self._opt_dev(dB)
+        if S is None:
+            S = dA.shape[-1] if dA is not None else (x0.shape[-1] if x0 is not None else 1)
+        if pts is None:
+            pts_d = None
+        elif isinstance(pts, torch.Tensor):
+            pts_d = self._dev(pts).reshape(-1, n)
+        else:
+            pts_d = self._dev(np.asarray(pts, dtype=np.float64).reshape(-1, n))
+        x0_d = self._opt_dev(x0)
+        P = pts_d.shape[0] if pts_d is not None else 1
+        H = int(N_max) - int(N_min) + 1
+        if H < 1:
+            raise ValueError("N_max < N_min")
+        out = {}
+        if "V" in want:
+            out["V"] = torch.empty((H, P, S), dtype=torch.float64, device=self.device)
+        if "u0" in want:
+            out["u0"] = torch.empty((H, P, m, S), dtype=torch.float64, device=self.device)
+        if "M_V" in want:
+            out["M_V"] = torch.empty((H, S), dtype=torch.float64, device=self.device)
+        if "flags" in want:
+            out["flags"] = torch.empty((H, P, S), dtype=torch.int32, device=self.device)
+        rc = self.lib.lqmpc_mpc_solve_range(self._h, S, _ptr(dA), _ptr(dB), int(N_min), int(N_max),
+                                            P if pts_d is not None else 0, _ptr(pts_d), _ptr(x0_d),
+                                            _ptr(out.get("V")), _ptr(out.get("u0")), _ptr(out.get("M_V")),
+                                            _ptr(out.get("flags")))
+        self._check(rc, "lqmpc_mpc_solve_range")
+        return out
+
+    @_streamed
     def simulate_batch(self, dA, dB, N: int, T: int, x0_shared=None, x0=None, S: Optional[int] = None,
                        want=("J_T", "flags", "n_active")):
         """Batched LQ_MPC_Simulator.simulate. x0_shared: (n,) one state for all samples, or x0: [n][S]."""
@@ -521,6 +562,82 @@ class Engine:
                                          _ptr(flags))
         self._check(rc, "lqmpc_bounds_batch")
         out = {k: detail[i] for i, k in enumerate(BOUND_FIELDS)}
+        out["flags"] = flags
+        if want_K:
+            out["K"] = K_out
+        if want_P:
+            out["P"] = P_out
+        return out
+
+    @_streamed
+    def bounds_range(self, dA, dB, N_min: int, N_max: int, e_A, e_B, M_V, x, p, V_expert: float, K=None,
+                     S: Optional[int] = None, bar_u: float = -1.0, bar_d_u: float = -1.0, strict_reference: bool = True,
+                     want_K=False, want_P=False, detail: bool = True):
+        """bounds_batch for every horizon N_min..N_max in one call. M_V: scalar, [S] (shared by every horizon) or
+        [H][S]. Returns [H][S] tensors per field (slot h = N - N_min) and flags [H][S]; K / P [..][S] once. With
+        detail=False only alpha, beta, xi, eta, bound and flags are produced (no [H][fields][S] table)."""
+        torch = self.torch
+        n, m = self.n, self.m
+        dA, dB = self._opt_dev(dA), self._opt_dev(dB)
+        if S is None:
+            S = dA.shape[-1] if dA is not None else 1
+        H = int(N_max) - int(N_min) + 1
+        if H < 1:
+            raise ValueError("N_max < N_min")
+
+        def per_sample(v, name, rows=1):
+            """scalar -> (None, v); [S] (or [rows][S]) -> contiguous device vector of rows * S entries."""
+            if np.isscalar(v) or (hasattr(v, "ndim") and v.ndim == 0):
+                return None, float(v)
+            t = self._dev(v)
+            if rows > 1 and t.numel() == S:                  # one [S] vector shared by every horizon
+                t = t.reshape(1, S).expand(rows, S).contiguous()
+            if t.numel() != rows * S:
+                raise ValueError("%s must be a scalar or hold %s entries, got %d"
+                                 % (name, "S = %d" % S if rows == 1 else "S or H * S = %d" % (rows * S), t.numel()))
+            return t.reshape(-1), 0.0
+
+        eA_d, eA_s = per_sample(e_A, "e_A")
+        eB_d, eB_s = per_sample(e_B, "e_B")
+        MV_d, MV_s = per_sample(M_V, "M_V", rows=H)
+        x_arr = x if isinstance(x, torch.Tensor) else np.asarray(x, dtype=np.float64)
+        x_sh = x_ps = None
+        if int(np.prod(x_arr.shape)) == n:
+            x_sh = self._dev(x_arr).reshape(n)
+        else:
+            x_ps = self._dev(x_arr).reshape(n, S)
+        K_sh = K_ps = None
+        if K is not None:
+            K_arr = K if isinstance(K, torch.Tensor) else np.asarray(K, dtype=np.float64)
+            if int(np.prod(K_arr.shape)) == m * n:
+                K_sh = self._dev(K_arr).reshape(m * n)
+            else:
+                K_ps = self._dev(K_arr).reshape(m * n, S)
+        NF = int(self.lib.lqmpc_bounds_fields())
+        assert NF == len(BOUND_FIELDS)
+        out = {}
+        if detail:
+            table = torch.empty((H, NF, S), dtype=torch.float64, device=self.device)
+            out.update({k: table[:, i] for i, k in enumerate(BOUND_FIELDS)})
+            ptrs = [None] * 5
+        else:
+            table = None
+            core = torch.empty((5, H, S), dtype=torch.float64, device=self.device)
+            for i, k in enumerate(("alpha", "beta", "xi", "eta", "bound")):
+                out[k] = core[i]
+            ptrs = [core[i] for i in range(5)]
+        flags = torch.empty((H, S), dtype=torch.int32, device=self.device)
+        K_out = torch.empty((m * n, S), dtype=torch.float64, device=self.device) if want_K else None
+        P_out = torch.empty((n * n, S), dtype=torch.float64, device=self.device) if want_P else None
+        p3 = _np_f64(p, (3,))
+        if getattr(self, "_poly_bar", None) is not None and (bar_u < 0.0 or bar_d_u < 0.0):
+            bar_u, bar_d_u = self._poly_bar
+        rc = self.lib.lqmpc_bounds_range(self._h, S, _ptr(dA), _ptr(dB), int(N_min), int(N_max), _ptr(eA_d),
+                                         _ptr(eB_d), eA_s, eB_s, _ptr(MV_d), MV_s, _ptr(x_sh), _ptr(x_ps), _ptr(K_ps),
+                                         _ptr(K_sh), _ptr(p3), float(V_expert), float(bar_u), float(bar_d_u),
+                                         int(bool(strict_reference)), *[_ptr(t) for t in ptrs], _ptr(table),
+                                         _ptr(K_out), _ptr(P_out), _ptr(flags))
+        self._check(rc, "lqmpc_bounds_range")
         out["flags"] = flags
         if want_K:
             out["K"] = K_out

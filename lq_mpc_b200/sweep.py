@@ -38,7 +38,7 @@ def _strided_columns(v, n_err):
 def error_horizon_sweep(engine, error_A, error_B, error_vec: Sequence[float], horizons: Sequence[int], F_u, Q,
                         N_points: int = 8, ext_radius_max: float = 1.5, p=(0.1, 1.0, 0.6), T: int = 30,
                         strict_reference: bool = True, group=None, keep_tables: bool = False,
-                        shard: Optional[tuple] = None, phase_times: bool = False):
+                        shard: Optional[tuple] = None, phase_times: bool = False, fused_horizons: bool = False):
     """Full error-level x horizon sweep on an engine whose TRUE problem (A, B, Q, R, box, N_opc) is already set.
 
     error_A (n,n,N_sys,n_err), error_B (n,m,N_sys,n_err): the reference's grid layout (numpy) — `shard` = (rank, world)
@@ -52,6 +52,12 @@ def error_horizon_sweep(engine, error_A, error_B, error_vec: Sequence[float], ho
       'evals', 'seconds' (device time of the sweep loop), and with keep_tables the raw [n_horizons][q][n_err][N_sys];
       with phase_times 'phase_seconds' = device time per kernel family over the whole sweep (CUDA events between the
       launches, read after the loop: no synchronisation is added).
+
+    fused_horizons=True evaluates the horizon axis with the range entry points: ONE mpc_solve_range over
+    min(horizons)..max(horizons) (one Riccati sweep per sample serves every horizon; the requested horizons are picked
+    from its [H] slots), the closed loops per horizon as before, and ONE bounds_range with the [H][S] M_V. Same keys,
+    same phase names; M_V and true_cost bit-equal to the default mode, the bound statistics within 1e-9 relative
+    (the Gram-spectrum search of the range stops at the same tolerance along a different path).
     """
     import torch
     n_err = len(error_vec)
@@ -96,16 +102,8 @@ def error_horizon_sweep(engine, error_A, error_B, error_vec: Sequence[float], ho
             ev = torch.cuda.Event(enable_timing=True)
             ev.record()
             marks.append(ev)
-    for h, N in enumerate(horizons):
-        N = int(N)
-        mark()
-        rs = engine.mpc_solve_batch(dA, dB, N, pts=ring, want=("M_V", "flags"))
-        mv = rs["M_V"]
-        mark()
-        sim = engine.simulate_batch(dA, dB, N, T, x0_shared=x_start_d, want=("J_T", "flags"))
-        mark()
-        b = engine.bounds_batch(dA, dB, N, e_per, e_per, mv, x_start_d, p, V_expert, strict_reference=strict_reference)
-        mark()
+
+    def reduce_horizon(rs_flags, mv, sim, b):
         cols = torch.cat([_strided_columns(v, n_err) for v in
                           (sim["J_T"], b["bound"], b["alpha"], b["beta"], b["xi"], b["eta"], mv)], dim=0)
         # K5 + the all-gather stay on the stream; the moments are read back ONCE after the loop (a .cpu() here would
@@ -114,13 +112,42 @@ def error_horizon_sweep(engine, error_A, error_B, error_vec: Sequence[float], ho
         bad = ((b["flags"] & (32 | 512)) != 0).to(torch.float64)       # BOUND_INVALID | DOMAIN_ERROR
         # incomplete solves (QP_MAXITER | DARE_NOCONV | LYAP_NOCONV | EIG_NOCONV | CHOL_FAIL) anywhere in the cell
         any_f = b["flags"] | sim["flags"]
-        for row in rs["flags"]:
+        for row in rs_flags:
             any_f = any_f | row
         fail = ((any_f & (4 | 8 | 64 | 128 | 256)) != 0).to(torch.float64)
         dev_counts.append(torch.stack([_strided_columns(bad, n_err).sum(dim=1),
                                        _strided_columns(fail, n_err).sum(dim=1)]))
         if keep_tables:
             tables.append(cols.reshape(len(QUANTITIES), n_err, N_sys).cpu().numpy())
+
+    if not fused_horizons:
+        for h, N in enumerate(horizons):
+            N = int(N)
+            mark()
+            rs = engine.mpc_solve_batch(dA, dB, N, pts=ring, want=("M_V", "flags"))
+            mv = rs["M_V"]
+            mark()
+            sim = engine.simulate_batch(dA, dB, N, T, x0_shared=x_start_d, want=("J_T", "flags"))
+            mark()
+            b = engine.bounds_batch(dA, dB, N, e_per, e_per, mv, x_start_d, p, V_expert,
+                                    strict_reference=strict_reference)
+            mark()
+            reduce_horizon(rs["flags"], mv, sim, b)
+    else:
+        N_lo, N_hi = int(min(horizons)), int(max(horizons))
+        pick = [int(N) - N_lo for N in horizons]                      # slots of the covering range
+        mark()
+        rs = engine.mpc_solve_range(dA, dB, N_lo, N_hi, pts=ring, want=("M_V", "flags"))
+        mark()
+        sims = [engine.simulate_batch(dA, dB, int(N), T, x0_shared=x_start_d, want=("J_T", "flags")) for N in horizons]
+        mark()
+        br = engine.bounds_range(dA, dB, N_lo, N_hi, e_per, e_per, rs["M_V"], x_start_d, p, V_expert,
+                                 strict_reference=strict_reference, detail=False)
+        mark()
+        for h, N in enumerate(horizons):
+            k = pick[h]
+            b = {q: br[q][k] for q in ("alpha", "beta", "xi", "eta", "bound", "flags")}
+            reduce_horizon(rs["flags"][k], rs["M_V"][k], sims[h], b)
     host_moments = torch.stack(dev_moments).cpu().numpy()              # [n_horizons][ranks][cols][6]
     host_counts = torch.stack(dev_counts).cpu().numpy()                # [n_horizons][2][n_err]
     mark()
