@@ -325,13 +325,21 @@ LQ_HD bool quartic_rho(double a, double b, double c, double d, double* rho_out) 
   return small_rem && (fprime * rho >= 4e-5) && (rho == rho);
 }
 
+// Characteristic polynomial of A / fro, fro = ||A||_F: x^4 + a x^3 + b x^2 + c x + d; for n = 3 it is the cubic times
+// x (d = 0), so x^3 + a x^2 + b x + c. The polynomial of A itself has the coefficients a fro, b fro^2, c fro^3, d fro^4.
+struct CharPoly {
+  double a, b, c, d, fro;
+};
+
+// Spectral radius from the characteristic polynomial; *cp receives that polynomial (all zero for the zero matrix).
 template <int n>
-LQ_HD bool spectral_radius_poly(const double* A, double* rho_out) {
+LQ_HD bool spectral_radius_poly(const double* A, double* rho_out, CharPoly* cp) {
   static_assert(n == 3 || n == 4, "closed-form path is for n = 3, 4");
   double ss = 0.0;
   LQ_UNROLL for (int i = 0; i < n * n; ++i) ss = fma(A[i], A[i], ss);
   if (!(ss > 1e-280 && ss < 1e280)) {
     *rho_out = 0.0;
+    cp->a = cp->b = cp->c = cp->d = cp->fro = 0.0;
     return ss == 0.0;                                   // the zero matrix; anything extreme goes to QR
   }
   const double is = rsqrt_pos(ss), fro = ss * is;
@@ -370,30 +378,48 @@ LQ_HD bool spectral_radius_poly(const double* A, double* rho_out) {
     c = -e3;
     d = det;
   }
+  cp->a = a; cp->b = b; cp->c = c; cp->d = d; cp->fro = fro;
   double rho;
   const bool ok = quartic_rho(a, b, c, d, &rho);
   *rho_out = rho * fro;
   return ok;
 }
 
+template <int n>
+LQ_HD bool spectral_radius_poly(const double* A, double* rho_out) {
+  CharPoly cp;
+  return spectral_radius_poly<n>(A, rho_out, &cp);
+}
+
 template <int n, bool kFast = (n == 3 || n == 4)>
 struct RhoFast {
+  static LQ_HD bool run(const double*, double*, CharPoly*) { return false; }
   static LQ_HD bool run(const double*, double*) { return false; }
 };
 template <int n>
 struct RhoFast<n, true> {
+  static LQ_HD bool run(const double* A, double* rho, CharPoly* cp) { return spectral_radius_poly<n>(A, rho, cp); }
   static LQ_HD bool run(const double* A, double* rho) { return spectral_radius_poly<n>(A, rho); }
 };
 
 // Spectral radius of a general real n x n matrix. *ok=false only if the QR fallback did not converge.
+// *cp_ok = true when the closed form (n = 3, 4) was accepted; *cp then holds the characteristic polynomial it used.
 template <int n>
-LQ_HD double spectral_radius(const double* A, bool* ok) {
+LQ_HD double spectral_radius(const double* A, bool* ok, CharPoly* cp, bool* cp_ok) {
   double rho;
-  if (RhoFast<n>::run(A, &rho)) {
+  *cp_ok = RhoFast<n>::run(A, &rho, cp);
+  if (*cp_ok) {
     *ok = true;
     return rho;
   }
   return spectral_radius_qr<n>(A, ok);
+}
+
+template <int n>
+LQ_HD double spectral_radius(const double* A, bool* ok) {
+  CharPoly cp;
+  bool cp_ok;
+  return spectral_radius<n>(A, ok, &cp, &cp_ok);
 }
 
 }  // namespace lq

@@ -41,7 +41,8 @@ struct DeviceSink {
 };
 
 // MINB = minimum resident CTAs per SM the register allocator must allow (occupancy vs. spills; see K1Tune below)
-template <int n, int m, int MINB, int THREADS = 128>
+// kLyapPoly: closed-loop cost from the characteristic polynomial where accepted (riccati.cuh, n = 3, 4)
+template <int n, int m, int MINB, int THREADS = 128, bool kLyapPoly = true>
 __global__ void __launch_bounds__(THREADS, MINB) eval_kernel(const __grid_constant__ lq::Problem<n, m> pb,
                                                          const __grid_constant__ EvalArgs a) {
   const int64_t s = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -54,12 +55,12 @@ __global__ void __launch_bounds__(THREADS, MINB) eval_kernel(const __grid_consta
 #pragma unroll
   for (int e = 0; e < n; ++e) x0[e] = ld_stream(a.x0 + (int64_t)e * a.ld + s);
   DeviceSink<n, m> sink{a, s};
-  lq::eval_sample<n, m>(pb, dA, dB, x0, a.N_min, a.N_max, a.T, a.Vn != nullptr, sink);
+  lq::eval_sample<n, m, DeviceSink<n, m>, kLyapPoly>(pb, dA, dB, x0, a.N_min, a.N_max, a.T, a.Vn != nullptr, sink);
 }
 
 // Same evaluation with the operands DRAWN IN THE KERNEL from the global sample index (sampler.cuh: seeded_sample):
 // no operand traffic at all — the fused "generate + evaluate" entry point north_star's Philox design implies.
-template <int n, int m, int MINB>
+template <int n, int m, int MINB, bool kLyapPoly = true>
 __global__ void __launch_bounds__(128, MINB) eval_seeded_kernel(const __grid_constant__ lq::Problem<n, m> pb,
                                                                 const __grid_constant__ EvalArgs a,
                                                                 const uint64_t seed, const int64_t first,
@@ -69,7 +70,7 @@ __global__ void __launch_bounds__(128, MINB) eval_seeded_kernel(const __grid_con
   double dA[n * n], dB[n * m], x0[n];
   lq::seeded_sample<n, m>(seed, first + s, e_A, e_B, dA, dB, x0);
   DeviceSink<n, m> sink{a, s};
-  lq::eval_sample<n, m>(pb, dA, dB, x0, a.N_min, a.N_max, a.T, a.Vn != nullptr, sink);
+  lq::eval_sample<n, m, DeviceSink<n, m>, kLyapPoly>(pb, dA, dB, x0, a.N_min, a.N_max, a.T, a.Vn != nullptr, sink);
 }
 
 template <int n, int m>
@@ -103,8 +104,14 @@ struct K1Tune {
   static constexpr int minb_nested = (n <= 4) ? 4 : 2;  // several horizons per sample
 };
 
-template <int n, int m>
-int launch_eval_t(lqmpc_ctx* ctx, const EvalArgs& a, cudaStream_t stream) {
+// LQMPC_K1_LYAP=doubling (n = 3, 4): the closed-loop cost by Lyapunov doubling for every sample (development A/B)
+bool k1_lyap_doubling() {
+  const char* v = getenv("LQMPC_K1_LYAP");
+  return v && v[0] == 'd';
+}
+
+template <int n, int m, bool kLyapPoly>
+int launch_eval_impl(lqmpc_ctx* ctx, const EvalArgs& a, cudaStream_t stream) {
   const lq::Problem<n, m>& pb = *reinterpret_cast<const lq::Problem<n, m>*>(ctx->pb);
   const int threads = 128;
   const int64_t blocks = (a.S + threads - 1) / threads;
@@ -126,25 +133,40 @@ int launch_eval_t(lqmpc_ctx* ctx, const EvalArgs& a, cudaStream_t stream) {
     constexpr int ts = (n <= 4) ? K1Tune<n, m>::threads_single : 128, mb = (n <= 4) ? K1Tune<n, m>::minb_single : 2;
     const int64_t bs = (a.S + ts - 1) / ts;
     if (bs > 0x7fffffffLL) return lq_set_error(ctx, LQMPC_EINVAL, "batch too large for one launch");
-    eval_kernel<n, m, mb, ts><<<(unsigned)bs, ts, 0, stream>>>(pb, a);
+    eval_kernel<n, m, mb, ts, kLyapPoly><<<(unsigned)bs, ts, 0, stream>>>(pb, a);
   } else
-    eval_kernel<n, m, K1Tune<n, m>::minb_nested><<<(unsigned)blocks, threads, 0, stream>>>(pb, a);
+    eval_kernel<n, m, K1Tune<n, m>::minb_nested, 128, kLyapPoly><<<(unsigned)blocks, threads, 0, stream>>>(pb, a);
   ctx->launches++;
   return lq_check_cuda(ctx, cudaGetLastError(), "eval_kernel launch");
 }
 
 template <int n, int m>
-int launch_eval_seeded_t(lqmpc_ctx* ctx, const EvalArgs& a, uint64_t seed, int64_t first, double e_A, double e_B) {
+int launch_eval_t(lqmpc_ctx* ctx, const EvalArgs& a, cudaStream_t stream) {
+  if constexpr (n == 3 || n == 4)
+    if (k1_lyap_doubling()) return launch_eval_impl<n, m, false>(ctx, a, stream);
+  return launch_eval_impl<n, m, true>(ctx, a, stream);
+}
+
+template <int n, int m, bool kLyapPoly>
+int launch_eval_seeded_impl(lqmpc_ctx* ctx, const EvalArgs& a, uint64_t seed, int64_t first, double e_A,
+                            double e_B) {
   const lq::Problem<n, m>& pb = *reinterpret_cast<const lq::Problem<n, m>*>(ctx->pb);
   const int threads = 128;
   const int64_t blocks = (a.S + threads - 1) / threads;
   if (blocks > 0x7fffffffLL) return lq_set_error(ctx, LQMPC_EINVAL, "batch too large for one launch");
   if (a.N_min == a.N_max)
-    eval_seeded_kernel<n, m, K1Tune<n, m>::minb_single><<<(unsigned)blocks, threads, 0, ctx->stream>>>(pb, a, seed, first, e_A, e_B);
+    eval_seeded_kernel<n, m, K1Tune<n, m>::minb_single, kLyapPoly><<<(unsigned)blocks, threads, 0, ctx->stream>>>(pb, a, seed, first, e_A, e_B);
   else
-    eval_seeded_kernel<n, m, K1Tune<n, m>::minb_nested><<<(unsigned)blocks, threads, 0, ctx->stream>>>(pb, a, seed, first, e_A, e_B);
+    eval_seeded_kernel<n, m, K1Tune<n, m>::minb_nested, kLyapPoly><<<(unsigned)blocks, threads, 0, ctx->stream>>>(pb, a, seed, first, e_A, e_B);
   ctx->launches++;
   return lq_check_cuda(ctx, cudaGetLastError(), "eval_seeded_kernel launch");
+}
+
+template <int n, int m>
+int launch_eval_seeded_t(lqmpc_ctx* ctx, const EvalArgs& a, uint64_t seed, int64_t first, double e_A, double e_B) {
+  if constexpr (n == 3 || n == 4)
+    if (k1_lyap_doubling()) return launch_eval_seeded_impl<n, m, false>(ctx, a, seed, first, e_A, e_B);
+  return launch_eval_seeded_impl<n, m, true>(ctx, a, seed, first, e_A, e_B);
 }
 
 template <int n, int m>

@@ -6,7 +6,8 @@
 //     from the finite-horizon Riccati recursion started at P (when no input bound is active).
 //   * closed loop on the TRUE plant (utils_class.py:277): x+ = (A + B K_0) x, cost accumulated as in
 //     utils_class.py:261,282-283; its T -> infinity limit is x0' S x0 with S the solution of the discrete Lyapunov
-//     equation S = W + Acl' S Acl, W = Q + K0' R K0, obtained here by squared doubling.
+//     equation S = W + Acl' S Acl, W = Q + K0' R K0. For n = 3, 4 the scalar x0' S x0 comes from the characteristic
+//     polynomial of Acl (lyapunov_cost_poly), elsewhere and where that is not accepted S is obtained by squared doubling.
 //   * stability check: spectral radius of the closed loop (utils.py:358 style eigvals + max|.|).
 //   * performance ratio: J / V_expert(x0), V_expert = x0' Pexp x0 the expert (true-model) optimal cost
 //     (utils_class.py:786) — Pexp is prepared once per problem on the device (prep kernel).
@@ -123,8 +124,85 @@ LQ_HD bool lyapunov_doubling(const double* Acl, const double* W, double* S) {
   return false;
 }
 
-// Closed-loop figures for one gain K on the true plant.
-template <int n, int m>
+// Smallest elimination pivot lyapunov_cost_poly accepts. Small pivots come with clustered or strongly non-normal
+// spectra and with rho near 1; calibrated on the host against a 50-digit Stein solve: with 1e-3 the worst accepted
+// relative error over those families is ~2.5e-12, without a threshold 1.2e-10 (tests/test_k1_closed_loop_cost.py).
+constexpr double kLyapPolyMinPivot = 1e-3;
+
+// J = x0' S x0 with S = W + Acl' S Acl (rho(Acl) < 1) from the characteristic polynomial of Acl, n = 3, 4, without S.
+// With x_k = Acl^k x0, c_ij = x_i' W x_j and gamma_d = sum_{k>=0} x_k' W x_{k+d} (J = gamma_0), Cayley-Hamilton gives
+// x_{k+n} = -sum_{r=1..n} a_r x_{k+n-r} (a_0 = 1); its inner product with x_{k+j} summed over k, j = 0..n, is
+//   sum_r a_r gamma_{|n-r-j|} = sum_r a_r sum_{i < min(j, n-r)} c_{i, i+|n-r-j|},
+// n + 1 equations in gamma_0..gamma_n that need only x_0..x_{n-1}. Taken in the order j = n..0 their first pivot is
+// a_0 = 1 and elimination needs no row swaps (in the order j = 0..n it would be det(Acl)). The result is accepted only
+// if every pivot exceeds kLyapPolyMinPivot in magnitude, J is finite and J >= c_00 + ... + c_{n-1,n-1}, the partial
+// sum S >= sum_{k<n} (Acl')^k W Acl^k guarantees; otherwise the caller runs lyapunov_doubling.
+template <int n>
+LQ_HD bool lyapunov_cost_poly(const CharPoly& cp, const double* Acl, const double* W, const double* x0, double* J) {
+  static_assert(n == 3 || n == 4, "characteristic-polynomial route is for n = 3, 4");
+  constexpr int n1 = n + 1;
+  const double f2 = cp.fro * cp.fro;
+  double al[n1];                                        // coefficients of the polynomial of Acl itself (unscaled)
+  al[0] = 1.0;
+  al[1] = cp.a * cp.fro;
+  al[2] = cp.b * f2;
+  al[3] = cp.c * (f2 * cp.fro);
+  if constexpr (n == 4) al[n] = cp.d * (f2 * f2);
+  double x[n * n], wx[n * n];                           // x[k*n + i] = (Acl^k x0)_i, wx[k*n + i] = (W x_k)_i
+  LQ_UNROLL for (int i = 0; i < n; ++i) x[i] = x0[i];
+  LQ_UNROLL for (int k = 1; k < n; ++k) mv<n, n>(Acl, x + (k - 1) * n, x + k * n);
+  LQ_UNROLL for (int k = 0; k < n; ++k) mv<n, n>(W, x + k * n, wx + k * n);
+  double c[n * n];                                      // c[i*n + j] = x_i' W x_j, i <= j
+  LQ_UNROLL for (int i = 0; i < n; ++i)
+    LQ_UNROLL for (int j = i; j < n; ++j) {
+      double acc = x[i * n] * wx[j * n];
+      LQ_UNROLL for (int e = 1; e < n; ++e) acc = fma(x[i * n + e], wx[j * n + e], acc);
+      c[i * n + j] = acc;
+    }
+  // row t is the equation j = n - t; columns are gamma_0..gamma_n. -0.0 is the additive identity the compiler folds.
+  double G[n1 * n1], h[n1];
+  LQ_UNROLL for (int t = 0; t < n1; ++t) {
+    const int j = n - t;
+    LQ_UNROLL for (int d = 0; d < n1; ++d) G[t * n1 + d] = -0.0;
+    h[t] = -0.0;
+    LQ_UNROLL for (int r = 0; r < n1; ++r) {
+      const int d = (n - r - j) < 0 ? (j + r - n) : (n - r - j);
+      G[t * n1 + d] += al[r];
+      const int lim = j < n - r ? j : n - r;
+      if (lim > 0) {
+        double s = c[d];
+        LQ_UNROLL for (int i = 1; i < lim; ++i) s += c[i * n + i + d];
+        h[t] = fma(al[r], s, h[t]);
+      }
+    }
+  }
+  double ip[n1];
+  bool piv_ok = true;
+  LQ_UNROLL for (int k = 0; k < n1; ++k) {
+    const double p = G[k * n1 + k];
+    piv_ok = piv_ok && (fabs(p) > kLyapPolyMinPivot);
+    ip[k] = rcp(p);
+    LQ_UNROLL for (int i = k + 1; i < n1; ++i) {
+      const double f = G[i * n1 + k] * ip[k];
+      LQ_UNROLL for (int col = k + 1; col < n1; ++col) G[i * n1 + col] = fma(-f, G[k * n1 + col], G[i * n1 + col]);
+      h[i] = fma(-f, h[k], h[i]);
+    }
+  }
+  double g[n1];
+  LQ_UNROLL for (int k = n1 - 1; k >= 0; --k) {
+    double s = h[k];
+    LQ_UNROLL for (int col = k + 1; col < n1; ++col) s = fma(-G[k * n1 + col], g[col], s);
+    g[k] = s * ip[k];
+  }
+  double psum = c[0];
+  LQ_UNROLL for (int i = 1; i < n; ++i) psum += c[i * n + i];
+  *J = g[0];
+  return piv_ok && fabs(g[0]) <= 1.79e308 && g[0] >= psum;
+}
+
+// Closed-loop figures for one gain K on the true plant. kLyapPoly (n = 3, 4): J from lyapunov_cost_poly where it is
+// accepted; false runs the doubling for every sample (the earlier path, kept as an A/B reference).
+template <int n, int m, bool kLyapPoly = true>
 LQ_HD void closed_loop_eval(const Problem<n, m>& pb, const double* K, const double* x0, int T,
                             double* J_inf, double* rho_out, double* J_T, int* flags) {
   double Acl[n * n], W[n * n], RK[m * n];
@@ -136,18 +214,24 @@ LQ_HD void closed_loop_eval(const Problem<n, m>& pb, const double* K, const doub
     }
   mm<m, m, n>(pb.R, K, RK);
   sym_add_mtm<m, n>(pb.Q, K, RK, W);
-  bool ok;
-  const double rho = spectral_radius<n>(Acl, &ok);
+  bool ok, cp_ok;
+  CharPoly cp;
+  const double rho = spectral_radius<n>(Acl, &ok, &cp, &cp_ok);
   if (!ok) *flags |= FLAG_EIG_NOCONV;
   *rho_out = rho;
   if (!(rho < 1.0)) {
     *flags |= FLAG_UNSTABLE;
     *J_inf = HUGE_VAL;
   } else {
-    double S[n * n];
-    if (!lyapunov_doubling<n>(Acl, W, S)) *flags |= FLAG_LYAP_NOCONV;
-    const double J = quad<n>(x0, S, x0);
-    if (!(fabs(J) <= 1.79e308)) *flags |= FLAG_NONFINITE;
+    double J;
+    bool fast = false;
+    if constexpr (kLyapPoly && (n == 3 || n == 4)) fast = cp_ok && lyapunov_cost_poly<n>(cp, Acl, W, x0, &J);
+    if (!fast) {
+      double S[n * n];
+      if (!lyapunov_doubling<n>(Acl, W, S)) *flags |= FLAG_LYAP_NOCONV;
+      J = quad<n>(x0, S, x0);
+      if (!(fabs(J) <= 1.79e308)) *flags |= FLAG_NONFINITE;
+    }
     *J_inf = J;
   }
   if (T > 0) {  // finite-T cost exactly as accumulated by utils_class.py:261,282-283
@@ -171,7 +255,7 @@ LQ_HD void closed_loop_eval(const Problem<n, m>& pb, const double* K, const doub
 }
 
 // Full per-sample evaluation over the nested horizons N_min..N_max. `sink(h, ...)` receives column h = N - N_min.
-template <int n, int m, class Sink>
+template <int n, int m, class Sink, bool kLyapPoly = true>
 LQ_HD void eval_sample(const Problem<n, m>& pb, const double* dA, const double* dB, const double* x0,
                        int N_min, int N_max, int T, bool want_vn, Sink& sink) {
   double Ah[n * n], Bh[n * m], P[n * n];
@@ -190,7 +274,7 @@ LQ_HD void eval_sample(const Problem<n, m>& pb, const double* dA, const double* 
     if (emit) {
       int flags = sticky;
       double J, rho, JT = 0.0;
-      closed_loop_eval<n, m>(pb, K, x0, T, &J, &rho, &JT, &flags);
+      closed_loop_eval<n, m, kLyapPoly>(pb, K, x0, T, &J, &rho, &JT, &flags);
       const double vn = want_vn ? quad<n>(x0, P, x0) : 0.0;
       sink(k - N_min, J, rho, J / v_exp, vn, JT, flags, K);
     }
