@@ -239,6 +239,31 @@ int lqmpc_column_sqdev(lqmpc_ctx* ctx, const double* table, int cols, int64_t S,
  * column; std = sqrt(M2 / count) as np.std (utils.py:898). Empty column: mean = M2 = NaN, max = -inf, min = +inf. */
 int lqmpc_column_moments(lqmpc_ctx* ctx, const double* table, int cols, int64_t S, int64_t ld, double* moments);
 
+/* Order statistics of the same tables, over the population the moments reduce: the entries with |x| <= 1.79e308
+ * ("finite" below; NaN, +-inf and the few doubles above 1.79e308 are left out), so the moments' count_finite is the
+ * count the ranks refer to.
+ * Exact selection by radix descent: a finite double x maps to the order-preserving key
+ *   key(x) = bits(x) ^ (x's sign bit set ? 0xFFFFFFFFFFFFFFFF : 0x8000000000000000)
+ * and the key of the entry of 0-based rank r among a column's finite entries is found one byte at a time, most
+ * significant first (pass 0), in 8 passes of histogram -> select. Multi-GPU: all-reduce `hist` with SUM between the
+ * two calls of every pass (lq_mpc_b200/stats.py); counts are integers, so every order of summation agrees.
+ *   lqmpc_column_radix_histogram : hist [cols][nsel][256] int64 = counts, by the byte of digit `pass`, of the finite
+ *     entries whose key agrees with prefix [cols][nsel] on the bytes above digit `pass`; 1 <= nsel <= 32.
+ *   lqmpc_column_radix_select    : for every (column, selector), the digit whose bucket holds rank[c][k]; the counts
+ *     of the buckets below it are subtracted from rank (in place) and the digit is written into prefix (in place).
+ *     Start with prefix = 0; after pass 7 prefix holds the key. A rank at or past the column's finite count leaves
+ *     rank and prefix unchanged.
+ *   lqmpc_column_argext : val [cols][2] = {max, min} of the finite entries, idx [cols][2] int64 = index_base + the
+ *     lowest position attaining each (index_base >= 0); a column without a finite entry gives -inf / +inf and -1.
+ * All pointers are device pointers; S = 0 is allowed (then `table` may be NULL). */
+#define LQMPC_RADIX_MAX_SEL 32
+int lqmpc_column_radix_histogram(lqmpc_ctx* ctx, const double* table, int cols, int64_t S, int64_t ld, int nsel,
+                                 int pass, const uint64_t* prefix, int64_t* hist);
+int lqmpc_column_radix_select(lqmpc_ctx* ctx, const int64_t* hist, int cols, int nsel, int pass, int64_t* rank,
+                              uint64_t* prefix);
+int lqmpc_column_argext(lqmpc_ctx* ctx, const double* table, int cols, int64_t S, int64_t ld, int64_t index_base,
+                        double* val, int64_t* idx);
+
 /* K6 — model-error grids generated on the device: the seeded, counter-based restatement of `random_matrix` /
  * `error_matrix_generator` (utils.py:779-847). For every error level i < n_err (bounds levels_host[i]) and perturbation
  * j in [j_first, j_first + N_sys): a rows x cols matrix with entries uniform in [-e, e], accepted when its Frobenius

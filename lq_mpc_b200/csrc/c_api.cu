@@ -737,6 +737,39 @@ int lqmpc_column_moments(lqmpc_ctx* ctx, const double* table, int cols, int64_t 
   return lq_launch_moments(ctx, table, cols, S, ld, moments);
 }
 
+int lqmpc_column_radix_histogram(lqmpc_ctx* ctx, const double* table, int cols, int64_t S, int64_t ld, int nsel,
+                                 int pass, const uint64_t* prefix, int64_t* hist) {
+  if (!ctx) return LQMPC_EINVAL;
+  if ((!table && S > 0) || !prefix || !hist || cols < 1 || S < 0 || ld < S)
+    return lq_set_error(ctx, LQMPC_EINVAL, "bad table/cols/S/ld/prefix/hist");
+  if (cols > 65535) return lq_set_error(ctx, LQMPC_EINVAL, "too many columns");
+  if (nsel < 1 || nsel > LQMPC_RADIX_MAX_SEL) return lq_set_error(ctx, LQMPC_EINVAL, "nsel outside 1..32");
+  if (pass < 0 || pass > 7) return lq_set_error(ctx, LQMPC_EINVAL, "pass outside 0..7");
+  cudaSetDevice(ctx->device);
+  return lq_launch_radix_hist(ctx, table, cols, S, ld, nsel, pass, prefix, hist);
+}
+
+int lqmpc_column_radix_select(lqmpc_ctx* ctx, const int64_t* hist, int cols, int nsel, int pass, int64_t* rank,
+                              uint64_t* prefix) {
+  if (!ctx) return LQMPC_EINVAL;
+  if (!hist || !rank || !prefix || cols < 1) return lq_set_error(ctx, LQMPC_EINVAL, "bad hist/rank/prefix/cols");
+  if (nsel < 1 || nsel > LQMPC_RADIX_MAX_SEL) return lq_set_error(ctx, LQMPC_EINVAL, "nsel outside 1..32");
+  if (pass < 0 || pass > 7) return lq_set_error(ctx, LQMPC_EINVAL, "pass outside 0..7");
+  cudaSetDevice(ctx->device);
+  return lq_launch_radix_select(ctx, hist, cols, nsel, pass, rank, prefix);
+}
+
+int lqmpc_column_argext(lqmpc_ctx* ctx, const double* table, int cols, int64_t S, int64_t ld, int64_t index_base,
+                        double* val, int64_t* idx) {
+  if (!ctx) return LQMPC_EINVAL;
+  if ((!table && S > 0) || !val || !idx || cols < 1 || S < 0 || ld < S)
+    return lq_set_error(ctx, LQMPC_EINVAL, "bad table/cols/S/ld/val/idx");
+  if (cols > 65535) return lq_set_error(ctx, LQMPC_EINVAL, "too many columns");
+  if (index_base < 0) return lq_set_error(ctx, LQMPC_EINVAL, "negative index_base");
+  cudaSetDevice(ctx->device);
+  return lq_launch_argext(ctx, table, cols, S, ld, index_base, val, idx);
+}
+
 int lqmpc_fp64_tensor_peak(lqmpc_ctx* ctx, double* tflops_out) {
   if (!ctx || !tflops_out) return LQMPC_EINVAL;
   cudaSetDevice(ctx->device);

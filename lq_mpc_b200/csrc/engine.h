@@ -166,6 +166,12 @@ int lq_launch_stats(lqmpc_ctx* ctx, const double* table, int cols, int64_t S, in
 int lq_launch_moments(lqmpc_ctx* ctx, const double* table, int cols, int64_t S, int64_t ld, double* out);
 int lq_launch_sqdev(lqmpc_ctx* ctx, const double* table, int cols, int64_t S, int64_t ld, const double* mean,
                     double* out);
+int lq_launch_radix_hist(lqmpc_ctx* ctx, const double* table, int cols, int64_t S, int64_t ld, int nsel, int pass,
+                         const uint64_t* prefix, int64_t* hist);
+int lq_launch_radix_select(lqmpc_ctx* ctx, const int64_t* hist, int cols, int nsel, int pass, int64_t* rank,
+                           uint64_t* prefix);
+int lq_launch_argext(lqmpc_ctx* ctx, const double* table, int cols, int64_t S, int64_t ld, int64_t index_base,
+                     double* val, int64_t* idx);
 bool lq_dyn_supported(int n, int m);
 int lq_dyn_set_problem(lqmpc_ctx* ctx, const double* A, const double* B, const double* Q, const double* R,
                        const double* P, const double* lo, const double* hi);

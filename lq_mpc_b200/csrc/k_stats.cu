@@ -273,3 +273,214 @@ int lq_launch_sqdev(lqmpc_ctx* ctx, const double* table, int cols, int64_t S, in
   ctx->launches += 2;
   return lq_check_cuda(ctx, cudaGetLastError(), "column sqdev launch");
 }
+
+// ---- exact order statistics by radix descent (lqmpc_column_radix_histogram / _select).
+// A finite double maps to an order-preserving uint64 key (negatives: all bits flipped; non-negatives: sign bit set),
+// so the key of the rank-r finite entry is found one 8-bit digit at a time, most significant first. Pass p counts, for
+// every (column, selector), the finite entries whose key agrees with the selector's prefix on the bits above digit p,
+// by their digit p. Counts are integers: the histogram is the same whatever the order of the atomics or the CTA count.
+namespace {
+
+constexpr int kRadixMaxSel = LQMPC_RADIX_MAX_SEL;   // 32 selectors x 256 bins x 4 B = 32 KB of shared memory
+
+__device__ __forceinline__ unsigned long long radix_key(double v) {
+  const unsigned long long b = static_cast<unsigned long long>(__double_as_longlong(v));
+  return (b >> 63) ? ~b : (b | 0x8000000000000000ull);
+}
+
+// grid = (nblk, cols), dynamic shared memory nuniq * 256 * 4 B. Selectors whose prefixes agree on the masked bits
+// have the same histogram: it is counted once (slot) and written to each of them.
+__global__ void __launch_bounds__(kThreads) radix_hist_kernel(const double* __restrict__ table, int64_t S,
+                                                              int64_t ld, int nblk, int nsel, int pass,
+                                                              const unsigned long long* __restrict__ prefix,
+                                                              unsigned long long* __restrict__ hist) {
+  extern __shared__ unsigned int sh[];
+  __shared__ unsigned long long pre[kRadixMaxSel];
+  __shared__ int slot[kRadixMaxSel];
+  __shared__ int nuniq;
+  const int c = blockIdx.y;
+  const double* col = table + (int64_t)c * ld;
+  const unsigned long long mask = pass ? (~0ull << (64 - 8 * pass)) : 0ull;
+  const int shift = 56 - 8 * pass;
+  if (threadIdx.x == 0) {
+    int u = 0;
+    for (int k = 0; k < nsel; ++k) {
+      const unsigned long long pk = prefix[(int64_t)c * nsel + k] & mask;
+      int s = -1;
+      for (int j = 0; j < u; ++j)
+        if (pre[j] == pk) { s = j; break; }
+      if (s < 0) { pre[u] = pk; s = u++; }
+      slot[k] = s;
+    }
+    nuniq = u;
+  }
+  __syncthreads();
+  const int nu = nuniq;
+  for (int i = threadIdx.x; i < nu * 256; i += kThreads) sh[i] = 0u;
+  __syncthreads();
+  auto count = [&](double v) {
+    if (!(fabs(v) <= 1.79e308)) return;
+    const unsigned long long key = radix_key(v);
+    const unsigned int d = (unsigned int)(key >> shift) & 255u;
+    for (int u = 0; u < nu; ++u)
+      if (((key ^ pre[u]) & mask) == 0ull) atomicAdd(&sh[u * 256 + d], 1u);
+  };
+  const int64_t per = ((S + nblk - 1) / nblk + 1) & ~(int64_t)1;
+  const int64_t lo = (int64_t)blockIdx.x * per;
+  int64_t hi = lo + per;
+  if (hi > S) hi = S;
+  if ((reinterpret_cast<uintptr_t>(col) & 15) == 0) {
+    const int64_t npair = (hi > lo) ? (hi - lo) / 2 : 0;
+    const double2* c2 = reinterpret_cast<const double2*>(col + lo);
+    for (int64_t i = threadIdx.x; i < npair; i += kThreads) {
+      const double2 v = __ldg(c2 + i);
+      count(v.x);
+      count(v.y);
+    }
+    if (threadIdx.x == 0 && hi > lo && ((hi - lo) & 1)) count(col[hi - 1]);
+  } else {
+    for (int64_t i = lo + threadIdx.x; i < hi; i += kThreads) count(col[i]);
+  }
+  __syncthreads();
+  for (int i = threadIdx.x; i < nsel * 256; i += kThreads) {
+    const unsigned int v = sh[slot[i >> 8] * 256 + (i & 255)];
+    if (v) atomicAdd(hist + ((int64_t)c * nsel) * 256 + i, (unsigned long long)v);
+  }
+}
+
+// one thread per (column, selector): the digit whose bucket holds the remaining rank; the counts below it leave the
+// rank, the digit joins the prefix. A rank outside the column (no finite entry) leaves both unchanged.
+__global__ void radix_select_kernel(const long long* __restrict__ hist, int cols, int nsel, int pass,
+                                    long long* __restrict__ rank, unsigned long long* __restrict__ prefix) {
+  const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= (int64_t)cols * nsel) return;
+  const long long* h = hist + t * 256;
+  const long long r = rank[t];
+  long long below = 0;
+  for (int d = 0; d < 256; ++d) {
+    const long long cnt = h[d];
+    if (r >= below && r < below + cnt) {
+      rank[t] = r - below;
+      prefix[t] |= (unsigned long long)d << (56 - 8 * pass);
+      return;
+    }
+    below += cnt;
+  }
+}
+
+// ---- arg-extremes: {max, min} of the finite entries with the lowest index attaining each.
+struct Arg {
+  double mx, mn;
+  long long imx, imn;   // -1: no finite entry yet
+};
+
+__device__ __forceinline__ Arg arg_merge(const Arg& a, const Arg& b) {
+  Arg r = a;
+  if (b.mx > a.mx || (b.mx == a.mx && b.imx >= 0 && (a.imx < 0 || b.imx < a.imx))) { r.mx = b.mx; r.imx = b.imx; }
+  if (b.mn < a.mn || (b.mn == a.mn && b.imn >= 0 && (a.imn < 0 || b.imn < a.imn))) { r.mn = b.mn; r.imn = b.imn; }
+  return r;
+}
+
+__device__ __forceinline__ void arg_acc(double v, long long i, Arg& p) {
+  if (fabs(v) <= 1.79e308) {   // entries arrive in increasing index order per thread: strict compares keep the first
+    if (v > p.mx) { p.mx = v; p.imx = i; }
+    if (v < p.mn) { p.mn = v; p.imn = i; }
+  }
+}
+
+__device__ __forceinline__ Arg arg_warp_fold(Arg p) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    Arg q;
+    q.mx = __shfl_xor_sync(0xffffffffu, p.mx, o); q.mn = __shfl_xor_sync(0xffffffffu, p.mn, o);
+    q.imx = __shfl_xor_sync(0xffffffffu, p.imx, o); q.imn = __shfl_xor_sync(0xffffffffu, p.imn, o);
+    p = arg_merge(p, q);
+  }
+  return p;
+}
+
+// grid = (nblk, cols); partial layout [cols][nblk] Arg
+__global__ void __launch_bounds__(kThreads) argext_partial_kernel(const double* __restrict__ table, int64_t S,
+                                                                 int64_t ld, int nblk, Arg* __restrict__ part) {
+  const int c = blockIdx.y;
+  const double* col = table + (int64_t)c * ld;
+  Arg p{-HUGE_VAL, HUGE_VAL, -1, -1};
+  const int64_t per = ((S + nblk - 1) / nblk + 1) & ~(int64_t)1;
+  const int64_t lo = (int64_t)blockIdx.x * per;
+  int64_t hi = lo + per;
+  if (hi > S) hi = S;
+  if ((reinterpret_cast<uintptr_t>(col) & 15) == 0) {
+    const int64_t npair = (hi > lo) ? (hi - lo) / 2 : 0;
+    const double2* c2 = reinterpret_cast<const double2*>(col + lo);
+    for (int64_t i = threadIdx.x; i < npair; i += kThreads) {
+      const double2 v = __ldg(c2 + i);
+      arg_acc(v.x, lo + 2 * i, p);
+      arg_acc(v.y, lo + 2 * i + 1, p);
+    }
+    if (threadIdx.x == 0 && hi > lo && ((hi - lo) & 1)) arg_acc(col[hi - 1], hi - 1, p);
+  } else {
+    for (int64_t i = lo + threadIdx.x; i < hi; i += kThreads) arg_acc(col[i], i, p);
+  }
+  p = arg_warp_fold(p);
+  __shared__ Arg sm[kThreads / 32];
+  if ((threadIdx.x & 31) == 0) sm[threadIdx.x >> 5] = p;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    Arg t = sm[0];
+    for (int w = 1; w < kThreads / 32; ++w) t = arg_merge(t, sm[w]);
+    part[(int64_t)c * nblk + blockIdx.x] = t;
+  }
+}
+
+// one warp per column -> val [cols][2] = {max, min}, idx [cols][2] (+ index_base; -1 for an empty column)
+__global__ void __launch_bounds__(32) argext_final_kernel(const Arg* __restrict__ part, int nblk, int64_t index_base,
+                                                         double* __restrict__ val, long long* __restrict__ idx) {
+  const int c = blockIdx.x;
+  Arg p{-HUGE_VAL, HUGE_VAL, -1, -1};
+  for (int b = threadIdx.x; b < nblk; b += 32) p = arg_merge(p, part[(int64_t)c * nblk + b]);
+  p = arg_warp_fold(p);
+  if (threadIdx.x == 0) {
+    val[2 * c] = p.mx;
+    val[2 * c + 1] = p.mn;
+    idx[2 * c] = p.imx >= 0 ? p.imx + index_base : -1;
+    idx[2 * c + 1] = p.imn >= 0 ? p.imn + index_base : -1;
+  }
+}
+
+}  // namespace
+
+int lq_launch_radix_hist(lqmpc_ctx* ctx, const double* table, int cols, int64_t S, int64_t ld, int nsel, int pass,
+                         const uint64_t* prefix, int64_t* hist) {
+  int rc = lq_check_cuda(ctx, cudaMemsetAsync(hist, 0, (size_t)cols * nsel * 256 * sizeof(int64_t), ctx->stream),
+                         "radix histogram clear");
+  if (rc || S == 0) return rc;
+  int nblk = pick_nblk(ctx, cols, S);
+  if ((S + nblk - 1) / nblk > ((int64_t)1 << 30)) nblk = (int)((S + ((int64_t)1 << 30) - 1) >> 30);  // uint32 bins
+  radix_hist_kernel<<<dim3(nblk, cols), kThreads, (size_t)nsel * 256 * sizeof(unsigned int), ctx->stream>>>(
+      table, S, ld, nblk, nsel, pass, reinterpret_cast<const unsigned long long*>(prefix),
+      reinterpret_cast<unsigned long long*>(hist));
+  ctx->launches += 1;
+  return lq_check_cuda(ctx, cudaGetLastError(), "column radix histogram launch");
+}
+
+int lq_launch_radix_select(lqmpc_ctx* ctx, const int64_t* hist, int cols, int nsel, int pass, int64_t* rank,
+                           uint64_t* prefix) {
+  const int64_t n = (int64_t)cols * nsel;
+  radix_select_kernel<<<(unsigned)((n + 127) / 128), 128, 0, ctx->stream>>>(
+      reinterpret_cast<const long long*>(hist), cols, nsel, pass, reinterpret_cast<long long*>(rank),
+      reinterpret_cast<unsigned long long*>(prefix));
+  ctx->launches += 1;
+  return lq_check_cuda(ctx, cudaGetLastError(), "column radix select launch");
+}
+
+int lq_launch_argext(lqmpc_ctx* ctx, const double* table, int cols, int64_t S, int64_t ld, int64_t index_base,
+                     double* val, int64_t* idx) {
+  const int nblk = pick_nblk(ctx, cols, S);
+  int rc = lq_reserve_ws(ctx, (size_t)cols * nblk * sizeof(Arg));
+  if (rc) return rc;
+  Arg* part = reinterpret_cast<Arg*>(ctx->ws);
+  argext_partial_kernel<<<dim3(nblk, cols), kThreads, 0, ctx->stream>>>(table, S, ld, nblk, part);
+  argext_final_kernel<<<cols, 32, 0, ctx->stream>>>(part, nblk, index_base, val, reinterpret_cast<long long*>(idx));
+  ctx->launches += 2;
+  return lq_check_cuda(ctx, cudaGetLastError(), "column argext launch");
+}

@@ -26,6 +26,8 @@ FLAG_EIG_NOCONV = 128
 FLAG_CHOL_FAIL = 256
 FLAG_DOMAIN_ERROR = 512
 
+RADIX_MAX_SEL = 32          # LQMPC_RADIX_MAX_SEL: selectors per lqmpc_column_radix_histogram call
+
 _c_double_p = ctypes.POINTER(ctypes.c_double)
 _c_int32_p = ctypes.POINTER(ctypes.c_int32)
 _vp = ctypes.c_void_p
@@ -65,6 +67,9 @@ ABI = {
     "lqmpc_column_stats": (_int, [_vp, _vp, _int, _i64, _i64, _vp]),
     "lqmpc_column_sqdev": (_int, [_vp, _vp, _int, _i64, _i64, _vp, _vp]),
     "lqmpc_column_moments": (_int, [_vp, _vp, _int, _i64, _i64, _vp]),
+    "lqmpc_column_radix_histogram": (_int, [_vp, _vp, _int, _i64, _i64, _int, _int, _vp, _vp]),
+    "lqmpc_column_radix_select": (_int, [_vp, _vp, _int, _int, _int, _vp, _vp]),
+    "lqmpc_column_argext": (_int, [_vp, _vp, _int, _i64, _i64, _i64, _vp, _vp]),
     "lqmpc_sample_error_grid": (_int, [_vp, ctypes.c_uint64, _int, _int, _int, _i64, _i64, _int, _vp, _i64, _int, _vp,
                                        _vp]),
     "lqmpc_fp64_peak": (_int, [_vp, _c_double_p]),
@@ -704,6 +709,53 @@ class Engine:
         self._check(self.lib.lqmpc_column_sqdev(self._h, _ptr(t), cols, S, S, _ptr(mean), _ptr(out)),
                     "lqmpc_column_sqdev")
         return out
+
+    def _table_view(self, table):
+        """[cols][S] table -> (tensor, cols, S, ld). A float64 CUDA tensor on this device whose rows are contiguous is
+        used in place (row stride = ld, storage offset kept), anything else is staged as a contiguous copy."""
+        torch = self.torch
+        t = table
+        if isinstance(t, torch.Tensor) and t.ndim == 1:
+            t = t.reshape(1, -1)
+        if not (isinstance(t, torch.Tensor) and t.device == self.device and t.dtype == torch.float64 and t.ndim == 2
+                and (t.stride(1) == 1 or t.shape[1] <= 1) and (t.shape[0] <= 1 or t.stride(0) >= t.shape[1])):
+            t = self._dev(table)
+            if t.ndim == 1:
+                t = t.reshape(1, -1)
+        cols, S = t.shape
+        return t, cols, S, (int(t.stride(0)) if cols > 1 else S)
+
+    @_streamed
+    def column_radix_histogram_raw(self, table, prefix, pass_: int):
+        """One radix pass (lqmpc_column_radix_histogram): prefix device int64 [cols][nsel] (the uint64 key prefixes,
+        nsel <= RADIX_MAX_SEL). Returns device int64 [cols][nsel][256]."""
+        torch = self.torch
+        t, cols, S, ld = self._table_view(table)
+        nsel = prefix.shape[1]
+        hist = torch.empty((cols, nsel, 256), dtype=torch.int64, device=self.device)
+        self._check(self.lib.lqmpc_column_radix_histogram(self._h, _ptr(t) if S else None, cols, S, ld, nsel,
+                                                          int(pass_), _ptr(prefix), _ptr(hist)),
+                    "lqmpc_column_radix_histogram")
+        return hist
+
+    @_streamed
+    def column_radix_select_raw(self, hist, pass_: int, rank, prefix):
+        """Digit pick of one radix pass (lqmpc_column_radix_select): updates rank and prefix [cols][nsel] in place."""
+        cols, nsel = rank.shape
+        self._check(self.lib.lqmpc_column_radix_select(self._h, _ptr(hist), cols, nsel, int(pass_), _ptr(rank),
+                                                       _ptr(prefix)), "lqmpc_column_radix_select")
+
+    @_streamed
+    def column_argext_raw(self, table, index_base: int = 0):
+        """Returns device (val [cols][2] = {max, min} of the finite entries, idx [cols][2] int64 = index_base + the
+        lowest position attaining each; -1 and -inf / +inf for a column without a finite entry)."""
+        torch = self.torch
+        t, cols, S, ld = self._table_view(table)
+        val = torch.empty((cols, 2), dtype=torch.float64, device=self.device)
+        idx = torch.empty((cols, 2), dtype=torch.int64, device=self.device)
+        self._check(self.lib.lqmpc_column_argext(self._h, _ptr(t) if S else None, cols, S, ld, int(index_base),
+                                                 _ptr(val), _ptr(idx)), "lqmpc_column_argext")
+        return val, idx
 
     # ------------------------------------------------------------------------------------------------ K6
     @_streamed

@@ -100,6 +100,18 @@ def device_error_grids(engine, n, m, error_vec, N_matrix, norm_type, seed=202405
     return (dA, dB, stats) if return_stats else (dA, dB)
 
 
+def perturbation_at(engine, seed, n, m, error_vec, N_matrix, norm_type, j, level):
+    """(dA (n, n), dB (n, m)) of global perturbation j at error level `level` of the grids `device_error_grids`
+    draws with the same arguments: K6 is counter-based, so drawing the single perturbation j (j_first=j, N_sys=1)
+    gives exactly the entries the full grid holds there. This maps an index reported by
+    `error_horizon_sweep(..., worst=True)` back to its sample."""
+    if not 0 <= j < 5 * N_matrix or not 0 <= level < len(error_vec):
+        raise ValueError("perturbation_at: j must be in [0, 5*N_matrix) and level in [0, len(error_vec))")
+    dA = engine.sample_error_grid(seed, 0, n, n, 1, error_vec, N_matrix, norm_type, j_first=int(j))
+    dB = engine.sample_error_grid(seed, 1, n, m, 1, error_vec, N_matrix, norm_type, j_first=int(j))
+    return (dA[:, level].cpu().numpy().reshape(n, n), dB[:, level].cpu().numpy().reshape(n, m))
+
+
 def grids_to_soa(error_A, error_B, level=None):
     """(n,n,N_sys,n_err), (n,m,N_sys,n_err) -> engine SoA [n*n][S], [n*m][S].
     level=None: every (system j, level i) pair, S = N_sys*n_err with s = j*n_err + i (the file's own C order);

@@ -38,7 +38,9 @@ def _strided_columns(v, n_err):
 def error_horizon_sweep(engine, error_A, error_B, error_vec: Sequence[float], horizons: Sequence[int], F_u, Q,
                         N_points: int = 8, ext_radius_max: float = 1.5, p=(0.1, 1.0, 0.6), T: int = 30,
                         strict_reference: bool = True, group=None, keep_tables: bool = False,
-                        shard: Optional[tuple] = None, phase_times: bool = False, fused_horizons: bool = False):
+                        shard: Optional[tuple] = None, phase_times: bool = False, fused_horizons: bool = False,
+                        quantiles: Optional[Sequence[float]] = None, worst: bool = False,
+                        j_first: Optional[int] = None):
     """Full error-level x horizon sweep on an engine whose TRUE problem (A, B, Q, R, box, N_opc) is already set.
 
     error_A (n,n,N_sys,n_err), error_B (n,m,N_sys,n_err): the reference's grid layout (numpy) — `shard` = (rank, world)
@@ -58,6 +60,17 @@ def error_horizon_sweep(engine, error_A, error_B, error_vec: Sequence[float], ho
     from its [H] slots), the closed loops per horizon as before, and ONE bounds_range with the [H][S] M_V. Same keys,
     same phase names; M_V and true_cost bit-equal to the default mode, the bound statistics within 1e-9 relative
     (the Gram-spectrum search of the range stops at the same tolerance along a different path).
+
+    Order statistics (opt-in; without them the sweep issues the same launches and returns the same values):
+      quantiles=(0.05, 0.5, 0.95) adds '<q>_quantile' [len(quantiles)][n_err][n_horizons] for q in QUANTITIES, equal
+        to np.quantile over the finite entries of each cell (see stats.column_quantiles), and 'quantiles'. The
+        per-horizon tables stay on the device ([n_horizons][q][n_err][N_sys] doubles) and ONE radix selection over
+        all their columns runs after the loop: one all-reduce per radix pass, whatever the number of horizons.
+      worst=True adds '<q>_argmax' / '<q>_argmin' [n_err][n_horizons] int64: the global perturbation index j (the
+        reference file's N_sys axis) attaining '<q>_max' / '<q>_min', lowest j on ties, -1 for a cell without a
+        finite entry. j_first = the global index of this rank's first perturbation: by default the shard's start for
+        numpy grids, 0 for device grids (pass the j_first given to `device_error_grids`). `sampling.perturbation_at`
+        regenerates the perturbation of a K6 grid from its index.
     """
     import torch
     n_err = len(error_vec)
@@ -72,6 +85,10 @@ def error_horizon_sweep(engine, error_A, error_B, error_vec: Sequence[float], ho
             lo, hi = _stats.shard_bounds(N_sys_all, shard[0], shard[1])
             error_A, error_B = error_A[:, :, lo:hi, :], error_B[:, :, lo:hi, :]
         N_sys = error_A.shape[2]
+        if j_first is None and shard is not None:
+            j_first = lo
+    if j_first is None:
+        j_first = 0
     # ---- nominal quantities (utils_class.py:757-764, 782-786)
     K_lqr = engine.dlqr_batch(S=1)["K"].cpu().numpy()[:, 0].reshape(-1, n)
     eps_lqr = local_radius(F_u, -K_lqr, Q)
@@ -90,7 +107,10 @@ def error_horizon_sweep(engine, error_A, error_B, error_vec: Sequence[float], ho
     n_invalid = np.zeros((n_err, len(horizons)))
     n_failed = np.zeros((n_err, len(horizons)))
     tables = [] if keep_tables else None
-    dev_moments, dev_counts = [], []
+    dev_moments, dev_counts, dev_argext = [], [], []
+    qs = _stats.check_quantiles(quantiles) if quantiles is not None else None
+    if qs is not None:                     # every horizon's table, kept for the one selection after the loop
+        qtab = torch.empty((len(horizons), len(QUANTITIES) * n_err, N_sys), dtype=torch.float64, device=engine.device)
     torch.cuda.synchronize(engine.device)
     t0 = time.perf_counter()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -103,9 +123,12 @@ def error_horizon_sweep(engine, error_A, error_B, error_vec: Sequence[float], ho
             ev.record()
             marks.append(ev)
 
-    def reduce_horizon(rs_flags, mv, sim, b):
-        cols = torch.cat([_strided_columns(v, n_err) for v in
-                          (sim["J_T"], b["bound"], b["alpha"], b["beta"], b["xi"], b["eta"], mv)], dim=0)
+    def reduce_horizon(h, rs_flags, mv, sim, b):
+        parts = [_strided_columns(v, n_err) for v in
+                 (sim["J_T"], b["bound"], b["alpha"], b["beta"], b["xi"], b["eta"], mv)]
+        cols = torch.cat(parts, dim=0) if qs is None else torch.cat(parts, dim=0, out=qtab[h])
+        if worst:
+            dev_argext.append(_stats.pack_argext(*engine.column_argext_raw(cols, j_first)))
         # K5 + the all-gather stay on the stream; the moments are read back ONCE after the loop (a .cpu() here would
         # drain the launch queue every horizon: ~0.4 ms of idle GPU per horizon, 5 % of the round-2 sweep)
         dev_moments.append(_stats.column_moments_device(engine, cols, group))
@@ -132,7 +155,7 @@ def error_horizon_sweep(engine, error_A, error_B, error_vec: Sequence[float], ho
             b = engine.bounds_batch(dA, dB, N, e_per, e_per, mv, x_start_d, p, V_expert,
                                     strict_reference=strict_reference)
             mark()
-            reduce_horizon(rs["flags"], mv, sim, b)
+            reduce_horizon(h, rs["flags"], mv, sim, b)
     else:
         N_lo, N_hi = int(min(horizons)), int(max(horizons))
         pick = [int(N) - N_lo for N in horizons]                      # slots of the covering range
@@ -147,9 +170,18 @@ def error_horizon_sweep(engine, error_A, error_B, error_vec: Sequence[float], ho
         for h, N in enumerate(horizons):
             k = pick[h]
             b = {q: br[q][k] for q in ("alpha", "beta", "xi", "eta", "bound", "flags")}
-            reduce_horizon(rs["flags"][k], rs["M_V"][k], sims[h], b)
+            reduce_horizon(h, rs["flags"][k], rs["M_V"][k], sims[h], b)
+    if qs is not None:
+        keys = _stats.column_quantile_keys(engine, qtab.view(-1, N_sys), qs,
+                                           torch.stack(dev_moments)[:, :, :, 2].sum(dim=1).reshape(-1), group)
+    if worst:
+        argext = _stats.gather_rows(torch.stack(dev_argext), group)  # [ranks][n_horizons][cols][4]
     host_moments = torch.stack(dev_moments).cpu().numpy()              # [n_horizons][ranks][cols][6]
     host_counts = torch.stack(dev_counts).cpu().numpy()                # [n_horizons][2][n_err]
+    if qs is not None:
+        host_keys = keys.cpu().numpy()
+    if worst:
+        host_argext = argext.cpu().numpy()
     mark()
     e1.record()
     torch.cuda.synchronize(engine.device)
@@ -176,6 +208,19 @@ def error_horizon_sweep(engine, error_A, error_B, error_vec: Sequence[float], ho
                 "ratio_true_max": res["true_cost_max"] / V_expert, "ratio_bound_max": res["bound_max"] / V_expert,
                 "evals": int(N_sys) * n_err * len(horizons), "seconds": e0.elapsed_time(e1) * 1e-3,
                 "wall_seconds": time.perf_counter() - t0})
+    n_q = len(QUANTITIES)
+    if qs is not None:
+        qv = _stats.finish_quantiles(host_keys, host_moments[:, :, :, 2].sum(axis=1).reshape(-1), qs)
+        qv = qv.reshape(len(qs), len(horizons), n_q, n_err)
+        for qi, q in enumerate(QUANTITIES):
+            res[q + "_quantile"] = np.ascontiguousarray(qv[:, :, qi, :].transpose(0, 2, 1))
+        res["quantiles"] = qs
+    if worst:
+        ax = _stats.merge_argext(host_argext.reshape(host_argext.shape[0], -1, 4))
+        for name in ("argmax", "argmin"):
+            a = ax[name].reshape(len(horizons), n_q, n_err)
+            for qi, q in enumerate(QUANTITIES):
+                res[q + "_" + name] = np.ascontiguousarray(a[:, qi, :].T)
     if keep_tables:
         res["tables"] = np.stack(tables)
     if phases is not None:
