@@ -17,7 +17,7 @@ LIB = os.path.join(LIBDIR, "liblqmpc_b200.so")
 SOURCES = ["c_api.cu", "k_eval.cu", "k_clqr.cu", "k_pclqr.cu", "k_bounds.cu", "k_stats.cu", "k_tiled.cu", "k_sampler.cu", "k_dyn.cu", "k_group.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xptxas", "-v", "--expt-relaxed-constexpr"]
-NVCC_FLAGS += os.environ.get("LQMPC_NVCC_EXTRA", "").split()     # development switches, e.g. -DLQ_K1_VARIANTS
+NVCC_FLAGS += os.environ.get("LQMPC_NVCC_EXTRA", "").split()     # development switches, e.g. -DLQ_K4_PROFILE
 
 
 def nvcc_path() -> str:

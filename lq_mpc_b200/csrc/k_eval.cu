@@ -94,7 +94,7 @@ __global__ void prepare_kernel(lq::Problem<n, m>* pb, int N_opc) {
 #endif
 template <int n, int m>
 struct K1Tune {
-  // measured on B200 (scripts/k1_probe.py and k1_sustained_probe.py, n=4 m=2, 1.25e7 samples). From a cold power state
+  // measured on B200 (n=4 m=2, 1.25e7 samples; DESIGN.md §5). From a cold power state
   // every budget ties for one horizon per sample (2 / 3 / 4 / 5 CTAs per SM: 3.50 / 3.61 / 3.55 / 3.51 ms), but the
   // kernel runs into the board's power cap and SUSTAINED the spill-free 255-register build wins clearly
   // (3.49 / 3.73 / 3.89 / 3.97 ms: spill traffic and the extra instructions cost power, i.e. clock). With all horizons
@@ -116,19 +116,6 @@ int launch_eval_impl(lqmpc_ctx* ctx, const EvalArgs& a, cudaStream_t stream) {
   const int threads = 128;
   const int64_t blocks = (a.S + threads - 1) / threads;
   if (blocks > 0x7fffffffLL) return lq_set_error(ctx, LQMPC_EINVAL, "batch too large for one launch");
-#ifdef LQ_K1_VARIANTS
-  if (n == 4 && m == 2) {   // development switch: occupancy experiments on the headline size
-    const char* v = getenv("LQMPC_K1_MINB");
-    const int mb = v ? atoi(v) : 0;
-    if (mb == 1) eval_kernel<n, m, 1><<<(unsigned)blocks, threads, 0, stream>>>(pb, a);
-    else if (mb == 3) eval_kernel<n, m, 3><<<(unsigned)blocks, threads, 0, stream>>>(pb, a);
-    else if (mb == 4) eval_kernel<n, m, 4><<<(unsigned)blocks, threads, 0, stream>>>(pb, a);
-    else if (mb == 5) eval_kernel<n, m, 5><<<(unsigned)blocks, threads, 0, stream>>>(pb, a);
-    else eval_kernel<n, m, 2><<<(unsigned)blocks, threads, 0, stream>>>(pb, a);
-    ctx->launches++;
-    return lq_check_cuda(ctx, cudaGetLastError(), "eval_kernel launch");
-  }
-#endif
   if (a.N_min == a.N_max) {
     constexpr int ts = (n <= 4) ? K1Tune<n, m>::threads_single : 128, mb = (n <= 4) ? K1Tune<n, m>::minb_single : 2;
     const int64_t bs = (a.S + ts - 1) / ts;
@@ -203,7 +190,8 @@ __global__ void __launch_bounds__(256) dfma_kernel(double* out, int iters, doubl
 }  // namespace
 
 int lq_launch_eval(lqmpc_ctx* ctx, const EvalArgs& a, cudaStream_t stream) {
-  if (lq_group_supported(ctx->n, ctx->m)) {   // n = 6, 8: lane-group kernel (k_group.cu); LQMPC_K1_GROUP=0: thread/sample
+  // n = 6, 8: lane-group kernel (k_group.cu) when LQMPC_K1_GROUP is unset; LQMPC_K1_GROUP=0: thread per sample
+  if (lq_group_supported(ctx->n, ctx->m)) {
     const char* v = getenv("LQMPC_K1_GROUP");
     if (!(v && v[0] == '0')) return lq_launch_eval_group(ctx, a, stream);
   }

@@ -10,7 +10,7 @@
 //     lanes of a group read the same address; the arenas of a warp's groups are staggered by 4 banks). The
 //     shared-memory return path moves 128 B per clock per SM whatever the broadcast, i.e. 16 doubles for 64 DFMA
 //     lanes: with R rows per lane a loaded double feeds R DFMAs, so R = 2 caps the FP64 pipe near one half and R = 4
-//     would lift the cap — but the unrolled R = 4 code overflows the instruction cache (measured, see the launcher);
+//     would lift the cap — but the unrolled R = 4 code overflows the instruction cache (measured, DESIGN.md §4);
 //   * A' X products read the left operand column-wise from the arena, so no transposed copy is kept; m x m and m x n
 //     quantities (G = R + B^'PB, its Cholesky factor, the gain) are reduced over the group with xor-shuffles and
 //     then REPLICATED in every lane, which keeps all control flow group-uniform; the gain and x0 live in the arena;
@@ -22,8 +22,6 @@
 // Loops whose trip count depends on the data (squarings, Lyapunov doubling) run to the warp's slowest group with
 // finished groups' state frozen, because the groups of a warp share __syncwarp and the shuffles.
 // Same evaluation, flags and outputs as riccati.cuh::eval_sample (the reference semantics are cited there).
-#include <stdlib.h>
-
 #include "engine.h"
 #include "sampler.cuh"
 
@@ -142,7 +140,7 @@ template <int n, int m, int L, bool NESTED>
 struct GroupLayout {
   static_assert(n % L == 0 && n % 2 == 0 && (n * m) % 2 == 0 && 32 % L == 0, "lane-group K1: n = L R, even sizes");
   static constexpr int R = n / L;
-  static constexpr int kThreads = (L == 2 && n >= 8) ? 64 : 128;   // arenas of a CTA stay below ~85 KB
+  static constexpr int kThreads = 128;
   static constexpr int kGroups = kThreads / L;
   // per-CTA constants (true plant and weights), then one arena per group
   static constexpr int oA = 0, oB = oA + n * n, oQ = oB + n * m, kConst = oQ + n * n;
@@ -699,16 +697,8 @@ int launch_group(lqmpc_ctx* ctx, const EvalArgs& a, cudaStream_t stream, const S
 bool lq_group_supported(int n, int m) { return (n == 8 && m == 2) || (n == 6 && m == 2); }
 
 int lq_launch_eval_group(lqmpc_ctx* ctx, const EvalArgs& a, cudaStream_t stream) {
-  if (ctx->n == 8 && ctx->m == 2) {
-    // measured on B200 (scripts/dims_probe.py 8 2 10 1e6): 4 lanes x 2 rows at 3 CTAs/SM (168 registers) 5.47 ms,
-    // at 2 CTAs/SM (254 registers, no spills) 5.97 ms; 2 lanes x 4 rows 6.19 ms (halves the shared-memory traffic per
-    // DFMA, but its unrolled code no longer fits the instruction cache: stall_no_instruction 3.2 per issue);
-    // thread per sample 18.3 ms. LQMPC_K1_GROUP = 2 / 4 select the other two builds (development A/B).
-    const char* v = getenv("LQMPC_K1_GROUP");
-    if (v && v[0] == '2') return launch_group<8, 2, 2, 2>(ctx, a, stream);
-    if (v && v[0] == '4') return launch_group<8, 2, 4, 2>(ctx, a, stream);
-    return launch_group<8, 2, 4, 3>(ctx, a, stream);
-  }
+  // n = 8: 4 lanes x 2 rows at 3 CTAs/SM, the fastest of the lane splits and register budgets measured (DESIGN.md §4)
+  if (ctx->n == 8 && ctx->m == 2) return launch_group<8, 2, 4, 3>(ctx, a, stream);
   if (ctx->n == 6 && ctx->m == 2) return launch_group<6, 2, 2, 2>(ctx, a, stream);
   return lq_set_error(ctx, LQMPC_EINVAL, "lane-group K1 is built for 6x2 and 8x2");
 }

@@ -8,7 +8,7 @@
 //     TMA engine (cp.async.bulk + mbarrier complete_tx); A^, P and the n x n temporaries live in shared memory
 //     (leading dimension n+4: the MMA fragment footprints hit the 32 banks with the minimum 2 wavefronts); every
 //     matrix product — n x n x n and the skinny n x 8 ones alike — is a set of warp-level FP64 tensor-core MMAs
-//     (mma.sync m8n8k4.f64 -> DMMA; a DFMA evaluation of the same fragments is kept for A/B timing).
+//     (mma.sync m8n8k4.f64 -> DMMA).
 //     The Riccati step is arranged so that the serial 8 x 8 Cholesky chain runs on ONE warp while the other three keep
 //     the tensor pipe busy:   P+ = Q + A^'P A^ - W W',  W = Z L^-T,  Z = A^'(P B^),  G = R + B^'P B^ = L L'
 //     — only W depends on the factorisation; X = P A^ and T = Q + A^'X (lower blocks, mirrored: P stays exactly
@@ -34,13 +34,6 @@ constexpr int kT = 128;
 #define LQ_K4_KUNROLL 8          // k-steps of a warp tile unrolled together: 1 / 2 / 4 / 8 measured 36.9 / 34.75 / 34.2 / 33.6 ms per 1.25e5 evals at 32 x 8 x 30
 #endif
 constexpr int kKUnroll = LQ_K4_KUNROLL;
-#ifndef LQ_K4_SPLIT1
-#define LQ_K4_SPLIT1 0           // single-tile products in two interleaved accumulator chains: measured SLOWER (34.0 vs 33.6 ms) — with 5 CTAs/SM the pipe, not the chain latency, is the limit
-#endif
-constexpr bool kSplitSkinny = (LQ_K4_SPLIT1 != 0);
-#ifndef LQ_K4_DMMA_DEFAULT
-#define LQ_K4_DMMA_DEFAULT true   // measured (DESIGN.md, K4): tensor-core MMAs beat the DFMA evaluation of the same tiles
-#endif
 
 // ------------------------------------------------------------------------------------------------ TMA / mbarrier
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -140,7 +133,7 @@ __device__ __forceinline__ void block_max_u32_sum(unsigned& a, double& t, unsign
 
 // ------------------------------------------------------------------------------------------------ warp-level MMA
 // Every matrix product of the Riccati step and of the Lyapunov doubling goes through ONE routine: a warp accumulates an
-// (8 MT) x (8 NT) block of C = A B as m8n8k4 FP64 tensor-core MMAs (DM = true: mma.sync -> DMMA), operands read
+// (8 MT) x (8 NT) block of C = A B as m8n8k4 FP64 tensor-core MMAs (mma.sync -> DMMA), operands read
 // straight from shared memory in fragment order:
 //     A fragment: lane (g = lane/4, tg = lane%4) holds A(row g, col tg)     B fragment: B(row tg, col g)
 //     C fragment: C(row g, cols 2 tg, 2 tg + 1)
@@ -148,58 +141,30 @@ __device__ __forceinline__ void block_max_u32_sum(unsigned& a, double& t, unsign
 // and 4 x 8 fragment footprints then map onto the 32 banks with exactly 2 wavefronts per 256-byte fragment, the
 // minimum. (Round-1 profile of the first version — 2 x 4 DFMA register tiles, leading dimension n + 2 — showed the
 // kernel bound by shared-memory wavefronts: 84 % of the LSU peak, 55 % of them bank conflicts.)
-// DM = false keeps a DFMA evaluation of the same fragments (each lane accumulates its two C entries) for A/B timing.
 __device__ __forceinline__ void dmma_m8n8k4(double& c0, double& c1, double a, double b) {
   asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};"
                : "+d"(c0), "+d"(c1)
                : "d"(a), "d"(b));
 }
 
-template <int MT, int NT, bool DM, class FA, class FB>
+template <int MT, int NT, class FA, class FB>
 __device__ __forceinline__ void warp_mma(int K, int r0, int c0, FA fa, FB fb, double (&c)[MT][NT][2]) {
   const int lane = threadIdx.x & 31, g = lane >> 2, tg = lane & 3;
 #pragma unroll
   for (int i = 0; i < MT; ++i)
 #pragma unroll
     for (int j = 0; j < NT; ++j) c[i][j][0] = c[i][j][1] = 0.0;
-  if (DM && MT * NT == 1 && kSplitSkinny) {
-    // one 8 x 8 output tile: its K / 4 MMAs would form ONE dependent chain (the skinny products P B^, Z, G — the last
-    // two sit on the chain warp's critical path). Two accumulators over alternating k-steps halve the chain.
-    double d0 = 0.0, d1 = 0.0;
 #pragma unroll kKUnroll
-    for (int k0 = 0; k0 < K; k0 += 8) {
-      const double a0 = fa(r0 + g, k0 + tg), b0 = fb(k0 + tg, c0 + g);
-      const double a1 = fa(r0 + g, k0 + 4 + tg), b1 = fb(k0 + 4 + tg, c0 + g);
-      dmma_m8n8k4(c[0][0][0], c[0][0][1], a0, b0);
-      dmma_m8n8k4(d0, d1, a1, b1);
-    }
-    c[0][0][0] += d0;
-    c[0][0][1] += d1;
-  } else if (DM) {
-#pragma unroll kKUnroll
-    for (int k0 = 0; k0 < K; k0 += 4) {
-      double av[MT], bv[NT];
+  for (int k0 = 0; k0 < K; k0 += 4) {
+    double av[MT], bv[NT];
 #pragma unroll
-      for (int i = 0; i < MT; ++i) av[i] = fa(r0 + 8 * i + g, k0 + tg);
+    for (int i = 0; i < MT; ++i) av[i] = fa(r0 + 8 * i + g, k0 + tg);
 #pragma unroll
-      for (int j = 0; j < NT; ++j) bv[j] = fb(k0 + tg, c0 + 8 * j + g);
+    for (int j = 0; j < NT; ++j) bv[j] = fb(k0 + tg, c0 + 8 * j + g);
 #pragma unroll
-      for (int i = 0; i < MT; ++i)
+    for (int i = 0; i < MT; ++i)
 #pragma unroll
-        for (int j = 0; j < NT; ++j) dmma_m8n8k4(c[i][j][0], c[i][j][1], av[i], bv[j]);
-    }
-  } else {
-    for (int k = 0; k < K; ++k) {
-#pragma unroll
-      for (int i = 0; i < MT; ++i) {
-        const double av = fa(r0 + 8 * i + g, k);
-#pragma unroll
-        for (int j = 0; j < NT; ++j) {
-          c[i][j][0] = fma(av, fb(k, c0 + 8 * j + 2 * tg), c[i][j][0]);
-          c[i][j][1] = fma(av, fb(k, c0 + 8 * j + 2 * tg + 1), c[i][j][1]);
-        }
-      }
-    }
+      for (int j = 0; j < NT; ++j) dmma_m8n8k4(c[i][j][0], c[i][j][1], av[i], bv[j]);
   }
 }
 
@@ -217,15 +182,15 @@ __device__ __forceinline__ void warp_mma_store(int r0, int c0, const double (&c)
 }
 
 // C = opA * B for n x n shared-memory operands (leading dimension LD), 4 warps, warp tile (n/2) x (n/2)
-template <int n, bool TA, bool DM, class Epi>
+template <int n, bool TA, class Epi>
 __device__ __forceinline__ void gemm_nn(const double* __restrict__ A, const double* __restrict__ B, Epi epi) {
   constexpr int LD = n + 4, T = n / 16;
   const int w = threadIdx.x >> 5;
   const int r0 = (w >> 1) * (n / 2), c0 = (w & 1) * (n / 2);
   double c[T][T][2];
-  warp_mma<T, T, DM>(n, r0, c0,
-                     [&](int i, int k) { return TA ? A[k * LD + i] : A[i * LD + k]; },
-                     [&](int k, int j) { return B[k * LD + j]; }, c);
+  warp_mma<T, T>(n, r0, c0,
+                 [&](int i, int k) { return TA ? A[k * LD + i] : A[i * LD + k]; },
+                 [&](int k, int j) { return B[k * LD + j]; }, c);
   warp_mma_store<T, T>(r0, c0, c, epi);
 }
 
@@ -289,7 +254,6 @@ __device__ __forceinline__ void z_ready_arrive() {
 }
 __device__ __forceinline__ void z_ready_wait() { asm volatile("bar.sync 1, %0;" ::"r"(kT) : "memory"); }
 
-// MB = CTAs per SM the register allocation is held to (5 -> <= 102 registers; shared memory fits 5 single-horizon CTAs)
 #ifdef LQ_K4_PROFILE
 // development build only: cycles per warp and phase (0 stage, 1 phase A, 2 phase B, 3 phase D, 4 closed loop,
 // 5 Lyapunov, 6 squarings, 7 hand-over / finish), accumulated in shared memory and added to a global table at exit
@@ -299,8 +263,9 @@ __device__ unsigned long long g_k4_prof[4 * 8];
 #define K4_PROF(idx) do { } while (0)
 #endif
 
-template <int n, int m, bool DM, int MB>
-__global__ void __launch_bounds__(kT, MB) tiled_eval_kernel(const TiledArgs a, const int nbig) {
+// register allocation held to 5 CTAs per SM (<= 102 registers): shared memory fits 5 single-horizon CTAs
+template <int n, int m>
+__global__ void __launch_bounds__(kT, 5) tiled_eval_kernel(const TiledArgs a, const int nbig) {
   using L = K4Smem<n, m>;
   using O = PbOff<n, m>;
   constexpr int LD = L::LD, NN = L::NN, LS = L::LS, M8 = L::M8, NW = n / 8, T = n / 16, HB = n / 2;
@@ -389,19 +354,19 @@ __global__ void __launch_bounds__(kT, MB) tiled_eval_kernel(const TiledArgs a, c
       // ---- phase A (all warps): P B^ (n x 8; warp w < n/8 owns row tile w) and X = P A^ (quadrants)
       if (w < NW) {
         double c[1][1][2];
-        warp_mma<1, 1, DM>(n, 8 * w, 0, [&](int i, int q) { return P[i * LD + q]; },
-                           [&](int q, int j) { return Bh[q * LS + j]; }, c);
+        warp_mma<1, 1>(n, 8 * w, 0, [&](int i, int q) { return P[i * LD + q]; },
+                       [&](int q, int j) { return Bh[q * LS + j]; }, c);
         warp_mma_store<1, 1>(8 * w, 0, c, [&](int i, int j, double v) { PB[i * LS + j] = v; });
       }
-      if (advance) gemm_nn<n, false, DM>(P, Ah, [&](int i, int j, double v) { X[i * LD + j] = v; });
+      if (advance) gemm_nn<n, false>(P, Ah, [&](int i, int j, double v) { X[i * LD + j] = v; });
       __syncthreads();
       K4_PROF(1);
       // ---- phase B: the chain warp factorises G while the workers form Z and the part of P+ that does not need it
       if (w == cw) {
         {
           double c[1][1][2];
-          warp_mma<1, 1, DM>(n, 0, 0, [&](int i, int q) { return Bh[q * LS + i]; },
-                             [&](int q, int j) { return PB[q * LS + j]; }, c);
+          warp_mma<1, 1>(n, 0, 0, [&](int i, int q) { return Bh[q * LS + i]; },
+                         [&](int q, int j) { return PB[q * LS + j]; }, c);
           warp_mma_store<1, 1>(0, 0, c, [&](int i, int j, double v) { G[i * LS + j] = Rs[i * LS + j] + v; });
         }
         __syncwarp();
@@ -466,8 +431,8 @@ __global__ void __launch_bounds__(kT, MB) tiled_eval_kernel(const TiledArgs a, c
         // Z = A^' (P B^): row tiles over the workers
         for (int t = widx; t < NW; t += 3) {
           double c[1][1][2];
-          warp_mma<1, 1, DM>(n, 8 * t, 0, [&](int i, int q) { return Ah[q * LD + i]; },
-                             [&](int q, int j) { return PB[q * LS + j]; }, c);
+          warp_mma<1, 1>(n, 8 * t, 0, [&](int i, int q) { return Ah[q * LD + i]; },
+                         [&](int q, int j) { return PB[q * LS + j]; }, c);
           warp_mma_store<1, 1>(8 * t, 0, c, [&](int i, int j, double v) { Z[i * LS + j] = v; });
         }
         z_ready_arrive();
@@ -475,8 +440,8 @@ __global__ void __launch_bounds__(kT, MB) tiled_eval_kernel(const TiledArgs a, c
         if (advance) {
           const int bi = (widx + 1) >> 1, bj = widx >> 1;            // (0,0), (1,0), (1,1)
           double c[T][T][2];
-          warp_mma<T, T, DM>(n, bi * HB, bj * HB, [&](int i, int q) { return Ah[q * LD + i]; },
-                             [&](int q, int j) { return X[q * LD + j]; }, c);
+          warp_mma<T, T>(n, bi * HB, bj * HB, [&](int i, int q) { return Ah[q * LD + i]; },
+                         [&](int q, int j) { return X[q * LD + j]; }, c);
           warp_mma_store<T, T>(bi * HB, bj * HB, c, [&](int i, int j, double v) {
             if (i >= j) {
               const double t = __ldg(gQ + i * n + j) + v;
@@ -492,8 +457,8 @@ __global__ void __launch_bounds__(kT, MB) tiled_eval_kernel(const TiledArgs a, c
       if (advance) {
         const int r0 = (w >> 1) * HB, c0 = (w & 1) * HB;
         double c[T][T][2];
-        warp_mma<T, T, DM>(M8, r0, c0, [&](int i, int q) { return PB[i * LS + q]; },
-                           [&](int q, int j) { return PB[j * LS + q]; }, c);
+        warp_mma<T, T>(M8, r0, c0, [&](int i, int q) { return PB[i * LS + q]; },
+                       [&](int q, int j) { return PB[j * LS + q]; }, c);
         warp_mma_store<T, T>(r0, c0, c, [&](int i, int j, double v) { P[i * LD + j] -= v; });
         __syncthreads();
         if (a.Pout && s == 0 && k == a.N_max) {            // problem preparation: the horizon-N cost-to-go itself
@@ -513,19 +478,19 @@ __global__ void __launch_bounds__(kT, MB) tiled_eval_kernel(const TiledArgs a, c
       // ---- closed loop on the TRUE plant: R K (8 x n), then A_cl = A + B K -> Mb, W = Q + K' R K -> Sb
       if (w < NW) {
         double c[1][1][2];
-        warp_mma<1, 1, DM>(M8, 0, 8 * w, [&](int i, int q) { return Rs[i * LS + q]; },
-                           [&](int q, int j) { return Kg[q * LD + j]; }, c);
+        warp_mma<1, 1>(M8, 0, 8 * w, [&](int i, int q) { return Rs[i * LS + q]; },
+                       [&](int q, int j) { return Kg[q * LD + j]; }, c);
         warp_mma_store<1, 1>(0, 8 * w, c, [&](int i, int j, double v) { RK[i * LD + j] = v; });
       }
       __syncthreads();
       {
         const int r0 = (w >> 1) * HB, c0 = (w & 1) * HB;
         double c[T][T][2];
-        warp_mma<T, T, DM>(M8, r0, c0, [&](int i, int q) { return (q < m) ? __ldg(gB + i * m + q) : 0.0; },
-                           [&](int q, int j) { return Kg[q * LD + j]; }, c);
+        warp_mma<T, T>(M8, r0, c0, [&](int i, int q) { return (q < m) ? __ldg(gB + i * m + q) : 0.0; },
+                       [&](int q, int j) { return Kg[q * LD + j]; }, c);
         warp_mma_store<T, T>(r0, c0, c, [&](int i, int j, double v) { Mb[i * LD + j] = __ldg(gA + i * n + j) + v; });
-        warp_mma<T, T, DM>(M8, r0, c0, [&](int i, int q) { return Kg[q * LD + i]; },
-                           [&](int q, int j) { return RK[q * LD + j]; }, c);
+        warp_mma<T, T>(M8, r0, c0, [&](int i, int q) { return Kg[q * LD + i]; },
+                       [&](int q, int j) { return RK[q * LD + j]; }, c);
         warp_mma_store<T, T>(r0, c0, c, [&](int i, int j, double v) { Sb[i * LD + j] = __ldg(gQ + i * n + j) + v; });
       }
       __syncthreads();
@@ -537,10 +502,10 @@ __global__ void __launch_bounds__(kT, MB) tiled_eval_kernel(const TiledArgs a, c
       unsigned* ru = reinterpret_cast<unsigned*>(red + 2 * (kT / 32));     // two groups of 2 * kT/32 unsigned
       int rp = 0;
       for (int it = 0; it < 64; ++it) {
-        gemm_nn<n, false, DM>(Sb, Mc, [&](int i, int j, double v) { Xc[i * LD + j] = v; });
+        gemm_nn<n, false>(Sb, Mc, [&](int i, int j, double v) { Xc[i * LD + j] = v; });
         __syncthreads();
         unsigned thi = 0, shi = 0;
-        gemm_nn<n, true, DM>(Mc, Xc, [&](int i, int j, double v) {
+        gemm_nn<n, true>(Mc, Xc, [&](int i, int j, double v) {
           const double nv = Sb[i * LD + j] + v;
           Sb[i * LD + j] = nv;
           thi = max(thi, hi_abs(v));
@@ -551,7 +516,7 @@ __global__ void __launch_bounds__(kT, MB) tiled_eval_kernel(const TiledArgs a, c
         if (hi_nonfinite(thi) || hi_nonfinite(shi)) { lflag = lq::FLAG_NONFINITE; nsq = it; break; }
         if (!(tmax > 1e-18 * smax)) { lflag = 0; nsq = it; break; }
         if (!(smax < 1e300)) { lflag = lq::FLAG_NONFINITE; nsq = it; break; }   // diverging (unstable loop)
-        gemm_nn<n, false, DM>(Mc, Mc, [&](int i, int j, double v) { Xc[i * LD + j] = v; });
+        gemm_nn<n, false>(Mc, Mc, [&](int i, int j, double v) { Xc[i * LD + j] = v; });
         __syncthreads();
         double* t = Mc; Mc = Xc; Xc = t;
       }
@@ -614,8 +579,8 @@ __global__ void __launch_bounds__(kT, MB) tiled_eval_kernel(const TiledArgs a, c
           {
             const int r0 = (w >> 1) * HB, c0 = (w & 1) * HB;
             double c[T][T][2];
-            warp_mma<T, T, DM>(n, r0, c0, [&](int i, int q) { return Mc[i * LD + q] * s2; },
-                               [&](int q, int j) { return Mc[q * LD + j]; }, c);
+            warp_mma<T, T>(n, r0, c0, [&](int i, int q) { return Mc[i * LD + q] * s2; },
+                           [&](int q, int j) { return Mc[q * LD + j]; }, c);
             warp_mma_store<T, T>(r0, c0, c, [&](int i, int j, double v) {
               Xc[i * LD + j] = v;
               lh = max(lh, hi_abs(v));
@@ -682,8 +647,8 @@ __global__ void __launch_bounds__(kT, MB) tiled_eval_kernel(const TiledArgs a, c
         // left to k4b: hand over A_cl = A + B K (rebuilt from the gain, the doubling consumed the shared-memory copy)
         const int r0 = (w >> 1) * HB, c0 = (w & 1) * HB;
         double c[T][T][2];
-        warp_mma<T, T, DM>(M8, r0, c0, [&](int i, int q) { return (q < m) ? __ldg(gB + i * m + q) : 0.0; },
-                           [&](int q, int j) { return Kg[q * LD + j]; }, c);
+        warp_mma<T, T>(M8, r0, c0, [&](int i, int q) { return (q < m) ? __ldg(gB + i * m + q) : 0.0; },
+                       [&](int q, int j) { return Kg[q * LD + j]; }, c);
         double* gout = a.Acl + o * (int64_t)(n * n);
         warp_mma_store<T, T>(r0, c0, c, [&](int i, int j, double v) { gout[i * n + j] = __ldg(gA + i * n + j) + v; });
         if (tid == 0) {
@@ -932,8 +897,6 @@ int launch_tiled_t(lqmpc_ctx* ctx, const TiledEval& t) {
   const int H = t.N_max - t.N_min + 1;
   const int nbig = (H > 1) ? 5 : 3;
   const size_t smem = k4a_smem_bytes<n, m>(nbig);
-  // FP64 tensor-core variant of the n x n x n products (n = 32): default decided by measurement (DESIGN.md, K4);
-  // LQMPC_K4_DMMA=0/1 overrides it for A/B runs.
   // spectral radius: repeated squaring inside k4a with the QR kernel as fallback (default), LQMPC_K4_RHO=qr: QR for all
   const char* rhov = getenv("LQMPC_K4_RHO");
   const int rho_qr = (rhov && rhov[0] == 'q') ? 1 : 0;
@@ -941,20 +904,10 @@ int launch_tiled_t(lqmpc_ctx* ctx, const TiledEval& t) {
   auto r_J = [](const TiledEval& tt, int64_t s0) { return tt.J ? tt.J + s0 : nullptr; };
   auto r_rho = [](const TiledEval& tt, int64_t s0) { return tt.rho ? tt.rho + s0 : nullptr; };
   auto r_ratio = [](const TiledEval& tt, int64_t s0) { return tt.ratio ? tt.ratio + s0 : nullptr; };
-  const char* dmv = getenv("LQMPC_K4_DMMA");
-  const bool use_dmma = dmv ? atoi(dmv) != 0 : LQ_K4_DMMA_DEFAULT;
-  // register budget: 5 CTAs/SM (<= 102 registers, what the single-horizon shared-memory plan admits) unless
-  // LQMPC_K4_OCC=4 asks for the 128-register build
-  const char* occv = getenv("LQMPC_K4_OCC");
-  const bool occ5 = occv ? atoi(occv) >= 5 : true;
-  using KernT = void (*)(const TiledArgs, const int);
-  KernT kerns[4] = {tiled_eval_kernel<n, m, false, 4>, tiled_eval_kernel<n, m, true, 4>,
-                    tiled_eval_kernel<n, m, false, 5>, tiled_eval_kernel<n, m, true, 5>};
-  KernT kern = kerns[(occ5 ? 2 : 0) + (use_dmma ? 1 : 0)];
+  const auto kern = tiled_eval_kernel<n, m>;
   static uint64_t attr_done = 0;                             // function attributes are per DEVICE: one bit each
   if (!((attr_done >> (ctx->device & 63)) & 1)) {
-    for (KernT kf : kerns)
-      cudaFuncSetAttribute(kf, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k4a_smem_bytes<n, m>(5));
+    cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k4a_smem_bytes<n, m>(5));
     cudaFuncSetAttribute(tiled_rho_kernel<n>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                          (int)((kT / 32) * (n * (n + 1) + 32) * sizeof(double)));
     attr_done |= (uint64_t)1 << (ctx->device & 63);

@@ -1,6 +1,5 @@
-"""Development probe (GPU box): K4 (n=32, m=8, N=30) parity vs the batched oracle + timing of the kernel variants:
-DFMA / DMMA products, 4 / 5 CTAs per SM, spectral radius by squaring (default) / by the QR kernel for every sample.
-Not part of the product."""
+"""Development probe (GPU box): K4 (n=32, m=8, N=30) parity vs the batched oracle + timing of the spectral-radius modes:
+by squaring (default) / by the QR kernel for every sample. Not part of the product."""
 import json, os, sys
 import numpy as np
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -23,9 +22,7 @@ bA = (torch.rand((S, n, n), device="cuda", dtype=torch.float64, generator=g) - 0
 bB = (torch.rand((S, n, m), device="cuda", dtype=torch.float64, generator=g) - 0.5) * 2e-3
 bx = torch.randn((S, n), device="cuda", dtype=torch.float64, generator=g)
 rho_by = {}
-for dm, occ, rho in (("1", "5", "sq"), ("1", "4", "sq"), ("1", "5", "qr"), ("1", "4", "qr"), ("0", "5", "sq")):
-    os.environ["LQMPC_K4_DMMA"] = dm
-    os.environ["LQMPC_K4_OCC"] = occ
+for rho in ("sq", "qr"):
     os.environ["LQMPC_K4_RHO"] = rho
     got = eng.eval_batch_tiled(dA, dB, x0, N, N)
     errs = {k: float(np.max(np.abs(got[k].cpu().numpy() - ref[k]) / np.abs(ref[k]))) for k in ("J", "rho", "ratio")}
@@ -43,7 +40,7 @@ for dm, occ, rho in (("1", "5", "sq"), ("1", "4", "sq"), ("1", "5", "qr"), ("1",
     res = {"parity": errs, "flags": np.unique(got["flags"].cpu().numpy()).tolist(), "S": S, "ms": ms,
            "evals_per_s": S / (ms * 1e-3), "unstable": int((r["flags"] & 1).sum()),
            "flags_big": np.unique(r["flags"].cpu().numpy()).tolist()}
-    tag = "dmma%s_occ%s_%s" % (dm, occ, rho)
+    tag = rho
     print(tag, json.dumps(res))
     out[tag] = res
 d = np.abs(rho_by["sq"] - rho_by["qr"]) / rho_by["qr"]

@@ -558,10 +558,10 @@ def test_warp_route_multi_sample_launch(engine, n, m):
 
 
 # ===================================================================================== C. host pipeline, every K1 build
-@pytest.mark.parametrize("n,m,group", [(n, m, None) for n, m in ALL_DIMS] + [(8, 2, "0"), (8, 2, "2"), (8, 2, "4"),
-                                                                            (6, 2, "0")])
+@pytest.mark.parametrize("n,m,group", [(n, m, None) for n, m in ALL_DIMS] + [(8, 2, "0"), (6, 2, "0")])
 def test_host_pipeline_every_k1_build(engine, n, m, group, monkeypatch):
-    """eval_batch_host at every compiled pair (the lane-group K1 at n = 6, 8 and its other builds via LQMPC_K1_GROUP),
+    """eval_batch_host at every compiled pair (the lane-group K1 at n = 6, 8, and its thread-per-sample alternative
+    via LQMPC_K1_GROUP=0),
     S = 3 chunks + 37 so that the last chunk is ragged (its leading dimension is the chunk, not its sample count),
     nested and single horizons: bit for bit the device-resident eval_batch."""
     import torch
