@@ -220,58 +220,116 @@ LQ_HD double spectral_radius_qr(const double* Ain, bool* ok) {
 // divisions per reflector) — 62 % of K1 in the round-1 profile.  For n <= 4 the spectrum is available in closed
 // form; what makes the closed form usable at 1e-9 parity is (i) Frobenius scaling so every coefficient is O(1),
 // (ii) coefficients from 2 x 2 minors (short sums, no powers of the matrix), (iii) Ferrari's factorisation used
-// only as the STARTING point of a Bairstow (Newton) refinement on the unmodified quartic, and (iv) an a-posteriori
-// acceptance test: remainder of the division ~ rounding level AND |p'(lambda*)| |lambda*| (the reciprocal
+// only as the STARTING point of a Bairstow (Newton) refinement on the unmodified quartic (so its resolvent cubic is
+// solved in float and polished once in double, and Bairstow stops once its update is negligible), and (iv) an
+// a-posteriori acceptance test: remainder of the division ~ rounding level AND |p'(lambda*)| |lambda*| (the reciprocal
 // condition number of the dominant root w.r.t. the coefficients) above a threshold that keeps the estimated
 // relative error of rho below ~1e-11.  Anything else falls back to the QR iteration, so the result is never
 // worse than before; typical closed loops (separated eigenvalues) take the fast path.
 // ---------------------------------------------------------------------------------------------------------------
 
+// Products the compiler may not fuse into a following addition. FMA contraction is decided per kernel instantiation,
+// and every K1 build (characteristic-polynomial or doubling closed-loop cost, one or several horizons) must round the
+// closed form identically: they report bit-identical rho. Host build: plain products (compiled without contraction).
+LQ_HD float fmul_nc(float a, float b) {
+#if defined(__CUDA_ARCH__)
+  return __fmul_rn(a, b);
+#else
+  return a * b;
+#endif
+}
+LQ_HD double dmul_nc(double a, double b) {
+#if defined(__CUDA_ARCH__)
+  return __dmul_rn(a, b);
+#else
+  return a * b;
+#endif
+}
+// sqrt_fast with the final product pinned the same way
+LQ_HD double sqrt_nc(double x) {
+#if defined(__CUDA_ARCH__)
+  return is_pos_normal(x) ? dmul_nc(x, rsqrt_pos(x)) : 0.0;
+#else
+  return sqrt(x);
+#endif
+}
+
 // max modulus of the roots of x^2 + p x + q, and (re, im >= 0) of the root attaining it
 LQ_HD double quad_rho(double p, double q, double* re, double* im, double* sq_abs_disc) {
   const double disc = fma(p, p, -4.0 * q);
-  const double sd = sqrt_fast(fabs(disc));
+  const double sd = sqrt_nc(fabs(disc));
   *sq_abs_disc = sd;
   if (disc < 0.0) {
     *re = -0.5 * p; *im = 0.5 * sd;
-    return sqrt_fast(fabs(q));
+    return sqrt_nc(fabs(q));
   }
   const double r = -0.5 * (p + dsign(sd, p));   // larger-magnitude root (no cancellation)
   *re = r; *im = 0.0;
   return fabs(r);
 }
 
-// largest real root of z^3 + A z^2 + B z + C (closed form + Newton polish)
-LQ_HD double cubic_largest_real_root(double A, double B, double C) {
-  const double third = 1.0 / 3.0;
-  const double A3 = A * third;
-  const double P = fma(-A, A3, B);                                  // B - A^2/3
-  const double Qc = fma(A3, fma(2.0 * A3, A3, -B), C);              // 2A^3/27 - AB/3 + C
-  const double hq = -0.5 * Qc, tp = P * third;
-  const double D = fma(hq, hq, tp * tp * tp);
-  double y;
-  if (D > 0.0) {
-    const double sD = sqrt_fast(D);
-    const double u = cbrt(hq + dsign(sD, hq));
-    y = (u != 0.0) ? u - tp / u : 0.0;
+// The resolvent cubic's root only seeds Ferrari's factor, which only seeds Bairstow, so the closed-form root is taken
+// in float (cbrt / acos / cos / divisions on the FP32 units, device: MUFU approximations without slow paths; host:
+// libm) and polished by one Newton step in double. Everything the result is judged by runs in double.
+LQ_HD float fsqrt0(float x) {                       // sqrt(x), 0 for x <= 0 and NaN
+#if defined(__CUDA_ARCH__)
+  return x > 0.0f ? fmul_nc(x, rsqrtf(x)) : 0.0f;
+#else
+  return x > 0.0f ? sqrtf(x) : 0.0f;
+#endif
+}
+LQ_HD float fdiv_approx(float x, float y) {
+#if defined(__CUDA_ARCH__)
+  return fmul_nc(x, __fdividef(1.0f, y));
+#else
+  return x / y;
+#endif
+}
+LQ_HD float fcos_approx(float x) {                  // |x| <= pi / 3 here
+#if defined(__CUDA_ARCH__)
+  return __cosf(x);
+#else
+  return cosf(x);
+#endif
+}
+
+// largest real root of z^3 + A z^2 + B z + C in float (closed form + Newton polish)
+LQ_HD float cubic_largest_real_root(float A, float B, float C) {
+  const float third = 1.0f / 3.0f;
+  const float A3 = fmul_nc(A, third);
+  const float P = fmaf(-A, A3, B);                                  // B - A^2/3
+  const float Qc = fmaf(A3, fmaf(2.0f * A3, A3, -B), C);            // 2A^3/27 - AB/3 + C
+  const float hq = -0.5f * Qc, tp = fmul_nc(P, third);
+  const float D = fmaf(hq, hq, tp * tp * tp);
+  float y;
+  if (D > 0.0f) {
+    const float sD = fsqrt0(D);
+    const float u = cbrtf(hq >= 0.0f ? hq + sD : hq - sD);
+    y = (u != 0.0f) ? u - fdiv_approx(tp, u) : 0.0f;
   } else {
-    const double t2 = -tp;                                          // >= 0 here
-    const double t = sqrt_fast(t2);
-    double arg = (t2 > 0.0) ? hq / (t2 * t) : 0.0;
-    arg = dmin(1.0, dmax(-1.0, arg));
-    y = 2.0 * t * cos(acos(arg) * third);
+    const float t2 = -tp;                                           // >= 0 here
+    const float t = fsqrt0(t2);
+    float arg = (t2 > 0.0f) ? fdiv_approx(hq, t2 * t) : 0.0f;
+    arg = fminf(1.0f, fmaxf(-1.0f, arg));
+    y = fmul_nc(2.0f * t, fcos_approx(acosf(arg) * third));
   }
-  double z = y - A3;
+  float z = y - A3;
   LQ_UNROLL for (int it = 0; it < 2; ++it) {
-    const double g = fma(fma(z + A, z, B), z, C);
-    const double dg = fma(fma(3.0, z, 2.0 * A), z, B);
-    if (dg > 1e-290) {                  // at the largest real root the slope is >= 0; never step on a flat spot
-      const double zn = fma(-g, rcp(dg), z);
+    const float g = fmaf(fmaf(z + A, z, B), z, C);
+    const float dg = fmaf(fmaf(3.0f, z, 2.0f * A), z, B);
+    if (dg > 1e-30f) {                  // at the largest real root the slope is >= 0; never step on a flat spot
+      const float zn = z - fdiv_approx(g, dg);
       z = (zn == zn) ? zn : z;
     }
   }
   return z;
 }
+
+// Bairstow stops once its update |dp| + |dq| is below kBairstowStep (quadratic convergence leaves ~1e-20 then), and
+// after kBairstowMaxSteps at most. Typical closed loops stop after one step; the cap serves slowly converging, nearly
+// repeated factors, which mostly fail the acceptance test anyway.
+constexpr double kBairstowStep = 1e-10;
+constexpr int kBairstowMaxSteps = 8;
 
 // Roots of x^4 + a x^3 + b x^2 + c x + d with all coefficients O(1) (scaled). Returns true and rho if trusted.
 LQ_HD bool quartic_rho(double a, double b, double c, double d, double* rho_out) {
@@ -280,36 +338,46 @@ LQ_HD bool quartic_rho(double a, double b, double c, double d, double* rho_out) 
   const double p = fma(-0.375, a2, b);
   const double q = fma(a, fma(0.125, a2, -0.5 * b), c);
   const double r = fma(a4, fma(a4, fma(-3.0 * a4, a4, b), -c), d);   // d - ac/4 + a^2 b/16 - 3a^4/256
-  // resolvent: z^3 + 2p z^2 + (p^2 - 4r) z - q^2, z = alpha^2 >= 0
-  const double B3 = fma(p, p, -4.0 * r);
-  double z = cubic_largest_real_root(2.0 * p, B3, -q * q);
+  // resolvent: z^3 + 2p z^2 + (p^2 - 4r) z - q^2, z = alpha^2 >= 0; float root, one Newton step in double
+  const double A = 2.0 * p, B3 = fma(p, p, -4.0 * r), C = -q * q;
+  double z = (double)cubic_largest_real_root((float)A, (float)B3, (float)C);
+  {
+    const double g = fma(fma(z + A, z, B3), z, C);
+    const double dg = fma(fma(3.0, z, 2.0 * A), z, B3);
+    if (dg > 1e-290) {
+      const double zn = fma(-g, rcp(dg), z);
+      z = (zn == zn) ? zn : z;
+    }
+  }
   z = dmax(z, 0.0);
-  const double alpha = sqrt_fast(z);
+  const double alpha = sqrt_nc(z);
   double w;                                                           // w = q / alpha, stable for alpha -> 0 too
-  if (z > 1e-6) w = q * rcp(alpha);
-  else w = dsign(sqrt_fast(dmax(fma(z, z + 2.0 * p, B3), 0.0)), q);
+  if (z > 1e-6) w = dmul_nc(q, rcp(alpha));
+  else w = dsign(sqrt_nc(dmax(fma(z, z + 2.0 * p, B3), 0.0)), q);
   const double beta = 0.5 * (p + z - w);
   // first factor in x: x^2 + p1 x + q1
   double p1 = fma(0.5, a, alpha);
   double q1 = fma(a4, a4 + alpha, beta);
-  double p2 = 0.0, q2 = 0.0, r1 = 0.0, r0 = 0.0;
   // Bairstow refinement of (p1, q1) on the original quartic; (p2, q2) is the quotient, (r1, r0) the remainder
-  LQ_UNROLL for (int it = 0; it < 4; ++it) {
-    p2 = a - p1;
-    q2 = b - fma(p1, p2, q1);
-    r1 = c - fma(p1, q2, q1 * p2);
-    r0 = fma(-q1, q2, d);
-    if (it == 3) break;
+  for (int it = 0; it < kBairstowMaxSteps; ++it) {
+    const double p2 = a - p1;
+    const double q2 = b - fma(p1, p2, q1);
+    const double r1 = c - fma(p1, q2, q1 * p2);
+    const double r0 = fma(-q1, q2, d);
     const double e = p1 - p2;
     const double j11 = fma(-p1, e, q1 - q2), j12 = e, j21 = -q1 * e, j22 = q1 - q2;
     const double det = fma(j11, j22, -j12 * j21);
-    if (det != 0.0) {
-      const double id = rcp(det);
-      const double dp = (fma(j22, r1, -j12 * r0)) * id;
-      const double dq = (fma(j11, r0, -j21 * r1)) * id;
-      p1 -= dp; q1 -= dq;
-    }
+    if (det == 0.0) break;
+    const double id = rcp(det);
+    const double dp = dmul_nc(fma(j22, r1, -j12 * r0), id);
+    const double dq = dmul_nc(fma(j11, r0, -j21 * r1), id);
+    p1 -= dp; q1 -= dq;
+    if (!(fabs(dp) + fabs(dq) > kBairstowStep)) break;   // converged (or NaN: the acceptance test rejects it)
   }
+  const double p2 = a - p1;
+  const double q2 = b - fma(p1, p2, q1);
+  const double r1 = c - fma(p1, q2, q1 * p2);
+  const double r0 = fma(-q1, q2, d);
   double re1, im1, sd1, re2, im2, sd2;
   const double rho1 = quad_rho(p1, q1, &re1, &im1, &sd1);
   const double rho2 = quad_rho(p2, q2, &re2, &im2, &sd2);
@@ -319,10 +387,11 @@ LQ_HD bool quartic_rho(double a, double b, double c, double d, double* rho_out) 
   const double dpq = first ? (p2 - p1) : (p1 - p2), dqq = first ? (q2 - q1) : (q1 - q2);
   const double re = first ? re1 : re2, im = first ? im1 : im2, sd = first ? sd1 : sd2;
   const double gr = fma(dpq, re, dqq), gi = dpq * im;
-  const double fprime = sd * sqrt_fast(fma(gr, gr, gi * gi));
+  // the conditioning product only meets a threshold, so float suffices for it (NaN fails the comparison)
+  const float fprime = (float)sd * fsqrt0((float)fma(gr, gr, gi * gi));
   *rho_out = rho;
   const bool small_rem = (fabs(r1) + fabs(r0)) <= 2e-14;
-  return small_rem && (fprime * rho >= 4e-5) && (rho == rho);
+  return small_rem && (fprime * (float)rho >= 4e-5f) && (rho == rho);
 }
 
 // Characteristic polynomial of A / fro, fro = ||A||_F: x^4 + a x^3 + b x^2 + c x + d; for n = 3 it is the cubic times
