@@ -1,4 +1,5 @@
-// k_eval.cu — K1: unconstrained certainty-equivalent MPC evaluation, one sample per thread (sm_100a).
+// k_eval.cu — K1: unconstrained certainty-equivalent MPC evaluation, one sample per thread; two per thread for
+// one-horizon launches at n <= 4 (sm_100a).
 //
 // Data movement: SoA operands, element e of sample s at ptr[e*ld + s]; a warp reads 32 consecutive samples of one
 // element (256 B, two full 128 B lines) with read-only, no-L1-allocate loads; every output is written the same way.
@@ -73,6 +74,108 @@ __global__ void __launch_bounds__(128, MINB) eval_seeded_kernel(const __grid_con
   lq::eval_sample<n, m, DeviceSink<n, m>, kLyapPoly>(pb, dA, dB, x0, a.N_min, a.N_max, a.T, a.Vn != nullptr, sink);
 }
 
+// ---- two samples per thread (one horizon, n <= 4). One sample per thread leaves the FP64 pipe about a third idle at 8
+// warps per SM: each Riccati step is a single dependency chain (PB -> G -> Cholesky -> solve -> P - YY' -> products).
+// Here a thread carries two samples through ONE straight-line Riccati loop body, so the scheduler always has a second
+// chain to issue from. Each sample runs eval_sample's operation sequence unchanged, so every output is bit-identical
+// to eval_kernel's. The closed loop runs once per sample in a loop that is not unrolled, with the sample's K and x0
+// picked by selects: one copy of its code (instruction cache) and no dynamically indexed array (local memory).
+constexpr int kPairThreads = 128;   // a CTA covers 2 * 128 consecutive samples: s0 = 256 b + t, s1 = s0 + 128
+
+template <int n, int m, bool kLyapPoly>
+__device__ __forceinline__ void eval_pair(const lq::Problem<n, m>& pb, const EvalArgs& a, int64_t s0, bool has1,
+                                          const double (&Ah)[2][n * n], const double (&Bh)[2][n * m],
+                                          const double (&x0)[2][n]) {
+  const int N = a.N_max;
+  const bool want_vn = a.Vn != nullptr;
+  double P[2][n * n], v_exp[2];
+  LQ_UNROLL for (int p = 0; p < 2; ++p) {
+    LQ_UNROLL for (int i = 0; i < n * n; ++i) P[p][i] = pb.Pt[i];
+    v_exp[p] = lq::quad<n>(x0[p], pb.Pexp, x0[p]);
+  }
+  lq::RicStage<n, m> st[2];
+  int sticky[2] = {0, 0};
+  for (int k = 1; k < N; ++k) {            // horizons 1..N-1: cost-to-go only
+    LQ_UNROLL for (int p = 0; p < 2; ++p) {
+      lq::riccati_factor<n, m>(P[p], Bh[p], pb.R, st[p]);
+      if (!st[p].ok) sticky[p] |= lq::FLAG_CHOL_FAIL;
+      lq::riccati_update<n, m>(st[p], Ah[p], pb.Q, P[p]);
+    }
+  }
+  double K[2][m * n], vn[2];
+  LQ_UNROLL for (int p = 0; p < 2; ++p) {  // horizon N: the gain, and the horizon-N cost-to-go only for Vn
+    lq::riccati_factor<n, m>(P[p], Bh[p], pb.R, st[p]);
+    if (!st[p].ok) sticky[p] |= lq::FLAG_CHOL_FAIL;
+    lq::riccati_gain<n, m>(st[p], Ah[p], K[p]);
+    if (want_vn) lq::riccati_update<n, m>(st[p], Ah[p], pb.Q, P[p]);
+    vn[p] = want_vn ? lq::quad<n>(x0[p], P[p], x0[p]) : 0.0;
+  }
+#pragma unroll 1
+  for (int p = 0; p < 2; ++p) {
+    const bool second = p != 0;
+    if (second && !has1) break;
+    double Kp[m * n], xp[n];
+    LQ_UNROLL for (int e = 0; e < m * n; ++e) Kp[e] = second ? K[1][e] : K[0][e];
+    LQ_UNROLL for (int i = 0; i < n; ++i) xp[i] = second ? x0[1][i] : x0[0][i];
+    int flags = second ? sticky[1] : sticky[0];
+    double J, rho, JT = 0.0;
+    lq::closed_loop_eval<n, m, kLyapPoly>(pb, Kp, xp, a.T, &J, &rho, &JT, &flags);
+    DeviceSink<n, m> sink{a, second ? s0 + kPairThreads : s0};
+    sink(0, J, rho, J / (second ? v_exp[1] : v_exp[0]), second ? vn[1] : vn[0], JT, flags, Kp);
+  }
+}
+
+// Tail: where s1 >= S the second slot runs the Riccati recursion on s0's operands and stores nothing.
+template <int n, int m, bool kLyapPoly>
+__global__ void __launch_bounds__(kPairThreads, 2) eval_pair_kernel(const __grid_constant__ lq::Problem<n, m> pb,
+                                                                    const __grid_constant__ EvalArgs a) {
+  const int64_t s0 = (int64_t)blockIdx.x * (2 * kPairThreads) + threadIdx.x;
+  if (s0 >= a.S) return;
+  const bool has1 = s0 + kPairThreads < a.S;
+  const int64_t s1 = has1 ? s0 + kPairThreads : s0;
+  double Ah[2][n * n], Bh[2][n * m], x0[2][n];
+  LQ_UNROLL for (int p = 0; p < 2; ++p) {
+    const int64_t s = p ? s1 : s0;
+    LQ_UNROLL for (int e = 0; e < n * n; ++e) Ah[p][e] = pb.A[e] + ld_stream(a.dA + (int64_t)e * a.ld + s);
+    LQ_UNROLL for (int e = 0; e < n * m; ++e) Bh[p][e] = pb.B[e] + ld_stream(a.dB + (int64_t)e * a.ld + s);
+    LQ_UNROLL for (int e = 0; e < n; ++e) x0[p][e] = ld_stream(a.x0 + (int64_t)e * a.ld + s);
+  }
+  eval_pair<n, m, kLyapPoly>(pb, a, s0, has1, Ah, Bh, x0);
+}
+
+// The seeded entry point with two samples per thread. The draws run in a loop that is not unrolled (one copy of the
+// Philox / Box-Muller code); after the first pass both slots hold s0's draw, so a tail thread skips the second. A^ and
+// B^ are formed inside the loop, right after the draw: there the compiler fuses e_A u + A into one FMA as it does in
+// eval_seeded_kernel, which keeps the two kernels bit-identical (across the loop boundary it could not).
+template <int n, int m, bool kLyapPoly>
+__global__ void __launch_bounds__(kPairThreads, 2) eval_pair_seeded_kernel(const __grid_constant__ lq::Problem<n, m> pb,
+                                                                           const __grid_constant__ EvalArgs a,
+                                                                           const uint64_t seed, const int64_t first,
+                                                                           const double e_A, const double e_B) {
+  const int64_t s0 = (int64_t)blockIdx.x * (2 * kPairThreads) + threadIdx.x;
+  if (s0 >= a.S) return;
+  const bool has1 = s0 + kPairThreads < a.S;
+  double Ah[2][n * n], Bh[2][n * m], x0[2][n];
+#pragma unroll 1
+  for (int p = 0; p < 2; ++p) {
+    if (p != 0 && !has1) break;
+    double tA[n * n], tB[n * m], tx[n];
+    lq::seeded_sample<n, m>(seed, first + s0 + (p != 0 ? kPairThreads : 0), e_A, e_B, tA, tB, tx);
+    LQ_UNROLL for (int e = 0; e < n * n; ++e) {
+      const double v = pb.A[e] + tA[e];
+      if (p == 0) Ah[0][e] = v;
+      Ah[1][e] = v;
+    }
+    LQ_UNROLL for (int e = 0; e < n * m; ++e) {
+      const double v = pb.B[e] + tB[e];
+      if (p == 0) Bh[0][e] = v;
+      Bh[1][e] = v;
+    }
+    LQ_UNROLL for (int e = 0; e < n; ++e) { if (p == 0) x0[0][e] = tx[e]; x0[1][e] = tx[e]; }
+  }
+  eval_pair<n, m, kLyapPoly>(pb, a, s0, has1, Ah, Bh, x0);
+}
+
 template <int n, int m>
 __global__ void prepare_kernel(lq::Problem<n, m>* pb, int N_opc) {
   if (threadIdx.x == 0 && blockIdx.x == 0) {
@@ -110,6 +213,13 @@ bool k1_lyap_doubling() {
   return v && v[0] == 'd';
 }
 
+// LQMPC_K1_PAIR=0: one sample per thread for one-horizon launches at n <= 4 too (the reference the tests compare the
+// two-sample kernels against, and the A/B)
+bool k1_pair() {
+  const char* v = getenv("LQMPC_K1_PAIR");
+  return !(v && v[0] == '0');
+}
+
 template <int n, int m, bool kLyapPoly>
 int launch_eval_impl(lqmpc_ctx* ctx, const EvalArgs& a, cudaStream_t stream) {
   const lq::Problem<n, m>& pb = *reinterpret_cast<const lq::Problem<n, m>*>(ctx->pb);
@@ -117,6 +227,13 @@ int launch_eval_impl(lqmpc_ctx* ctx, const EvalArgs& a, cudaStream_t stream) {
   const int64_t blocks = (a.S + threads - 1) / threads;
   if (blocks > 0x7fffffffLL) return lq_set_error(ctx, LQMPC_EINVAL, "batch too large for one launch");
   if (a.N_min == a.N_max) {
+    if constexpr (n <= 4)
+      if (k1_pair()) {
+        const int64_t bp = (a.S + 2 * kPairThreads - 1) / (2 * kPairThreads);
+        eval_pair_kernel<n, m, kLyapPoly><<<(unsigned)bp, kPairThreads, 0, stream>>>(pb, a);
+        ctx->launches++;
+        return lq_check_cuda(ctx, cudaGetLastError(), "eval_pair_kernel launch");
+      }
     constexpr int ts = (n <= 4) ? K1Tune<n, m>::threads_single : 128, mb = (n <= 4) ? K1Tune<n, m>::minb_single : 2;
     const int64_t bs = (a.S + ts - 1) / ts;
     if (bs > 0x7fffffffLL) return lq_set_error(ctx, LQMPC_EINVAL, "batch too large for one launch");
@@ -141,6 +258,13 @@ int launch_eval_seeded_impl(lqmpc_ctx* ctx, const EvalArgs& a, uint64_t seed, in
   const int threads = 128;
   const int64_t blocks = (a.S + threads - 1) / threads;
   if (blocks > 0x7fffffffLL) return lq_set_error(ctx, LQMPC_EINVAL, "batch too large for one launch");
+  if constexpr (n <= 4)
+    if (a.N_min == a.N_max && k1_pair()) {
+      const int64_t bp = (a.S + 2 * kPairThreads - 1) / (2 * kPairThreads);
+      eval_pair_seeded_kernel<n, m, kLyapPoly><<<(unsigned)bp, kPairThreads, 0, ctx->stream>>>(pb, a, seed, first, e_A, e_B);
+      ctx->launches++;
+      return lq_check_cuda(ctx, cudaGetLastError(), "eval_pair_seeded_kernel launch");
+    }
   if (a.N_min == a.N_max)
     eval_seeded_kernel<n, m, K1Tune<n, m>::minb_single, kLyapPoly><<<(unsigned)blocks, threads, 0, ctx->stream>>>(pb, a, seed, first, e_A, e_B);
   else
