@@ -40,6 +40,7 @@ extern "C" {
 #define LQMPC_FLAG_EIG_NOCONV 128
 #define LQMPC_FLAG_CHOL_FAIL 256
 #define LQMPC_FLAG_DOMAIN_ERROR 512
+#define LQMPC_FLAG_TAIL_UNCERTIFIED 1024
 
 typedef struct lqmpc_ctx lqmpc_ctx;
 
@@ -157,6 +158,25 @@ int lqmpc_set_input_polytope(lqmpc_ctx* ctx, int p, const double* F_u_host);
 int lqmpc_simulate_batch(lqmpc_ctx* ctx, int64_t S, const double* dA, const double* dB, int N, int T,
                          const double* x0_shared, const double* x0, double* J_T, double* X, double* U,
                          int32_t* flags, int32_t* n_active);
+
+/* K2c — infinite-horizon cost of the K2b closed loop, J_inf = lim_{T->inf} J_T, exact (no truncation) and certified.
+ * Inside the feasibility ellipsoid {x' P0 x <= c*} of the unconstrained N-stage plan the exact QP returns u = K0 x, so
+ * from there on the TRUE closed loop A + B K0 has cost matrix S = W + (A + B K0)' S (A + B K0), W = Q + K0' R K0. The
+ * level set {x' S x <= c_S}, c_S = (1 - 1e-9) c* / lambda_max(L^-1 P0 L^-T) (S = L L'), is invariant and lies inside
+ * the ellipsoid. The closed loop runs with the exact QP (box or installed polytope) until the first step tau <= T_max
+ * whose state is in that set: J_inf = sum_{t<tau} (x_t'Q x_t + u_t'R u_t) + x_tau' S x_tau.
+ *   J_inf [S], T_cert [S] (= tau), flags [S]: the OR of the plan, every step's solve, the tail and the bits below;
+ *   NULL = skip. Initial state as lqmpc_simulate_batch.
+ *   rho(A + B K0) >= 1: J_inf = +inf, T_cert = -1, LQMPC_FLAG_UNSTABLE (K1's convention; no simulation).
+ *   No certificate within T_max steps, or S not obtained / not positive definite (LQMPC_FLAG_LYAP_NOCONV where the
+ *   Lyapunov solve failed): J_inf = NaN, T_cert = -1, LQMPC_FLAG_TAIL_UNCERTIFIED. The certificate is sufficient, not
+ *   necessary: "uncertified" is no verdict of instability.
+ *   Without input bounds c* = +inf: T_cert = 0 and J_inf = x0' S x0, K1's J for the same horizon.
+ * Regulation only: LQMPC_EINVAL with references installed (the state does not converge to the origin), for
+ * T_max < 0, and unless exactly one of x0_shared / x0 is given. Not available on the tiled (n = 16 / 32) route. */
+int lqmpc_simulate_inf_batch(lqmpc_ctx* ctx, int64_t S, const double* dA, const double* dB, int N, int T_max,
+                             const double* x0_shared, const double* x0, double* J_inf, int32_t* T_cert,
+                             int32_t* flags);
 
 /* K3 — batched bound coefficients: LQ_RDP_Calculator.energy_decreasing (utils_class.py:344-373) and
  * .energy_bound (utils_class.py:308-342) with every helper they call (utils.py: local_radius, ex_stability_lq,

@@ -106,7 +106,7 @@ int pipe_abort(lqmpc_ctx* ctx, int rc) {
 
 extern "C" {
 
-int lqmpc_abi_version(void) { return 2; }
+int lqmpc_abi_version(void) { return 3; }
 
 const char* lqmpc_supported_dims(void) { return LQ_DIMS_STRING; }
 
@@ -596,6 +596,24 @@ int lqmpc_simulate_batch(lqmpc_ctx* ctx, int64_t S, const double* dA, const doub
   a.S = S; a.dA = dA; a.dB = dB; a.N = N; a.T = T; a.npts = 1; a.pts = x0_shared; a.x0 = x0;
   a.J_T = J_T; a.X = X; a.U = U; a.flags = flags; a.n_active = n_active;
   return ctx->dyn ? lq_dyn_mpc(ctx, a, true) : lq_launch_mpc(ctx, a, true);
+}
+
+int lqmpc_simulate_inf_batch(lqmpc_ctx* ctx, int64_t S, const double* dA, const double* dB, int N, int T_max,
+                             const double* x0_shared, const double* x0, double* J_inf, int32_t* T_cert,
+                             int32_t* flags) {
+  if (!ctx) return LQMPC_EINVAL;
+  if (!ctx->has_problem) return lq_set_error(ctx, LQMPC_ESTATE, "problem not set");
+  if (S < 0 || N < 1 || T_max < 0) return lq_set_error(ctx, LQMPC_EINVAL, "bad S/N/T_max");
+  if (S == 0) return LQMPC_OK;
+  if ((x0_shared == nullptr) == (x0 == nullptr))
+    return lq_set_error(ctx, LQMPC_EINVAL, "give exactly one of x0_shared / x0");
+  // with references the state does not converge to the origin and the reference's J_T does not subtract them
+  if (ctx->ref_ld > 0) return lq_set_error(ctx, LQMPC_EINVAL, "the infinite-horizon cost is for regulation (no references)");
+  cudaSetDevice(ctx->device);
+  MpcArgs a{};
+  a.S = S; a.dA = dA; a.dB = dB; a.N = N; a.T = T_max; a.npts = 1; a.pts = x0_shared; a.x0 = x0;
+  a.J_inf = J_inf; a.T_cert = T_cert; a.flags = flags;
+  return ctx->dyn ? lq_dyn_simulate_inf(ctx, a) : lq_launch_simulate_inf(ctx, a);
 }
 
 int lqmpc_bounds_fields(void) { return (int)lq::BF_COUNT; }

@@ -716,4 +716,105 @@ LQ_HD int simulate_sample(const Problem<n, m>& pb, const Plan<n, m>& pl, int N, 
   return flags;
 }
 
+// Infinite-horizon cost of the closed loop of simulate_sample (regulation only), exact and certified.
+// Inside the certificate ellipsoid E = {x' P0 x <= cstar} the exact solve returns u = K0 x (the unconstrained law), so
+// the tail is governed by the TRUE closed loop A_cl = A + B K0 with stage weight W = Q + K0' R K0 and cost matrix
+// S = W + A_cl' S A_cl. Along it x+' S x+ = x' S x - x' W x, so the level set {x' S x <= c_S} is invariant, and with
+// c_S = (1 - 1e-9) cstar / lambda_max(L^-1 P0 L^-T) (S = L L') it lies inside E: from the first t = tau whose state is
+// in it, the law is K0 x forever and the remaining cost is x_tau' S x_tau. Hence
+//     J_inf = sum_{t < tau} (x_t' Q x_t + u_t' R u_t) + x_tau' S x_tau = lim_{T -> inf} J_T,
+// with the exact QP (`solve(x, u)`, returns its flags) for the steps before tau. rho(A_cl) >= 1: J_inf = +inf and
+// FLAG_UNSTABLE (no simulation). No certificate within T_max steps, S not positive definite or not obtained: J_inf =
+// NaN, *T_cert = -1 and FLAG_TAIL_UNCERTIFIED — the certificate is sufficient, not necessary, so this is no verdict of
+// instability. cstar = +inf (no input bounds) certifies at tau = 0: J_inf = x0' S x0. `pl` holds P0 (and K0 where
+// Plan::kHoldK0; the workspace gains of plan_prepare otherwise).
+// inf_tail: S and c_S (NaN when there is no certificate: unstable, S not obtained or not positive definite, cstar < 0).
+template <int n, int m>
+LQ_HD int inf_tail(const Problem<n, m>& pb, const Plan<n, m>& pl, int N, double cstar, const WsView& ws, double* S,
+                   double* cS) {
+  const ClqrLayout<n, m> L(N);
+  double K0[m * n], Acl[n * n], W[n * n];
+  {
+    double RK[m * n];
+    LQ_UNROLL for (int e = 0; e < m * n; ++e) K0[e] = Plan<n, m>::kHoldK0 ? pl.K0[Plan<n, m>::kHoldK0 ? e : 0]
+                                                                           : ws[L.oKu + e];
+    LQ_UNROLL for (int i = 0; i < n; ++i)
+      LQ_UNROLL for (int j = 0; j < n; ++j) {
+        double acc = pb.A[i * n + j];
+        LQ_UNROLL for (int k = 0; k < m; ++k) acc = fma(pb.B[i * m + k], K0[k * n + j], acc);
+        Acl[i * n + j] = acc;
+      }
+    mm<m, m, n>(pb.R, K0, RK);
+    sym_add_mtm<m, n>(pb.Q, K0, RK, W);
+  }
+  int flags = 0;
+  *cS = NAN;
+  bool ok;
+  const double rho = spectral_radius<n>(Acl, &ok);
+  if (!ok) flags |= FLAG_EIG_NOCONV;
+  if (!(rho < 1.0)) return flags | FLAG_UNSTABLE;
+  if (!lyapunov_doubling<n>(Acl, W, S)) return flags | FLAG_LYAP_NOCONV;
+  // lambda_max(L^-1 P0 L^-T): two forward substitutions, Z = L^-1 P0, then L^-1 Z' (P0 symmetric)
+  double Lc[n * n], Lci[n], Z[n * n], M[n * n];
+  LQ_UNROLL for (int i = 0; i < n * n; ++i) { Lc[i] = S[i]; Z[i] = pl.P0[i]; }
+  if (!chol_inv<n>(Lc, Lci)) return flags;                             // S not positive definite
+  solve_l<n, n>(Lc, Z);
+  LQ_UNROLL for (int i = 0; i < n; ++i)
+    LQ_UNROLL for (int j = 0; j < n; ++j) M[i * n + j] = Z[j * n + i];
+  solve_l<n, n>(Lc, M);
+  LQ_UNROLL for (int i = 0; i < n; ++i)
+    LQ_UNROLL for (int j = i + 1; j < n; ++j) {
+      const double v = 0.5 * (M[i * n + j] + M[j * n + i]);
+      M[i * n + j] = v; M[j * n + i] = v;
+    }
+  double lmin, lmax;
+  sym_eig_minmax<n>(M, &lmin, &lmax);
+  if (lmax > 0.0 && cstar > 0.0) *cS = (1.0 - 1e-9) * cstar / lmax;   // cstar < 0: no certificate ellipsoid
+  return flags;
+}
+
+template <int n, int m, class Solve>
+LQ_HD int certified_closed_loop(const Problem<n, m>& pb, const Plan<n, m>& pl, int N, double cstar, int T_max,
+                                const double* x0, const WsView& ws, Solve solve, double* J_inf, int* T_cert) {
+  double S[n * n], cS;
+  int flags = inf_tail<n, m>(pb, pl, N, cstar, ws, S, &cS);
+  *T_cert = -1;
+  if (flags & FLAG_UNSTABLE) {
+    *J_inf = HUGE_VAL;
+    return flags;
+  }
+  *J_inf = NAN;
+  if (!(cS >= 0.0)) return flags | FLAG_TAIL_UNCERTIFIED;
+  double x[n], xn[n], u[m];
+  LQ_UNROLL for (int i = 0; i < n; ++i) x[i] = x0[i];
+  double cost = 0.0;
+  for (int t = 0;; ++t) {
+    const double v = quad<n>(x, S, x);
+    if (v <= cS) {
+      *J_inf = cost + v;
+      *T_cert = t;
+      return flags;
+    }
+    if (t >= T_max) break;
+    flags |= solve(x, u);
+    cost += quad<n>(x, pb.Q, x);
+    cost += quad<m>(u, pb.R, u);
+    step_model<n, m>(pb.A, pb.B, x, u, xn);
+    LQ_UNROLL for (int i = 0; i < n; ++i) x[i] = xn[i];
+  }
+  return flags | FLAG_TAIL_UNCERTIFIED;
+}
+
+// Infinite-horizon closed loop with the input box: plan_prepare's P0, K0 and cstar, clqr_solve for the steps before
+// the certificate. Returns the flags of the plan, of every solve and of the tail.
+template <int n, int m>
+LQ_HD int simulate_inf_sample(const Problem<n, m>& pb, Plan<n, m>& pl, int N, int T_max, const double* x0,
+                              const WsView& ws, double* J_inf, int* T_cert) {
+  const int pf = plan_prepare<n, m>(pb, pl, N, ws, /*certificate=*/true);
+  return pf | certified_closed_loop<n, m>(pb, pl, N, pl.cstar, T_max, x0, ws, [&](const double* x, double* u) {
+    double V;
+    return clqr_solve<n, m>(pb, pl, N, x, ws, u, &V);
+  }, J_inf, T_cert);
+}
+
 }  // namespace lq

@@ -1119,4 +1119,81 @@ __device__ __forceinline__ int dyn_clqr_solve(int lane, Arena& ar, const DynPb& 
   return flags;
 }
 
+// ------------------------------------------------------------------------------------------------ K2c pieces
+// Infinite-horizon closed loop (clqr.cuh: certified_closed_loop, run-time sizes).
+// Box feasibility certificate of the unconstrained plan (clqr.cuh: plan_prepare's cstar): a copy of P0 (big[4], as
+// dyn_plan_prepare leaves it; not modified) is factored as L D L' in big[6], the gains ws.Ku propagate Phi_k (big[2] /
+// big[3] / big[5]), and cstar = (1 - 1e-9) min_{k,j} b_j^2 / (g_{k,j} P0^-1 g_{k,j}'), g_k = K_k Phi_k. Returns +inf
+// without input bounds, -1 when P0 is not positive definite or the box does not hold the origin in its interior.
+// Needs an arena of 7; big[2], big[3], big[5], big[6], ar.xa, ar.xb, ar.Y and ar.T_mn are scratch.
+__device__ __forceinline__ double dyn_box_certificate(int lane, Arena& ar, const DynPb& pb, int N, const QpWs& ws) {
+  const int n = ar.n, m = ar.m, ld = ar.ld;
+  if (!pb.has_bounds) return HUGE_VAL;
+  double* Lp = ar.big[6];
+  wcopy(lane, n, n, ar.big[4], ld, Lp, ld);
+  bool ok = wldl(lane, n, Lp, ld, ar.xa, ar.xb);
+  for (int j = 0; j < m; ++j) ok = ok && (dmin(-pb.ulo[j], pb.uhi[j]) > 0.0);
+  if (!ok) return -1.0;
+  double* Phi = ar.big[2]; double* Acl = ar.big[3]; double* Pn = ar.big[5];
+  for (int e = lane; e < n * n; e += 32) { const int i = e / n, j = e - i * n; Phi[i * ld + j] = (i == j) ? 1.0 : 0.0; }
+  __syncwarp();
+  double cs = HUGE_VAL;
+  for (int k = 0; k < N; ++k) {
+    const double* K = ws.Ku + (size_t)k * m * n;
+    wgemm<false, false>(lane, m, n, n, K, n, Phi, ld, ar.T_mn, n);                     // g = K_k Phi_k (m x n)
+    if (lane < m) {                                        // y = L^-1 g_j' (unit L) in column j of ar.Y, q = y' D^-1 y
+      const double b = dmin(-pb.ulo[lane], pb.uhi[lane]);
+      double q = 0.0;
+      for (int i = 0; i < n; ++i) {
+        double acc = ar.T_mn[lane * n + i];
+        for (int c = 0; c < i; ++c) acc = fma(-Lp[i * ld + c], ar.Y[c * m + lane], acc);
+        ar.Y[i * m + lane] = acc;
+        q = fma(acc * ar.xa[i], acc, q);
+      }
+      if (b * b < 1e300 && q > 0.0) cs = dmin(cs, b * b / q);
+    }
+    __syncwarp();
+    if (k + 1 < N) {
+      wgemm<false, false>(lane, n, m, n, ar.Bh, m, K, n, Acl, ld, 1.0, ar.big[0], ld, 1.0);   // Ah + Bh K_k
+      wgemm<false, false>(lane, n, n, n, Acl, ld, Phi, ld, Pn, ld);
+      wcopy(lane, n, n, Pn, ld, Phi, ld);
+    }
+  }
+  cs = wmind(cs);
+  return (cs == cs) ? cs * (1.0 - 1e-9) : -1.0;
+}
+
+// Level c_S = (1 - 1e-9) cstar / lambda_max(L^-1 P0 L^-T) of the invariant set {x' S x <= c_S} (S = L L'), with P0
+// in big[1] and S in big[5]. Copies S to big[6] (kept for the closed loop: dyn_clqr_solve uses big[1..5]) and returns
+// NaN when S is not positive definite. With S = L D L' (unit L), the matrix is D^-1/2 L^-1 P0 L^-T D^-1/2; big[2..5]
+// are scratch.
+__device__ __forceinline__ double dyn_tail_level(int lane, Arena& ar, double cstar) {
+  const int n = ar.n, ld = ar.ld;
+  double* Ls = ar.big[5]; double* Z = ar.big[2]; double* M = ar.big[3]; const double* P0 = ar.big[1];
+  wcopy(lane, n, n, Ls, ld, ar.big[6], ld);
+  if (!wldl(lane, n, Ls, ld, ar.xa, ar.xb)) return NAN;
+  for (int c = lane; c < n; c += 32)                       // Z = L^-1 P0, lane = column
+    for (int i = 0; i < n; ++i) {
+      double acc = P0[i * ld + c];
+      for (int k = 0; k < i; ++k) acc = fma(-Ls[i * ld + k], Z[k * ld + c], acc);
+      Z[i * ld + c] = acc;
+    }
+  __syncwarp();
+  for (int c = lane; c < n; c += 32)                       // M = L^-1 Z', lane = column
+    for (int i = 0; i < n; ++i) {
+      double acc = Z[c * ld + i];
+      for (int k = 0; k < i; ++k) acc = fma(-Ls[i * ld + k], M[k * ld + c], acc);
+      M[i * ld + c] = acc;
+    }
+  __syncwarp();
+  for (int e = lane; e < n * n; e += 32) {                 // D^-1/2 (.) D^-1/2, symmetrised, into big[4]
+    const int i = e / n, j = e - i * n;
+    ar.big[4][i * ld + j] = 0.5 * (M[i * ld + j] + M[j * ld + i]) * sqrt(ar.xa[i] * ar.xa[j]);
+  }
+  __syncwarp();
+  const double lmax = wsym_extreme(lane, n, ar.big[4], ld, true, M, ld, ar.v);
+  __syncwarp();
+  return (lmax > 0.0 && cstar > 0.0) ? (1.0 - 1e-9) * cstar / lmax : NAN;
+}
+
 }  // namespace lqd

@@ -97,6 +97,8 @@ struct MpcArgs {
   int ref_ld = 0;
   const double* polyF = nullptr;   // filled by the polytope launcher (device, row-major [p][m])
   int polyP = 0;
+  double* J_inf = nullptr;         // infinite-horizon closed loop (lq_launch_simulate_inf, T = T_max): [S]
+  int32_t* T_cert = nullptr;       // [S]
 };
 
 struct BoundsArgs {
@@ -159,6 +161,8 @@ int lq_launch_dmma_peak(lqmpc_ctx* ctx, double* tflops);
 int lq_launch_mpc(lqmpc_ctx* ctx, const MpcArgs& a, bool simulate);
 int lq_launch_mpc_poly(lqmpc_ctx* ctx, const MpcArgs& a, bool simulate);
 int lq_launch_mpc_range(lqmpc_ctx* ctx, const MpcArgs& a);
+int lq_launch_simulate_inf(lqmpc_ctx* ctx, const MpcArgs& a);
+int lq_launch_simulate_inf_poly(lqmpc_ctx* ctx, const MpcArgs& a);
 int lq_launch_bounds(lqmpc_ctx* ctx, const BoundsArgs& a);
 bool lq_bounds_range_fused(lqmpc_ctx* ctx, const BoundsArgs& a);
 int lq_launch_bounds_range(lqmpc_ctx* ctx, const BoundsArgs& a);
@@ -178,6 +182,7 @@ int lq_dyn_set_problem(lqmpc_ctx* ctx, const double* A, const double* B, const d
 int lq_dyn_get_prepared(lqmpc_ctx* ctx, double* out);
 int lq_dyn_eval(lqmpc_ctx* ctx, const EvalArgs& a, cudaStream_t stream);
 int lq_dyn_mpc(lqmpc_ctx* ctx, MpcArgs a, bool simulate);
+int lq_dyn_simulate_inf(lqmpc_ctx* ctx, MpcArgs a);
 int lq_dyn_bounds(lqmpc_ctx* ctx, const BoundsArgs& a);
 int lq_dyn_dlqr(lqmpc_ctx* ctx, int64_t S, const double* dA, const double* dB, double* K, double* P, int32_t* flags);
 bool lq_tiled_supported(int n, int m);

@@ -19,3 +19,13 @@ int lq_launch_mpc_range(lqmpc_ctx* ctx, const MpcArgs& a) {
 #undef X
   return lq_set_error(ctx, LQMPC_EINVAL, "unsupported (n, m); see lqmpc_supported_dims()");
 }
+
+// Infinite-horizon closed loop (lqmpc_simulate_inf_batch): box here, the polytope family in k_pclqr.cu.
+int lq_launch_simulate_inf(lqmpc_ctx* ctx, const MpcArgs& a) {
+  if (ctx->poly_p > 0) return lq_launch_simulate_inf_poly(ctx, a);
+#define X(N_, M_) \
+  if (ctx->n == N_ && ctx->m == M_) return launch_simulate_inf_t<N_, M_, false>(ctx, a);
+  LQ_FOR_EACH_DIM(X)
+#undef X
+  return lq_set_error(ctx, LQMPC_EINVAL, "unsupported (n, m); see lqmpc_supported_dims()");
+}

@@ -153,6 +153,29 @@ __global__ void __launch_bounds__(128, K2Occupancy<n, m>::min_blocks) simulate_k
   }
 }
 
+// Infinite-horizon closed loop (clqr.cuh: certified_closed_loop): J_inf [S], T_cert [S], flags [S]; a.T = T_max.
+template <int n, int m, bool POLY>
+__global__ void __launch_bounds__(128, K2Occupancy<n, m>::min_blocks) simulate_inf_kernel(
+    const __grid_constant__ lq::Problem<n, m> pb, const __grid_constant__ MpcArgs a) {
+  const int64_t tid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  const int64_t nthreads = (int64_t)gridDim.x * blockDim.x;
+  const lq::WsView ws{a.ws + tid, nthreads};
+  for (int64_t s = tid; s < a.S; s += nthreads) {
+    lq::Plan<n, m> pl;
+    load_plan<n, m>(a, pb, s, pl);
+    double x0[n];
+#pragma unroll
+    for (int i = 0; i < n; ++i) x0[i] = a.pts ? a.pts[i] : a.x0[(int64_t)i * a.S + s];
+    double J;
+    int tc;
+    const int f = POLY ? lq::psimulate_inf_sample<n, m>(pb, pl, a.N, a.T, x0, lq::Poly{a.polyF, a.polyP}, ws, &J, &tc)
+                       : lq::simulate_inf_sample<n, m>(pb, pl, a.N, a.T, x0, ws, &J, &tc);
+    if (a.J_inf) a.J_inf[s] = J;
+    if (a.T_cert) a.T_cert[s] = tc;
+    if (a.flags) a.flags[s] = f;
+  }
+}
+
 template <int n, int m, bool POLY>
 int launch_mpc_t(lqmpc_ctx* ctx, MpcArgs a, bool sim) {
   const lq::Problem<n, m>& pb = *reinterpret_cast<const lq::Problem<n, m>*>(ctx->pb);
@@ -186,6 +209,32 @@ int launch_mpc_t(lqmpc_ctx* ctx, MpcArgs a, bool sim) {
     mpc_solve_kernel<n, m, POLY><<<(unsigned)blocks, threads, 0, ctx->stream>>>(pb, a);
   ctx->launches++;
   return lq_check_cuda(ctx, cudaGetLastError(), sim ? "simulate_kernel launch" : "mpc_solve_kernel launch");
+}
+
+// The grid cap and workspace sizing of launch_mpc_t; the caller has rejected references.
+template <int n, int m, bool POLY>
+int launch_simulate_inf_t(lqmpc_ctx* ctx, MpcArgs a) {
+  const lq::Problem<n, m>& pb = *reinterpret_cast<const lq::Problem<n, m>*>(ctx->pb);
+  int sms = 148;
+  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, ctx->device);
+  const int threads = 128;
+  int64_t blocks = (a.S + threads - 1) / threads;
+  int occ = 0;
+  cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, simulate_inf_kernel<n, m, POLY>, threads, 0);
+  if (occ < 1) occ = 1;
+  int waves = (a.N >= 20) ? 1 : 3;
+  if (const char* wv = getenv("LQMPC_K2_WAVES")) { if (atoi(wv) > 0) waves = atoi(wv); }
+  const int64_t cap = (int64_t)sms * occ * waves;
+  if (blocks > cap) blocks = cap;
+  const int64_t nthreads = blocks * threads;
+  const int64_t per = lq::clqr_ws_doubles<n, m>(a.N);
+  int rc = lq_reserve_ws(ctx, (size_t)(per * nthreads) * sizeof(double));
+  if (rc) return rc;
+  a.ws = reinterpret_cast<double*>(ctx->ws);
+  if (POLY) { a.polyF = ctx->poly_dev; a.polyP = ctx->poly_p; }
+  simulate_inf_kernel<n, m, POLY><<<(unsigned)blocks, threads, 0, ctx->stream>>>(pb, a);
+  ctx->launches++;
+  return lq_check_cuda(ctx, cudaGetLastError(), "simulate_inf_kernel launch");
 }
 
 template <int n, int m>

@@ -221,6 +221,61 @@ __global__ void __launch_bounds__(kMaxWarpsPerCta * 32) dyn_mpc_kernel(const Dyn
   }
 }
 
+// Infinite-horizon closed loop (clqr.cuh: certified_closed_loop): J_inf [S], T_cert [S], flags [S]; a.T = T_max.
+// Arena of 7: dyn_clqr_solve works in big[0..5], the tail matrix S stays in big[6].
+__global__ void __launch_bounds__(kMaxWarpsPerCta * 32) dyn_simulate_inf_kernel(const DynPb pb, const MpcArgs a) {
+  const int lane = threadIdx.x & 31, n = pb.n, m = pb.m;
+  Arena ar;
+  ar.carve(warp_arena(7, n, m), n, m, 7);
+  const int wpc = blockDim.x >> 5;
+  const int64_t wid = (int64_t)blockIdx.x * wpc + (threadIdx.x >> 5), nw = (int64_t)gridDim.x * wpc;
+  QpWs ws;
+  ws.carve(a.ws + (size_t)wid * QpWs::doubles(n, m, a.N), n, m, a.N);
+  double* x = ar.v + 32;                                   // closed-loop state (n <= 32 doubles)
+  double* u0 = ar.v + 8;                                   // m <= 8 doubles no routine of the solve touches
+  for (int64_t s = wid; s < a.S; s += nw) {
+    load_model(lane, ar, pb, a.dA, a.dB, a.S, s);
+    int flags = lqd::dyn_plan_prepare(lane, ar, pb, a.N, ws);          // K0 in ar.Kt, P0 in big[4]
+    const double cstar = lqd::dyn_box_certificate(lane, ar, pb, a.N, ws);
+    lqd::wcopy(lane, n, n, ar.big[4], ar.ld, ar.big[1], ar.ld);         // P0 (dyn_closed_loop overwrites big[4])
+    for (int i = lane; i < n; i += 32) ar.x[i] = a.pts ? a.pts[i] : a.x0[(int64_t)i * a.S + s];
+    __syncwarp();
+    double J0, rho, JT;
+    lqd::dyn_closed_loop(lane, ar, pb, 0, &J0, &rho, &JT, &flags);     // S in big[5]
+    double J = NAN;
+    int tc = -1;
+    if (flags & lq::FLAG_UNSTABLE) {
+      J = HUGE_VAL;
+    } else {
+      const double cS = (flags & lq::FLAG_LYAP_NOCONV) ? NAN : lqd::dyn_tail_level(lane, ar, cstar);
+      for (int i = lane; i < n; i += 32) x[i] = ar.x[i];
+      __syncwarp();
+      double cost = 0.0;
+      for (int t = 0; cS >= 0.0; ++t) {
+        const double v = lqd::wquad(lane, n, x, ar.big[6], ar.ld, x);
+        if (v <= cS) { J = cost + v; tc = t; break; }
+        if (t >= a.T) break;
+        double V;
+        flags |= lqd::dyn_clqr_solve(lane, ar, pb, a.N, x, ws, u0, &V, lq::Refs());
+        if (lane < m) ar.u[lane] = u0[lane];
+        __syncwarp();
+        cost += lqd::wquad(lane, n, x, pb.Q, n, x);
+        cost += lqd::wquad(lane, m, ar.u, pb.R, m, ar.u);
+        lqd::dyn_step_model(lane, n, m, pb.A, n, pb.B, x, ar.u, ar.xn);
+        for (int i = lane; i < n; i += 32) x[i] = ar.xn[i];
+        __syncwarp();
+      }
+      if (tc < 0) flags |= lq::FLAG_TAIL_UNCERTIFIED;
+    }
+    if (lane == 0) {
+      if (a.J_inf) a.J_inf[s] = J;
+      if (a.T_cert) a.T_cert[s] = tc;
+      if (a.flags) a.flags[s] = flags;
+    }
+    __syncwarp();
+  }
+}
+
 // ---------------------------------------------------------------------------------------------------- K3 / dlqr
 __global__ void __launch_bounds__(kMaxWarpsPerCta * 32) dyn_bounds_kernel(const DynPb pb, const BoundsArgs a,
                                                                        const int dlqr_only, double* K_dlqr,
@@ -384,6 +439,23 @@ int lq_dyn_mpc(lqmpc_ctx* ctx, MpcArgs a, bool sim) {
   dyn_mpc_kernel<<<blocks, w * 32, w * per_arena, ctx->stream>>>(pb, a, sim ? 1 : 0);
   ctx->launches++;
   return lq_check_cuda(ctx, cudaGetLastError(), "dyn_mpc_kernel launch");
+}
+
+int lq_dyn_simulate_inf(lqmpc_ctx* ctx, MpcArgs a) {
+  if (ctx->poly_p > 0)
+    return lq_set_error(ctx, LQMPC_EINVAL, "general input polytopes need a compiled (n, m) pair; see lqmpc_supported_dims()");
+  const DynPb pb = make_pb(ctx);
+  const size_t per_arena = Arena::doubles(pb.n, pb.m, 7) * sizeof(double);
+  int blocks, w;
+  int rc = grid_for(ctx, (const void*)dyn_simulate_inf_kernel, per_arena, a.S, &blocks, &w);
+  if (rc) return rc;
+  const size_t per = QpWs::doubles(pb.n, pb.m, a.N);
+  rc = lq_reserve_ws(ctx, per * (size_t)blocks * w * sizeof(double));
+  if (rc) return rc;
+  a.ws = reinterpret_cast<double*>(ctx->ws);
+  dyn_simulate_inf_kernel<<<blocks, w * 32, w * per_arena, ctx->stream>>>(pb, a);
+  ctx->launches++;
+  return lq_check_cuda(ctx, cudaGetLastError(), "dyn_simulate_inf_kernel launch");
 }
 
 int lq_dyn_bounds(lqmpc_ctx* ctx, const BoundsArgs& a) {

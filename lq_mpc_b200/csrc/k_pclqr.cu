@@ -9,3 +9,11 @@ int lq_launch_mpc_poly(lqmpc_ctx* ctx, const MpcArgs& a, bool sim) {
 #undef X
   return lq_set_error(ctx, LQMPC_EINVAL, "unsupported (n, m); see lqmpc_supported_dims()");
 }
+
+int lq_launch_simulate_inf_poly(lqmpc_ctx* ctx, const MpcArgs& a) {
+#define X(N_, M_) \
+  if (ctx->n == N_ && ctx->m == M_) return launch_simulate_inf_t<N_, M_, true>(ctx, a);
+  LQ_FOR_EACH_DIM(X)
+#undef X
+  return lq_set_error(ctx, LQMPC_EINVAL, "unsupported (n, m); see lqmpc_supported_dims()");
+}

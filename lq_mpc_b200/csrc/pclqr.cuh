@@ -396,4 +396,62 @@ LQ_HD int psimulate_sample(const Problem<n, m>& pb, const Plan<n, m>& pl, int N,
   return flags;
 }
 
+// Feasibility certificate of the unconstrained plan for the polytope (plan_prepare's argument with rows F_i instead of
+// box components): the planned input is u_k = g_k x_0, g_k = K_k Phi_k, so by Cauchy-Schwarz in the P0 metric
+//     F_i u_k <= sqrt(F_i g_k P0^-1 g_k' F_i') sqrt(x_0' P0 x_0),
+// and x_0' P0 x_0 <= cstar := min_{k,i} 1 / (F_i g_k P0^-1 g_k' F_i') keeps every planned input inside F_u u <= 1.
+// Reads the gains plan_prepare stored (ws.Ku). Returns cstar with the 1 - 1e-9 margin, -1 when P0 is not positive
+// definite.
+template <int n, int m>
+LQ_HD double poly_certificate(const Plan<n, m>& pl, int N, const Poly& py, const WsView& ws) {
+  const ClqrLayout<n, m> L(N);
+  double Lc[n * n], Lci[n], Phi[n * n];
+  LQ_UNROLL for (int i = 0; i < n * n; ++i) Lc[i] = pl.P0[i];
+  if (!chol_inv<n>(Lc, Lci)) return -1.0;
+  LQ_UNROLL for (int i = 0; i < n; ++i)
+    LQ_UNROLL for (int j = 0; j < n; ++j) Phi[i * n + j] = (i == j) ? 1.0 : 0.0;
+  double cs = HUGE_VAL;
+  for (int k = 0; k < N; ++k) {
+    double K[m * n], g[m * n];
+    LQ_UNROLL for (int e = 0; e < m * n; ++e) K[e] = ws[L.oKu + (int64_t)k * (m * n) + e];
+    mm<m, n, n>(K, Phi, g);
+    for (int r = 0; r < py.p; ++r) {
+      double y[n], q = 0.0;                                  // y = L^-1 (F_r g)', q = y'y
+      LQ_UNROLL for (int i = 0; i < n; ++i) {
+        double acc = 0.0;
+        LQ_UNROLL for (int j = 0; j < m; ++j) acc = fma(py.f(r, j, m), g[j * n + i], acc);
+        LQ_UNROLL for (int c = 0; c < i; ++c) acc = fma(-Lc[i * n + c], y[c], acc);
+        y[i] = acc * Lci[i];
+        q = fma(y[i], y[i], q);
+      }
+      if (q > 0.0) cs = dmin(cs, 1.0 / q);
+    }
+    if (k + 1 < N) {
+      double Acl[n * n], Pn[n * n];
+      LQ_UNROLL for (int i = 0; i < n; ++i)
+        LQ_UNROLL for (int j = 0; j < n; ++j) {
+          double acc = pl.Ah[i * n + j];
+          LQ_UNROLL for (int r = 0; r < m; ++r) acc = fma(pl.Bh[i * m + r], K[r * n + j], acc);
+          Acl[i * n + j] = acc;
+        }
+      mm<n, n, n>(Acl, Phi, Pn);
+      LQ_UNROLL for (int i = 0; i < n * n; ++i) Phi[i] = Pn[i];
+    }
+  }
+  return (cs == cs) ? cs * (1.0 - 1e-9) : -1.0;
+}
+
+// Infinite-horizon closed loop with the input polytope (clqr.cuh: certified_closed_loop): the unconstrained plan of
+// plan_prepare, the polytope certificate above, pclqr_solve for the steps before the certificate.
+template <int n, int m>
+LQ_HD int psimulate_inf_sample(const Problem<n, m>& pb, Plan<n, m>& pl, int N, int T_max, const double* x0,
+                               const Poly& py, const WsView& ws, double* J_inf, int* T_cert) {
+  const int pf = plan_prepare<n, m>(pb, pl, N, ws, /*certificate=*/false);
+  const double cstar = poly_certificate<n, m>(pl, N, py, ws);
+  return pf | certified_closed_loop<n, m>(pb, pl, N, cstar, T_max, x0, ws, [&](const double* x, double* u) {
+    double V;
+    return pclqr_solve<n, m>(pb, pl, N, x, py, ws, u, &V);
+  }, J_inf, T_cert);
+}
+
 }  // namespace lq

@@ -28,7 +28,8 @@ enum Flags : int {
   FLAG_LYAP_NOCONV = 64,   // Lyapunov doubling hit its iteration cap
   FLAG_EIG_NOCONV = 128,   // QR iteration did not converge
   FLAG_CHOL_FAIL = 256,    // R + B'PB not positive definite
-  FLAG_DOMAIN_ERROR = 512  // math.log / math.sqrt domain error (the reference raises ValueError, utils.py:506-507,514)
+  FLAG_DOMAIN_ERROR = 512, // math.log / math.sqrt domain error (the reference raises ValueError, utils.py:506-507,514)
+  FLAG_TAIL_UNCERTIFIED = 1024  // infinite-horizon closed loop: no invariant-set certificate within T_max steps
 };
 
 template <int n, int m>

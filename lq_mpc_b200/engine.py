@@ -25,6 +25,7 @@ FLAG_LYAP_NOCONV = 64
 FLAG_EIG_NOCONV = 128
 FLAG_CHOL_FAIL = 256
 FLAG_DOMAIN_ERROR = 512
+FLAG_TAIL_UNCERTIFIED = 1024
 
 RADIX_MAX_SEL = 32          # LQMPC_RADIX_MAX_SEL: selectors per lqmpc_column_radix_histogram call
 
@@ -55,6 +56,7 @@ ABI = {
     "lqmpc_set_input_polytope": (_int, [_vp, _int, _vp]),
     "lqmpc_mpc_solve_batch": (_int, [_vp, _i64, _vp, _vp, _int, _int] + [_vp] * 6),
     "lqmpc_simulate_batch": (_int, [_vp, _i64, _vp, _vp, _int, _int] + [_vp] * 7),
+    "lqmpc_simulate_inf_batch": (_int, [_vp, _i64, _vp, _vp, _int, _int] + [_vp] * 5),
     "lqmpc_bounds_fields": (_int, []),
     "lqmpc_bounds_batch": (_int, [_vp, _i64, _vp, _vp, _int, _vp, _vp, ctypes.c_double, ctypes.c_double, _vp,
                                   ctypes.c_double, _vp, _vp, _vp, _vp, _vp, ctypes.c_double, ctypes.c_double,
@@ -515,6 +517,37 @@ class Engine:
                                            _ptr(out.get("J_T")), _ptr(out.get("X")), _ptr(out.get("U")),
                                            _ptr(out.get("flags")), _ptr(out.get("n_active")))
         self._check(rc, "lqmpc_simulate_batch")
+        return out
+
+    @_streamed
+    def simulate_inf_batch(self, dA, dB, N: int, T_max: int = 1000, x0_shared=None, x0=None, S: Optional[int] = None,
+                           want=("J_inf", "T_cert", "flags")):
+        """Infinite-horizon cost of the simulate_batch closed loop (lqmpc_simulate_inf_batch): J_inf [S] (+inf:
+        unstable, NaN: not certified within T_max steps), T_cert [S] (the certified step, -1 when there is none),
+        flags [S]. x0_shared: (n,) one state for all samples, or x0: [n][S]. Regulation only."""
+        torch = self.torch
+        n = self.n
+        dA, dB = self._opt_dev(dA), self._opt_dev(dB)
+        if S is None:
+            S = dA.shape[-1] if dA is not None else (x0.shape[-1] if x0 is not None else 1)
+        if x0_shared is None:
+            xs = None
+        elif isinstance(x0_shared, torch.Tensor):
+            xs = self._dev(x0_shared).reshape(n)
+        else:
+            xs = self._dev(np.asarray(x0_shared, dtype=np.float64).reshape(n))
+        x0_d = self._opt_dev(x0)
+        out = {}
+        if "J_inf" in want:
+            out["J_inf"] = torch.empty((S,), dtype=torch.float64, device=self.device)
+        if "T_cert" in want:
+            out["T_cert"] = torch.empty((S,), dtype=torch.int32, device=self.device)
+        if "flags" in want:
+            out["flags"] = torch.empty((S,), dtype=torch.int32, device=self.device)
+        rc = self.lib.lqmpc_simulate_inf_batch(self._h, S, _ptr(dA), _ptr(dB), int(N), int(T_max), _ptr(xs),
+                                               _ptr(x0_d), _ptr(out.get("J_inf")), _ptr(out.get("T_cert")),
+                                               _ptr(out.get("flags")))
+        self._check(rc, "lqmpc_simulate_inf_batch")
         return out
 
     # ------------------------------------------------------------------------------------------------ K3

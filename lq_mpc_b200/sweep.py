@@ -40,7 +40,7 @@ def error_horizon_sweep(engine, error_A, error_B, error_vec: Sequence[float], ho
                         strict_reference: bool = True, group=None, keep_tables: bool = False,
                         shard: Optional[tuple] = None, phase_times: bool = False, fused_horizons: bool = False,
                         quantiles: Optional[Sequence[float]] = None, worst: bool = False,
-                        j_first: Optional[int] = None):
+                        j_first: Optional[int] = None, infinite_horizon: bool = False, T_max: int = 1000):
     """Full error-level x horizon sweep on an engine whose TRUE problem (A, B, Q, R, box, N_opc) is already set.
 
     error_A (n,n,N_sys,n_err), error_B (n,m,N_sys,n_err): the reference's grid layout (numpy) — `shard` = (rank, world)
@@ -71,9 +71,19 @@ def error_horizon_sweep(engine, error_A, error_B, error_vec: Sequence[float], ho
         finite entry. j_first = the global index of this rank's first perturbation: by default the shard's start for
         numpy grids, 0 for device grids (pass the j_first given to `device_error_grids`). `sampling.perturbation_at`
         regenerates the perturbation of a K6 grid from its index.
+
+    infinite_horizon=True (opt-in like the order statistics) adds, in both modes, one simulate_inf_batch per horizon
+    (same grids and x_start; T_max bounds the steps before the certificate, see Engine.simulate_inf_batch) and the
+    reduced quantity 'true_cost_inf' (the certified J_inf = lim J_T) with the statistics of every other quantity
+    (moments, and '_quantile' / '_argmax' / '_argmin' when those are on), 'ratio_true_inf_max', and the counts
+    'n_uncertified' / 'n_inf' [n_err][n_horizons] of its NaN (not certified within T_max) and +inf (unstable) entries,
+    which the statistics leave out. Its launches are timed with the closed loops ('simulate' phase). Only J_inf is
+    read from them: an incomplete solve in their steps before the certificate is not added to 'n_failed', which keeps
+    every key of the plain sweep as it is without the option.
     """
     import torch
     n_err = len(error_vec)
+    quants = QUANTITIES + ("true_cost_inf",) if infinite_horizon else QUANTITIES
     on_device = isinstance(error_A, torch.Tensor)          # SoA [n*n][N_sys*n_err] from K6 (already this rank's shard)
     if on_device:
         n = engine.n
@@ -103,14 +113,16 @@ def error_horizon_sweep(engine, error_A, error_B, error_vec: Sequence[float], ho
     e_per = engine._dev(np.tile(np.asarray(error_vec, dtype=np.float64), N_sys))
     ring = engine._dev(x0_vec.T.copy())
     x_start_d = engine._dev(x_start)                               # staged once: the loop below issues no H2D copy
-    res = {q + "_" + s: np.zeros((n_err, len(horizons))) for q in QUANTITIES for s in ("max", "min", "mean", "std")}
+    res = {q + "_" + s: np.zeros((n_err, len(horizons))) for q in quants for s in ("max", "min", "mean", "std")}
     n_invalid = np.zeros((n_err, len(horizons)))
     n_failed = np.zeros((n_err, len(horizons)))
+    n_uncertified = np.zeros((n_err, len(horizons)))
+    n_inf = np.zeros((n_err, len(horizons)))
     tables = [] if keep_tables else None
     dev_moments, dev_counts, dev_argext = [], [], []
     qs = _stats.check_quantiles(quantiles) if quantiles is not None else None
     if qs is not None:                     # every horizon's table, kept for the one selection after the loop
-        qtab = torch.empty((len(horizons), len(QUANTITIES) * n_err, N_sys), dtype=torch.float64, device=engine.device)
+        qtab = torch.empty((len(horizons), len(quants) * n_err, N_sys), dtype=torch.float64, device=engine.device)
     torch.cuda.synchronize(engine.device)
     t0 = time.perf_counter()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -123,9 +135,11 @@ def error_horizon_sweep(engine, error_A, error_B, error_vec: Sequence[float], ho
             ev.record()
             marks.append(ev)
 
-    def reduce_horizon(h, rs_flags, mv, sim, b):
+    def reduce_horizon(h, rs_flags, mv, sim, b, sinf=None):
         parts = [_strided_columns(v, n_err) for v in
                  (sim["J_T"], b["bound"], b["alpha"], b["beta"], b["xi"], b["eta"], mv)]
+        if sinf is not None:
+            parts.append(_strided_columns(sinf["J_inf"], n_err))
         cols = torch.cat(parts, dim=0) if qs is None else torch.cat(parts, dim=0, out=qtab[h])
         if worst:
             dev_argext.append(_stats.pack_argext(*engine.column_argext_raw(cols, j_first)))
@@ -138,10 +152,12 @@ def error_horizon_sweep(engine, error_A, error_B, error_vec: Sequence[float], ho
         for row in rs_flags:
             any_f = any_f | row
         fail = ((any_f & (4 | 8 | 64 | 128 | 256)) != 0).to(torch.float64)
-        dev_counts.append(torch.stack([_strided_columns(bad, n_err).sum(dim=1),
-                                       _strided_columns(fail, n_err).sum(dim=1)]))
+        counts = [bad, fail]
+        if sinf is not None:
+            counts += [torch.isnan(sinf["J_inf"]).to(torch.float64), torch.isinf(sinf["J_inf"]).to(torch.float64)]
+        dev_counts.append(torch.stack([_strided_columns(c, n_err).sum(dim=1) for c in counts]))
         if keep_tables:
-            tables.append(cols.reshape(len(QUANTITIES), n_err, N_sys).cpu().numpy())
+            tables.append(cols.reshape(len(quants), n_err, N_sys).cpu().numpy())
 
     if not fused_horizons:
         for h, N in enumerate(horizons):
@@ -151,11 +167,13 @@ def error_horizon_sweep(engine, error_A, error_B, error_vec: Sequence[float], ho
             mv = rs["M_V"]
             mark()
             sim = engine.simulate_batch(dA, dB, N, T, x0_shared=x_start_d, want=("J_T", "flags"))
+            sinf = engine.simulate_inf_batch(dA, dB, N, T_max, x0_shared=x_start_d, want=("J_inf",)) \
+                if infinite_horizon else None
             mark()
             b = engine.bounds_batch(dA, dB, N, e_per, e_per, mv, x_start_d, p, V_expert,
                                     strict_reference=strict_reference)
             mark()
-            reduce_horizon(h, rs["flags"], mv, sim, b)
+            reduce_horizon(h, rs["flags"], mv, sim, b, sinf)
     else:
         N_lo, N_hi = int(min(horizons)), int(max(horizons))
         pick = [int(N) - N_lo for N in horizons]                      # slots of the covering range
@@ -163,6 +181,8 @@ def error_horizon_sweep(engine, error_A, error_B, error_vec: Sequence[float], ho
         rs = engine.mpc_solve_range(dA, dB, N_lo, N_hi, pts=ring, want=("M_V", "flags"))
         mark()
         sims = [engine.simulate_batch(dA, dB, int(N), T, x0_shared=x_start_d, want=("J_T", "flags")) for N in horizons]
+        sinfs = [engine.simulate_inf_batch(dA, dB, int(N), T_max, x0_shared=x_start_d, want=("J_inf",))
+                 for N in horizons] if infinite_horizon else [None] * len(horizons)
         mark()
         br = engine.bounds_range(dA, dB, N_lo, N_hi, e_per, e_per, rs["M_V"], x_start_d, p, V_expert,
                                  strict_reference=strict_reference, detail=False)
@@ -170,7 +190,7 @@ def error_horizon_sweep(engine, error_A, error_B, error_vec: Sequence[float], ho
         for h, N in enumerate(horizons):
             k = pick[h]
             b = {q: br[q][k] for q in ("alpha", "beta", "xi", "eta", "bound", "flags")}
-            reduce_horizon(h, rs["flags"][k], rs["M_V"][k], sims[h], b)
+            reduce_horizon(h, rs["flags"][k], rs["M_V"][k], sims[h], b, sinfs[h])
     if qs is not None:
         keys = _stats.column_quantile_keys(engine, qtab.view(-1, N_sys), qs,
                                            torch.stack(dev_moments)[:, :, :, 2].sum(dim=1).reshape(-1), group)
@@ -186,12 +206,15 @@ def error_horizon_sweep(engine, error_A, error_B, error_vec: Sequence[float], ho
     e1.record()
     torch.cuda.synchronize(engine.device)
     for h in range(len(horizons)):
-        st = _stats.merge_moments(host_moments[h])                     # [len(QUANTITIES)*n_err] columns
-        for qi, q in enumerate(QUANTITIES):
+        st = _stats.merge_moments(host_moments[h])                     # [len(quants)*n_err] columns
+        for qi, q in enumerate(quants):
             for sname in ("max", "min", "mean", "std"):
                 res[q + "_" + sname][:, h] = st[sname][qi * n_err:(qi + 1) * n_err]
         n_invalid[:, h] = host_counts[h, 0]
         n_failed[:, h] = host_counts[h, 1]
+        if infinite_horizon:
+            n_uncertified[:, h] = host_counts[h, 2]
+            n_inf[:, h] = host_counts[h, 3]
     phases = None
     if phase_times:
         phases = {"ring_solves": 0.0, "simulate": 0.0, "bounds": 0.0, "stats_and_packing": 0.0}
@@ -200,26 +223,33 @@ def error_horizon_sweep(engine, error_A, error_B, error_vec: Sequence[float], ho
             phases[names[i % 4]] += marks[i].elapsed_time(marks[i + 1]) * 1e-3
     import torch.distributed as dist
     if dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1:
-        t = torch.from_numpy(np.stack([n_invalid, n_failed])).to(engine.device)   # (column_stats merged the moments)
+        counts = [n_invalid, n_failed] + ([n_uncertified, n_inf] if infinite_horizon else [])
+        t = torch.from_numpy(np.stack(counts)).to(engine.device)   # (column_stats merged the moments)
         dist.all_reduce(t, group=group)
-        n_invalid, n_failed = t.cpu().numpy()
+        t = t.cpu().numpy()
+        n_invalid, n_failed = t[0], t[1]
+        if infinite_horizon:
+            n_uncertified, n_inf = t[2], t[3]
     res.update({"error": np.asarray(error_vec, dtype=np.float64), "horizon": np.asarray(horizons),
                 "V_expert": V_expert, "x_start": x_start, "epsilon_lqr": eps_lqr, "n_invalid": n_invalid, "n_failed": n_failed,
                 "ratio_true_max": res["true_cost_max"] / V_expert, "ratio_bound_max": res["bound_max"] / V_expert,
                 "evals": int(N_sys) * n_err * len(horizons), "seconds": e0.elapsed_time(e1) * 1e-3,
                 "wall_seconds": time.perf_counter() - t0})
-    n_q = len(QUANTITIES)
+    if infinite_horizon:
+        res.update({"ratio_true_inf_max": res["true_cost_inf_max"] / V_expert, "n_uncertified": n_uncertified,
+                    "n_inf": n_inf})
+    n_q = len(quants)
     if qs is not None:
         qv = _stats.finish_quantiles(host_keys, host_moments[:, :, :, 2].sum(axis=1).reshape(-1), qs)
         qv = qv.reshape(len(qs), len(horizons), n_q, n_err)
-        for qi, q in enumerate(QUANTITIES):
+        for qi, q in enumerate(quants):
             res[q + "_quantile"] = np.ascontiguousarray(qv[:, :, qi, :].transpose(0, 2, 1))
         res["quantiles"] = qs
     if worst:
         ax = _stats.merge_argext(host_argext.reshape(host_argext.shape[0], -1, 4))
         for name in ("argmax", "argmin"):
             a = ax[name].reshape(len(horizons), n_q, n_err)
-            for qi, q in enumerate(QUANTITIES):
+            for qi, q in enumerate(quants):
                 res[q + "_" + name] = np.ascontiguousarray(a[:, qi, :].T)
     if keep_tables:
         res["tables"] = np.stack(tables)
