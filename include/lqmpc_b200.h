@@ -41,6 +41,7 @@ extern "C" {
 #define LQMPC_FLAG_CHOL_FAIL 256
 #define LQMPC_FLAG_DOMAIN_ERROR 512
 #define LQMPC_FLAG_TAIL_UNCERTIFIED 1024
+#define LQMPC_FLAG_ASCENT_MAXITER 2048
 
 typedef struct lqmpc_ctx lqmpc_ctx;
 
@@ -177,6 +178,35 @@ int lqmpc_simulate_batch(lqmpc_ctx* ctx, int64_t S, const double* dA, const doub
 int lqmpc_simulate_inf_batch(lqmpc_ctx* ctx, int64_t S, const double* dA, const double* dB, int N, int T_max,
                              const double* x0_shared, const double* x0, double* J_inf, int32_t* T_cert,
                              int32_t* flags);
+
+/* Worst-case model error of the unconstrained law (K1's J_inf at one horizon N). One sample per thread, every compiled
+ * (n, m) pair; the input box, an installed polytope and references do not enter (as lqmpc_eval_batch).
+ * dA [n*n][S], dB [n*m][S], x0 [n][S] (device, SoA). LQMPC_ESTATE without a problem; LQMPC_EINVAL on the
+ * run-time-dimension route, on a tiled-only context and for N < 1; S = 0 returns OK and launches nothing.
+ *
+ * lqmpc_eval_grad_batch: J, rho, ratio [S] as lqmpc_eval_batch (N_min = N_max = N; here J comes from Lyapunov doubling)
+ * and the exact gradient gA = dJ/d(dA) [n*n][S], gB = dJ/d(dB) [n*m][S] by the adjoint of the Riccati recursion and the
+ * closed loop (csrc/worst.cuh), O(N n^3) per sample. Unstable (J = +inf, LQMPC_FLAG_UNSTABLE) and failed entries
+ * (LQMPC_FLAG_CHOL_FAIL, _LYAP_NOCONV, _EIG_NOCONV, _NONFINITE) have NaN gradients. Any output may be NULL. */
+int lqmpc_eval_grad_batch(lqmpc_ctx* ctx, int64_t S, const double* dA, const double* dB, const double* x0, int N,
+                          double* J, double* rho, double* ratio, double* gA, double* gB, int32_t* flags);
+
+/* lqmpc_worst_case_batch: projected ascent of J from every sample over {||dA|| <= e_A, ||dB|| <= e_B}, each block
+ * separately; norm_type 0 = Frobenius, 1 = spectral, 2 = entrywise max. In u = (dA / e_A, dB / e_B) with gradient
+ * g = (e_A dJ/d(dA), e_B dJ/d(dB)): the start is projected onto the set; the ascent stops when the stationarity residual
+ * r = ||Proj(u + g/||g||) - u||_2 <= tol (r = 0 when g = 0); trial steps u+ = Proj(u + t g) take t = 0.5 / ||g|| first,
+ * then the Barzilai-Borwein step s's / (-s'y) when s'y < 0 and 10 t otherwise, and are accepted when
+ * J(u+) >= J(u) + 1e-4 g.(u+ - u), else t <- t / 4. A block with e = 0 stays zero. J never decreases from the projected
+ * start's value.
+ *   dA_out [n*n][S], dB_out [n*m][S]: the final perturbation (may alias dA / dB); J, rho, ratio [S]; iters [S] (accepted
+ *   steps); flags [S]. Any output may be NULL.
+ *   An unstable trial lies in the set and destabilises the loop: it is returned, J = +inf, LQMPC_FLAG_UNSTABLE. A trial
+ *   with another failure flag is rejected; a start with one is returned as it is. LQMPC_FLAG_ASCENT_MAXITER: max_iter
+ *   accepted steps (or a line search that shrank t by 4^60) without r <= tol.
+ * LQMPC_EINVAL besides the above: e_A / e_B negative or not finite, unknown norm_type, max_iter < 0, tol <= 0. */
+int lqmpc_worst_case_batch(lqmpc_ctx* ctx, int64_t S, const double* dA, const double* dB, const double* x0, int N,
+                           double e_A, double e_B, int norm_type, int max_iter, double tol, double* dA_out,
+                           double* dB_out, double* J, double* rho, double* ratio, int32_t* iters, int32_t* flags);
 
 /* K3 — batched bound coefficients: LQ_RDP_Calculator.energy_decreasing (utils_class.py:344-373) and
  * .energy_bound (utils_class.py:308-342) with every helper they call (utils.py: local_radius, ex_stability_lq,

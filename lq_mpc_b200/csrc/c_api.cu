@@ -106,7 +106,7 @@ int pipe_abort(lqmpc_ctx* ctx, int rc) {
 
 extern "C" {
 
-int lqmpc_abi_version(void) { return 3; }
+int lqmpc_abi_version(void) { return 4; }
 
 const char* lqmpc_supported_dims(void) { return LQ_DIMS_STRING; }
 
@@ -614,6 +614,59 @@ int lqmpc_simulate_inf_batch(lqmpc_ctx* ctx, int64_t S, const double* dA, const 
   a.S = S; a.dA = dA; a.dB = dB; a.N = N; a.T = T_max; a.npts = 1; a.pts = x0_shared; a.x0 = x0;
   a.J_inf = J_inf; a.T_cert = T_cert; a.flags = flags;
   return ctx->dyn ? lq_dyn_simulate_inf(ctx, a) : lq_launch_simulate_inf(ctx, a);
+}
+
+namespace {
+
+// shared checks of lqmpc_eval_grad_batch / lqmpc_worst_case_batch
+int worst_check(lqmpc_ctx* ctx, int64_t S, const double* dA, const double* dB, const double* x0, int N) {
+  if (!ctx->has_problem) {
+    if (ctx->has_tiled)
+      return lq_set_error(ctx, LQMPC_EINVAL, "the worst-case entry points need a compiled (n, m) pair; see "
+                                             "lqmpc_supported_dims() (not the tiled route)");
+    return lq_set_error(ctx, LQMPC_ESTATE, "problem not set");
+  }
+  if (ctx->dyn)
+    return lq_set_error(ctx, LQMPC_EINVAL, "the worst-case entry points need a compiled (n, m) pair; see "
+                                           "lqmpc_supported_dims() (not the run-time-dimension route)");
+  if (S < 0 || N < 1) return lq_set_error(ctx, LQMPC_EINVAL, "bad S/N");
+  if (S > 0 && (!dA || !dB || !x0)) return lq_set_error(ctx, LQMPC_EINVAL, "null input");
+  return LQMPC_OK;
+}
+
+}  // namespace
+
+int lqmpc_eval_grad_batch(lqmpc_ctx* ctx, int64_t S, const double* dA, const double* dB, const double* x0, int N,
+                          double* J, double* rho, double* ratio, double* gA, double* gB, int32_t* flags) {
+  if (!ctx) return LQMPC_EINVAL;
+  int rc = worst_check(ctx, S, dA, dB, x0, N);
+  if (rc || S == 0) return rc;
+  cudaSetDevice(ctx->device);
+  WorstArgs a{};
+  a.S = S; a.dA = dA; a.dB = dB; a.x0 = x0; a.N = N;
+  a.J = J; a.rho = rho; a.ratio = ratio; a.gA = gA; a.gB = gB; a.flags = flags;
+  return lq_launch_eval_grad(ctx, a);
+}
+
+int lqmpc_worst_case_batch(lqmpc_ctx* ctx, int64_t S, const double* dA, const double* dB, const double* x0, int N,
+                           double e_A, double e_B, int norm_type, int max_iter, double tol, double* dA_out,
+                           double* dB_out, double* J, double* rho, double* ratio, int32_t* iters, int32_t* flags) {
+  if (!ctx) return LQMPC_EINVAL;
+  int rc = worst_check(ctx, S, dA, dB, x0, N);
+  if (rc) return rc;
+  if (!(e_A >= 0.0 && e_A <= 1.79e308) || !(e_B >= 0.0 && e_B <= 1.79e308))
+    return lq_set_error(ctx, LQMPC_EINVAL, "e_A / e_B must be finite and >= 0");
+  if (norm_type < 0 || norm_type > 2)
+    return lq_set_error(ctx, LQMPC_EINVAL, "norm_type: 0 (Frobenius), 1 (spectral) or 2 (entrywise max)");
+  if (max_iter < 0) return lq_set_error(ctx, LQMPC_EINVAL, "max_iter < 0");
+  if (!(tol > 0.0)) return lq_set_error(ctx, LQMPC_EINVAL, "tol must be > 0");
+  if (S == 0) return LQMPC_OK;
+  cudaSetDevice(ctx->device);
+  WorstArgs a{};
+  a.S = S; a.dA = dA; a.dB = dB; a.x0 = x0; a.N = N;
+  a.eA = e_A; a.eB = e_B; a.norm = norm_type; a.max_iter = max_iter; a.tol = tol;
+  a.dA_out = dA_out; a.dB_out = dB_out; a.J = J; a.rho = rho; a.ratio = ratio; a.iters = iters; a.flags = flags;
+  return lq_launch_worst_case(ctx, a);
 }
 
 int lqmpc_bounds_fields(void) { return (int)lq::BF_COUNT; }

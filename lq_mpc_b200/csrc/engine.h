@@ -131,6 +131,27 @@ struct BoundsArgs {
   int polyP = 0;
 };
 
+// lqmpc_eval_grad_batch / lqmpc_worst_case_batch (k_worst.cu): SoA operands [elements][S]; any output may be NULL
+struct WorstArgs {
+  int64_t S;
+  const double* dA;   // [n*n][S]
+  const double* dB;   // [n*m][S]
+  const double* x0;   // [n][S]
+  int N;
+  double eA = 0.0, eB = 0.0, tol = 0.0;   // ascent only
+  int norm = 0, max_iter = 0;
+  double* J = nullptr;          // [S]
+  double* rho = nullptr;
+  double* ratio = nullptr;
+  int32_t* flags = nullptr;
+  double* gA = nullptr;         // gradient pass: [n*n][S], [n*m][S]
+  double* gB = nullptr;
+  double* dA_out = nullptr;     // ascent: the final perturbation (may alias dA / dB)
+  double* dB_out = nullptr;
+  int32_t* iters = nullptr;     // ascent: accepted steps [S]
+  double* ws = nullptr;         // filled by the launcher
+};
+
 struct TiledEval {
   int64_t S;
   const double* dA;   // [S][n*n] array of matrices
@@ -163,6 +184,8 @@ int lq_launch_mpc_poly(lqmpc_ctx* ctx, const MpcArgs& a, bool simulate);
 int lq_launch_mpc_range(lqmpc_ctx* ctx, const MpcArgs& a);
 int lq_launch_simulate_inf(lqmpc_ctx* ctx, const MpcArgs& a);
 int lq_launch_simulate_inf_poly(lqmpc_ctx* ctx, const MpcArgs& a);
+int lq_launch_eval_grad(lqmpc_ctx* ctx, const WorstArgs& a);
+int lq_launch_worst_case(lqmpc_ctx* ctx, const WorstArgs& a);
 int lq_launch_bounds(lqmpc_ctx* ctx, const BoundsArgs& a);
 bool lq_bounds_range_fused(lqmpc_ctx* ctx, const BoundsArgs& a);
 int lq_launch_bounds_range(lqmpc_ctx* ctx, const BoundsArgs& a);

@@ -363,6 +363,48 @@ LQ_HD void sym_eig_minmax(const double* Sin, double* lmin, double* lmax) {
   *lmin = lo; *lmax = hi;
 }
 
+// Full eigen-decomposition S = V diag(w) V' of a small symmetric matrix by the cyclic Jacobi sweeps of
+// sym_eig_minmax, with the rotations accumulated into V (row-major, eigenvector j in column j).
+template <int n>
+LQ_HD void sym_eig_jacobi(const double* Sin, double* w, double* V) {
+  double a[n * n];
+  LQ_UNROLL for (int i = 0; i < n * n; ++i) a[i] = Sin[i];
+  LQ_UNROLL for (int i = 0; i < n; ++i)
+    LQ_UNROLL for (int j = 0; j < n; ++j) V[i * n + j] = (i == j) ? 1.0 : 0.0;
+  for (int sweep = 0; sweep < 30 && n > 1; ++sweep) {
+    double off = 0.0, diag = 0.0;
+    LQ_UNROLL for (int i = 0; i < n; ++i) {
+      diag = dmax(diag, fabs(a[i * n + i]));
+      LQ_UNROLL for (int j = i + 1; j < n; ++j) off = dmax(off, fabs(a[i * n + j]));
+    }
+    if (off <= 1e-300 || off <= 1e-17 * diag) break;
+    LQ_UNROLL for (int p = 0; p < n - 1; ++p)
+      LQ_UNROLL for (int q = p + 1; q < n; ++q) {
+        const double apq = a[p * n + q];
+        if (fabs(apq) > 0.0) {
+          const double theta = (a[q * n + q] - a[p * n + p]) / (2.0 * apq);
+          const double t = dsign(1.0, theta) / (fabs(theta) + sqrt(fma(theta, theta, 1.0)));
+          const double c = 1.0 / sqrt(fma(t, t, 1.0));
+          const double s = t * c;
+          LQ_UNROLL for (int k = 0; k < n; ++k) {   // columns p, q of a and of V
+            const double akp = a[k * n + p], akq = a[k * n + q];
+            a[k * n + p] = c * akp - s * akq;
+            a[k * n + q] = s * akp + c * akq;
+            const double vkp = V[k * n + p], vkq = V[k * n + q];
+            V[k * n + p] = c * vkp - s * vkq;
+            V[k * n + q] = s * vkp + c * vkq;
+          }
+          LQ_UNROLL for (int k = 0; k < n; ++k) {   // rows p, q
+            const double apk = a[p * n + k], aqk = a[q * n + k];
+            a[p * n + k] = c * apk - s * aqk;
+            a[q * n + k] = s * apk + c * aqk;
+          }
+        }
+      }
+  }
+  LQ_UNROLL for (int i = 0; i < n; ++i) w[i] = a[i * n + i];
+}
+
 // Spectral norm of an (r x c) matrix: sqrt(lambda_max of the smaller Gram matrix).
 template <int r, int c>
 LQ_HD double norm2(const double* M) {

@@ -26,6 +26,9 @@ FLAG_EIG_NOCONV = 128
 FLAG_CHOL_FAIL = 256
 FLAG_DOMAIN_ERROR = 512
 FLAG_TAIL_UNCERTIFIED = 1024
+FLAG_ASCENT_MAXITER = 2048
+
+WORST_NORMS = {"f": 0, "2": 1, "max": 2}   # norm_type of lqmpc_worst_case_batch
 
 RADIX_MAX_SEL = 32          # LQMPC_RADIX_MAX_SEL: selectors per lqmpc_column_radix_histogram call
 
@@ -57,6 +60,9 @@ ABI = {
     "lqmpc_mpc_solve_batch": (_int, [_vp, _i64, _vp, _vp, _int, _int] + [_vp] * 6),
     "lqmpc_simulate_batch": (_int, [_vp, _i64, _vp, _vp, _int, _int] + [_vp] * 7),
     "lqmpc_simulate_inf_batch": (_int, [_vp, _i64, _vp, _vp, _int, _int] + [_vp] * 5),
+    "lqmpc_eval_grad_batch": (_int, [_vp, _i64, _vp, _vp, _vp, _int] + [_vp] * 6),
+    "lqmpc_worst_case_batch": (_int, [_vp, _i64, _vp, _vp, _vp, _int, ctypes.c_double, ctypes.c_double, _int, _int,
+                                      ctypes.c_double] + [_vp] * 7),
     "lqmpc_bounds_fields": (_int, []),
     "lqmpc_bounds_batch": (_int, [_vp, _i64, _vp, _vp, _int, _vp, _vp, ctypes.c_double, ctypes.c_double, _vp,
                                   ctypes.c_double, _vp, _vp, _vp, _vp, _vp, ctypes.c_double, ctypes.c_double,
@@ -548,6 +554,57 @@ class Engine:
                                                _ptr(x0_d), _ptr(out.get("J_inf")), _ptr(out.get("T_cert")),
                                                _ptr(out.get("flags")))
         self._check(rc, "lqmpc_simulate_inf_batch")
+        return out
+
+    # ------------------------------------------------------------------------------------------------ worst case
+    def _worst_operands(self, dA, dB, x0):
+        n, m = self.n, self.m
+        dA, dB, x0 = self._dev(dA), self._dev(dB), self._dev(x0)
+        S = dA.shape[-1]
+        if dA.numel() != n * n * S or dB.numel() != n * m * S or x0.numel() != n * S:
+            raise ValueError("operand shapes do not match (n, m, S)")
+        return dA, dB, x0, S
+
+    @_streamed
+    def eval_grad_batch(self, dA, dB, x0, N: int):
+        """J_inf of the unconstrained law (as eval_batch at one horizon N) and its exact gradient in the model error
+        (lqmpc_eval_grad_batch). dA [n*n][S], dB [n*m][S], x0 [n][S]. Returns device tensors J, rho, ratio [S],
+        gA [n*n][S] = dJ/d(dA), gB [n*m][S] = dJ/d(dB) (NaN where unstable or failed) and flags [S]."""
+        torch = self.torch
+        n, m = self.n, self.m
+        dA, dB, x0, S = self._worst_operands(dA, dB, x0)
+        f64 = dict(dtype=torch.float64, device=self.device)
+        out = {k: torch.empty((S,), **f64) for k in ("J", "rho", "ratio")}
+        out["gA"], out["gB"] = torch.empty((n * n, S), **f64), torch.empty((n * m, S), **f64)
+        out["flags"] = torch.empty((S,), dtype=torch.int32, device=self.device)
+        rc = self.lib.lqmpc_eval_grad_batch(self._h, S, _ptr(dA), _ptr(dB), _ptr(x0), int(N), _ptr(out["J"]),
+                                            _ptr(out["rho"]), _ptr(out["ratio"]), _ptr(out["gA"]), _ptr(out["gB"]),
+                                            _ptr(out["flags"]))
+        self._check(rc, "lqmpc_eval_grad_batch")
+        return out
+
+    @_streamed
+    def worst_case_batch(self, dA, dB, x0, N: int, e_A: float, e_B: float, norm: str = "f", max_iter: int = 200,
+                         tol: float = 1e-8):
+        """Projected ascent of J_inf from every sample over {||dA|| <= e_A, ||dB|| <= e_B} (lqmpc_worst_case_batch);
+        norm: "f" (Frobenius), "2" (spectral) or "max" (entrywise). Operands as eval_grad_batch. Returns device tensors
+        dA [n*n][S], dB [n*m][S] (the final perturbation), J, rho, ratio [S], iters [S] (accepted steps) and flags [S]
+        (FLAG_UNSTABLE: the set holds a destabilising error, J = +inf; FLAG_ASCENT_MAXITER: budget exhausted)."""
+        torch = self.torch
+        n, m = self.n, self.m
+        if norm not in WORST_NORMS:
+            raise ValueError("norm must be one of %s" % sorted(WORST_NORMS))
+        dA, dB, x0, S = self._worst_operands(dA, dB, x0)
+        f64 = dict(dtype=torch.float64, device=self.device)
+        out = {"dA": torch.empty((n * n, S), **f64), "dB": torch.empty((n * m, S), **f64)}
+        out.update({k: torch.empty((S,), **f64) for k in ("J", "rho", "ratio")})
+        out["iters"] = torch.empty((S,), dtype=torch.int32, device=self.device)
+        out["flags"] = torch.empty((S,), dtype=torch.int32, device=self.device)
+        rc = self.lib.lqmpc_worst_case_batch(self._h, S, _ptr(dA), _ptr(dB), _ptr(x0), int(N), float(e_A), float(e_B),
+                                             WORST_NORMS[norm], int(max_iter), float(tol), _ptr(out["dA"]),
+                                             _ptr(out["dB"]), _ptr(out["J"]), _ptr(out["rho"]), _ptr(out["ratio"]),
+                                             _ptr(out["iters"]), _ptr(out["flags"]))
+        self._check(rc, "lqmpc_worst_case_batch")
         return out
 
     # ------------------------------------------------------------------------------------------------ K3

@@ -1,0 +1,46 @@
+"""Worst-case model error of the unconstrained law: sample, then ascend.
+
+`worst_case_search` evaluates K1's performance ratio J_inf / V_expert(x0) on every sampled perturbation, takes the
+`top_k` largest as starts and runs the projected ascent of `Engine.worst_case_batch` from each over the error set
+{||dA|| <= e_A, ||dB|| <= e_B}. Sampling alone rarely lands near the worst case of a many-dimensional error set; the
+ascent moves each start to a stationary point of J_inf on the set (or to an error that destabilises the loop).
+
+The operands are the engine's SoA layout: the grids `sampling.device_error_grids` returns (one error level, norm
+'f' or '2') or `sampling.synth_samples_soa` draws (norm 'max'). Every step runs on the device.
+"""
+from __future__ import annotations
+
+from .engine import FLAG_UNSTABLE
+
+
+def worst_case_search(engine, dA, dB, x0, N: int, e_A: float, e_B: float, norm: str, top_k: int = 256,
+                      max_iter: int = 200, tol: float = 1e-8):
+    """dA [n*n][S], dB [n*m][S]; x0 [n][S] or one shared state [n]. Returns a dict:
+      sampled_max_ratio, sampled_argmax: K1's largest ratio over the S samples and its index;
+      per start (ordered by sampled ratio, +inf first, ties to the lowest index), device tensors: start_index,
+        ratio_start, ratio, J, dA [n*n][k], dB [n*m][k], iters, flags;
+      best_ratio, best_index: the largest ascended ratio and the sample index it started from;
+      n_unstable: ascents that found a destabilising error in the set (ratio = +inf)."""
+    torch = engine.torch
+    n = engine.n
+    dA, dB = engine._dev(dA), engine._dev(dB)
+    S = dA.shape[-1]
+    x0 = engine._dev(x0)
+    if x0.numel() == n and S != 1:
+        x0 = x0.reshape(n, 1).expand(n, S).contiguous()
+    ratio = engine.eval_batch(dA, dB, x0, N, N, want=("ratio",))["ratio"][0]
+    key = torch.nan_to_num(ratio, nan=-float("inf"), posinf=float("inf"))
+    order = torch.sort(key, descending=True, stable=True).indices
+    k = min(int(top_k), S)
+    idx = order[:k]
+    res = engine.worst_case_batch(dA[:, idx], dB[:, idx], x0[:, idx], N, e_A, e_B, norm, max_iter, tol)
+    best = int(torch.argmax(torch.nan_to_num(res["ratio"], nan=-float("inf"))).item()) if k else -1
+    return {
+        "sampled_max_ratio": float(key[order[0]].item()) if S else float("nan"),
+        "sampled_argmax": int(order[0].item()) if S else -1,
+        "start_index": idx, "ratio_start": ratio[idx], "ratio": res["ratio"], "J": res["J"], "dA": res["dA"],
+        "dB": res["dB"], "iters": res["iters"], "flags": res["flags"],
+        "best_ratio": float(res["ratio"][best].item()) if k else float("nan"),
+        "best_index": int(idx[best].item()) if k else -1,
+        "n_unstable": int(((res["flags"] & FLAG_UNSTABLE) != 0).sum().item()),
+    }
