@@ -208,6 +208,34 @@ int lqmpc_worst_case_batch(lqmpc_ctx* ctx, int64_t S, const double* dA, const do
                            double e_A, double e_B, int norm_type, int max_iter, double tol, double* dA_out,
                            double* dB_out, double* J, double* rho, double* ratio, int32_t* iters, int32_t* flags);
 
+/* Worst case over every initial state. For a given model error the performance ratio J_inf(x0) / V_expert(x0) =
+ * x0'S x0 / x0'P_exp x0 (S the closed-loop cost matrix S = W + A_cl'S A_cl, P_exp the expert matrix) is a Rayleigh
+ * quotient, so its supremum over x0 != 0 is
+ *   gamma(dA, dB) = lambda_max(L^-1 S L^-T),  P_exp = L L',
+ * attained at x_worst = L^-T w (w the top eigenvector), normalised to x_worst'P_exp x_worst = 1 with its entry of
+ * largest magnitude positive (ties to the lowest index). Same scope, operands and validation as the two calls above,
+ * without x0: LQMPC_ESTATE without a problem; LQMPC_EINVAL on the run-time-dimension route, on a tiled-only context,
+ * for N < 1 and for null inputs; S = 0 returns OK and launches nothing. Every output may be NULL.
+ *
+ * lqmpc_ratio_sup_batch: gamma, x_worst [n][S], the relative eigengap gap = (lambda_1 - lambda_2) / lambda_1 [S] (1 at
+ * n = 1), rho [S], flags [S], and with gA / gB non-NULL the gradient gA = dgamma/d(dA) [n*n][S], gB = dgamma/d(dB)
+ * [n*m][S] (x_worst'(dS)x_worst by the adjoint of lqmpc_eval_grad_batch at x0 = x_worst). The gradient is exact
+ * where lambda_max is simple; as gap -> 0 gamma has a kink and the gradient is that of one branch. A call without gA
+ * and gB computes the value only. Unstable: gamma = +inf, x_worst, gap and the gradient NaN, LQMPC_FLAG_UNSTABLE;
+ * LQMPC_FLAG_CHOL_FAIL, _LYAP_NOCONV, _NONFINITE as lqmpc_eval_grad_batch; _EIG_NOCONV also when the Jacobi
+ * eigensolver misses its off-diagonal tolerance.
+ *
+ * lqmpc_worst_case_sup_batch: the projected ascent of lqmpc_worst_case_batch (same e_A, e_B, norm_type, max_iter, tol,
+ * checks and stopping rule) with gamma in place of J, i.e. the joint ascent over (dA, dB, x0) of J / V_expert. Outputs
+ * dA_out / dB_out (may alias dA / dB), gamma, x_worst, rho, iters, flags at the final point. The result is a stationary
+ * point of gamma on the error set (a local maximum in general, or an error that destabilises the loop), not a
+ * certified global maximum. */
+int lqmpc_ratio_sup_batch(lqmpc_ctx* ctx, int64_t S, const double* dA, const double* dB, int N, double* gamma,
+                          double* x_worst, double* gap, double* rho, double* gA, double* gB, int32_t* flags);
+int lqmpc_worst_case_sup_batch(lqmpc_ctx* ctx, int64_t S, const double* dA, const double* dB, int N, double e_A,
+                               double e_B, int norm_type, int max_iter, double tol, double* dA_out, double* dB_out,
+                               double* gamma, double* x_worst, double* rho, int32_t* iters, int32_t* flags);
+
 /* K3 — batched bound coefficients: LQ_RDP_Calculator.energy_decreasing (utils_class.py:344-373) and
  * .energy_bound (utils_class.py:308-342) with every helper they call (utils.py: local_radius, ex_stability_lq,
  * ex_stability_bounds, fc_omega_eta, fc_ec_h, fc_ec_E, fc_ec_theta, fc_ec_g_*, geo_M, my_eigen, sl_syn_*,

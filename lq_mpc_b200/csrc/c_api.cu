@@ -106,7 +106,7 @@ int pipe_abort(lqmpc_ctx* ctx, int rc) {
 
 extern "C" {
 
-int lqmpc_abi_version(void) { return 4; }
+int lqmpc_abi_version(void) { return 5; }
 
 const char* lqmpc_supported_dims(void) { return LQ_DIMS_STRING; }
 
@@ -618,8 +618,9 @@ int lqmpc_simulate_inf_batch(lqmpc_ctx* ctx, int64_t S, const double* dA, const 
 
 namespace {
 
-// shared checks of lqmpc_eval_grad_batch / lqmpc_worst_case_batch
-int worst_check(lqmpc_ctx* ctx, int64_t S, const double* dA, const double* dB, const double* x0, int N) {
+// shared checks of the worst-case entry points; the sup-over-x0 ones take no x0 and pass need_x0 = false
+int worst_check(lqmpc_ctx* ctx, int64_t S, const double* dA, const double* dB, const double* x0, int N,
+                bool need_x0 = true) {
   if (!ctx->has_problem) {
     if (ctx->has_tiled)
       return lq_set_error(ctx, LQMPC_EINVAL, "the worst-case entry points need a compiled (n, m) pair; see "
@@ -630,7 +631,18 @@ int worst_check(lqmpc_ctx* ctx, int64_t S, const double* dA, const double* dB, c
     return lq_set_error(ctx, LQMPC_EINVAL, "the worst-case entry points need a compiled (n, m) pair; see "
                                            "lqmpc_supported_dims() (not the run-time-dimension route)");
   if (S < 0 || N < 1) return lq_set_error(ctx, LQMPC_EINVAL, "bad S/N");
-  if (S > 0 && (!dA || !dB || !x0)) return lq_set_error(ctx, LQMPC_EINVAL, "null input");
+  if (S > 0 && (!dA || !dB || (need_x0 && !x0))) return lq_set_error(ctx, LQMPC_EINVAL, "null input");
+  return LQMPC_OK;
+}
+
+// the ascent's settings, shared by lqmpc_worst_case_batch / lqmpc_worst_case_sup_batch
+int ascent_check(lqmpc_ctx* ctx, double e_A, double e_B, int norm_type, int max_iter, double tol) {
+  if (!(e_A >= 0.0 && e_A <= 1.79e308) || !(e_B >= 0.0 && e_B <= 1.79e308))
+    return lq_set_error(ctx, LQMPC_EINVAL, "e_A / e_B must be finite and >= 0");
+  if (norm_type < 0 || norm_type > 2)
+    return lq_set_error(ctx, LQMPC_EINVAL, "norm_type: 0 (Frobenius), 1 (spectral) or 2 (entrywise max)");
+  if (max_iter < 0) return lq_set_error(ctx, LQMPC_EINVAL, "max_iter < 0");
+  if (!(tol > 0.0)) return lq_set_error(ctx, LQMPC_EINVAL, "tol must be > 0");
   return LQMPC_OK;
 }
 
@@ -654,19 +666,42 @@ int lqmpc_worst_case_batch(lqmpc_ctx* ctx, int64_t S, const double* dA, const do
   if (!ctx) return LQMPC_EINVAL;
   int rc = worst_check(ctx, S, dA, dB, x0, N);
   if (rc) return rc;
-  if (!(e_A >= 0.0 && e_A <= 1.79e308) || !(e_B >= 0.0 && e_B <= 1.79e308))
-    return lq_set_error(ctx, LQMPC_EINVAL, "e_A / e_B must be finite and >= 0");
-  if (norm_type < 0 || norm_type > 2)
-    return lq_set_error(ctx, LQMPC_EINVAL, "norm_type: 0 (Frobenius), 1 (spectral) or 2 (entrywise max)");
-  if (max_iter < 0) return lq_set_error(ctx, LQMPC_EINVAL, "max_iter < 0");
-  if (!(tol > 0.0)) return lq_set_error(ctx, LQMPC_EINVAL, "tol must be > 0");
-  if (S == 0) return LQMPC_OK;
+  rc = ascent_check(ctx, e_A, e_B, norm_type, max_iter, tol);
+  if (rc || S == 0) return rc;
   cudaSetDevice(ctx->device);
   WorstArgs a{};
   a.S = S; a.dA = dA; a.dB = dB; a.x0 = x0; a.N = N;
   a.eA = e_A; a.eB = e_B; a.norm = norm_type; a.max_iter = max_iter; a.tol = tol;
   a.dA_out = dA_out; a.dB_out = dB_out; a.J = J; a.rho = rho; a.ratio = ratio; a.iters = iters; a.flags = flags;
   return lq_launch_worst_case(ctx, a);
+}
+
+int lqmpc_ratio_sup_batch(lqmpc_ctx* ctx, int64_t S, const double* dA, const double* dB, int N, double* gamma,
+                          double* x_worst, double* gap, double* rho, double* gA, double* gB, int32_t* flags) {
+  if (!ctx) return LQMPC_EINVAL;
+  int rc = worst_check(ctx, S, dA, dB, nullptr, N, false);
+  if (rc || S == 0) return rc;
+  cudaSetDevice(ctx->device);
+  WorstArgs a{};
+  a.S = S; a.dA = dA; a.dB = dB; a.x0 = nullptr; a.N = N;
+  a.J = gamma; a.rho = rho; a.gA = gA; a.gB = gB; a.flags = flags;
+  return lq_launch_ratio_sup(ctx, a, x_worst, gap);
+}
+
+int lqmpc_worst_case_sup_batch(lqmpc_ctx* ctx, int64_t S, const double* dA, const double* dB, int N, double e_A,
+                               double e_B, int norm_type, int max_iter, double tol, double* dA_out, double* dB_out,
+                               double* gamma, double* x_worst, double* rho, int32_t* iters, int32_t* flags) {
+  if (!ctx) return LQMPC_EINVAL;
+  int rc = worst_check(ctx, S, dA, dB, nullptr, N, false);
+  if (rc) return rc;
+  rc = ascent_check(ctx, e_A, e_B, norm_type, max_iter, tol);
+  if (rc || S == 0) return rc;
+  cudaSetDevice(ctx->device);
+  WorstArgs a{};
+  a.S = S; a.dA = dA; a.dB = dB; a.x0 = nullptr; a.N = N;
+  a.eA = e_A; a.eB = e_B; a.norm = norm_type; a.max_iter = max_iter; a.tol = tol;
+  a.dA_out = dA_out; a.dB_out = dB_out; a.J = gamma; a.rho = rho; a.iters = iters; a.flags = flags;
+  return lq_launch_worst_case_sup(ctx, a, x_worst);
 }
 
 int lqmpc_bounds_fields(void) { return (int)lq::BF_COUNT; }

@@ -186,6 +186,10 @@ int lq_launch_simulate_inf(lqmpc_ctx* ctx, const MpcArgs& a);
 int lq_launch_simulate_inf_poly(lqmpc_ctx* ctx, const MpcArgs& a);
 int lq_launch_eval_grad(lqmpc_ctx* ctx, const WorstArgs& a);
 int lq_launch_worst_case(lqmpc_ctx* ctx, const WorstArgs& a);
+// sup over x0 (lqmpc_ratio_sup_batch / lqmpc_worst_case_sup_batch): a.x0 is not read, a.J receives gamma; x_worst
+// [n][S] and gap [S] may be NULL
+int lq_launch_ratio_sup(lqmpc_ctx* ctx, const WorstArgs& a, double* x_worst, double* gap);
+int lq_launch_worst_case_sup(lqmpc_ctx* ctx, const WorstArgs& a, double* x_worst);
 int lq_launch_bounds(lqmpc_ctx* ctx, const BoundsArgs& a);
 bool lq_bounds_range_fused(lqmpc_ctx* ctx, const BoundsArgs& a);
 int lq_launch_bounds_range(lqmpc_ctx* ctx, const BoundsArgs& a);

@@ -364,20 +364,22 @@ LQ_HD void sym_eig_minmax(const double* Sin, double* lmin, double* lmax) {
 }
 
 // Full eigen-decomposition S = V diag(w) V' of a small symmetric matrix by the cyclic Jacobi sweeps of
-// sym_eig_minmax, with the rotations accumulated into V (row-major, eigenvector j in column j).
+// sym_eig_minmax, with the rotations accumulated into V (row-major, eigenvector j in column j). Returns false when 30
+// sweeps end before the off-diagonal tolerance holds.
 template <int n>
-LQ_HD void sym_eig_jacobi(const double* Sin, double* w, double* V) {
+LQ_HD bool sym_eig_jacobi(const double* Sin, double* w, double* V) {
   double a[n * n];
   LQ_UNROLL for (int i = 0; i < n * n; ++i) a[i] = Sin[i];
   LQ_UNROLL for (int i = 0; i < n; ++i)
     LQ_UNROLL for (int j = 0; j < n; ++j) V[i * n + j] = (i == j) ? 1.0 : 0.0;
+  bool conv = n == 1;
   for (int sweep = 0; sweep < 30 && n > 1; ++sweep) {
     double off = 0.0, diag = 0.0;
     LQ_UNROLL for (int i = 0; i < n; ++i) {
       diag = dmax(diag, fabs(a[i * n + i]));
       LQ_UNROLL for (int j = i + 1; j < n; ++j) off = dmax(off, fabs(a[i * n + j]));
     }
-    if (off <= 1e-300 || off <= 1e-17 * diag) break;
+    if (off <= 1e-300 || off <= 1e-17 * diag) { conv = true; break; }
     LQ_UNROLL for (int p = 0; p < n - 1; ++p)
       LQ_UNROLL for (int q = p + 1; q < n; ++q) {
         const double apq = a[p * n + q];
@@ -403,6 +405,7 @@ LQ_HD void sym_eig_jacobi(const double* Sin, double* w, double* V) {
       }
   }
   LQ_UNROLL for (int i = 0; i < n; ++i) w[i] = a[i * n + i];
+  return conv;
 }
 
 // Spectral norm of an (r x c) matrix: sqrt(lambda_max of the smaller Gram matrix).

@@ -12,6 +12,11 @@
 // (envelope theorem), so the reverse sweep k = N-1..1 needs no derivative of the gains: with F_k = A^ + B^ K(k),
 //   X = 2 P(k-1) F_k Pbar,  dJ/dA^ += X,  dJ/dB^ += X K(k)',  Pbar <- F_k Pbar F_k'.
 // The sweep reads the pairs (P(k-1), K(k)), k = 1..N-1, that the forward pass stores in the strided workspace.
+//
+// Sup over the initial state (SUP = true). The performance ratio J / V_expert = x0'S x0 / x0'P_exp x0 is a Rayleigh
+// quotient, so its worst case over x0 is gamma = lambda_max(L^-1 S L^-T), P_exp = L L', attained at x* = L^-T w (w the
+// top eigenvector). J := gamma replaces x0'S x0, and where lambda_max is simple dgamma = x*'dS x*: the adjoint above
+// with x0 = x*. Where it is repeated gamma has an upward kink, which an ascent is not trapped by.
 #pragma once
 #include "clqr.cuh"
 
@@ -50,12 +55,73 @@ LQ_HD void solve_l_inv(const double* L, const double* dinv, double* X) {
     }
 }
 
+// The Cholesky factor of the constant expert matrix, P_exp = L L' (chol_inv: reciprocal diagonal in Li), formed once
+// per thread for the SUP mode.
+template <int n>
+struct ExpertFactor {
+  double L[n * n], Li[n];
+  bool ok;
+};
+
+template <int n, int m>
+LQ_HD ExpertFactor<n> expert_factor(const Problem<n, m>& pb) {
+  ExpertFactor<n> f;
+  LQ_UNROLL for (int i = 0; i < n * n; ++i) f.L[i] = pb.Pexp[i];
+  f.ok = chol_inv<n>(f.L, f.Li);
+  return f;
+}
+
+// gamma = lambda_max(L^-1 S L^-T), the worst state x* = L^-T w (normalised to x*'P_exp x* = 1, its entry of largest
+// magnitude positive, ties to the lowest index) and the relative eigengap (lambda_1 - lambda_2) / lambda_1 (1 at n = 1).
+// Returns CHOL_FAIL (P_exp not positive definite; all outputs NaN) or EIG_NOCONV (Jacobi off its tolerance).
+template <int n>
+LQ_HD int sup_ratio(const ExpertFactor<n>& ef, const double* S, double* gamma, double* xs, double* gap) {
+  if (!ef.ok) {
+    *gamma = *gap = NAN;
+    LQ_UNROLL for (int i = 0; i < n; ++i) xs[i] = NAN;
+    return FLAG_CHOL_FAIL;
+  }
+  double T[n * n], M[n * n];
+  LQ_UNROLL for (int i = 0; i < n * n; ++i) T[i] = S[i];
+  solve_l_inv<n, n>(ef.L, ef.Li, T);             // L^-1 S
+  LQ_UNROLL for (int i = 0; i < n; ++i)
+    LQ_UNROLL for (int j = 0; j < n; ++j) M[i * n + j] = T[j * n + i];
+  solve_l_inv<n, n>(ef.L, ef.Li, M);             // L^-1 (L^-1 S)' = L^-1 S L^-T
+  LQ_UNROLL for (int i = 0; i < n; ++i)
+    LQ_UNROLL for (int j = i + 1; j < n; ++j) M[i * n + j] = M[j * n + i] = 0.5 * (M[i * n + j] + M[j * n + i]);
+  double w[n], V[n * n];
+  const bool conv = sym_eig_jacobi<n>(M, w, V);
+  // the top eigenpair by selects (no dynamic index into registers)
+  double l1 = w[0], l2 = -HUGE_VAL, v[n];
+  LQ_UNROLL for (int i = 0; i < n; ++i) v[i] = V[i * n];
+  LQ_UNROLL for (int j = 1; j < n; ++j) {
+    const bool top = w[j] > l1;
+    l2 = dmax(l2, top ? l1 : w[j]);
+    l1 = top ? w[j] : l1;
+    LQ_UNROLL for (int i = 0; i < n; ++i) v[i] = top ? V[i * n + j] : v[i];
+  }
+  double vv = 0.0;
+  LQ_UNROLL for (int i = 0; i < n; ++i) vv = fma(v[i], v[i], vv);
+  vv = 1.0 / sqrt(vv);
+  LQ_UNROLL for (int i = 0; i < n; ++i) v[i] *= vv;
+  solve_lt_inv<n, 1>(ef.L, ef.Li, v);
+  double big = v[0];
+  LQ_UNROLL for (int i = 1; i < n; ++i) big = (fabs(v[i]) > fabs(big)) ? v[i] : big;
+  LQ_UNROLL for (int i = 0; i < n; ++i) xs[i] = (big < 0.0) ? -v[i] : v[i];
+  *gamma = l1;
+  *gap = (n == 1) ? 1.0 : (l1 - l2) / l1;
+  return conv ? 0 : FLAG_EIG_NOCONV;
+}
+
 // J (and rho) at the model error (dA, dB); with gA / gB non-null also dJ/d(dA) [n*n] and dJ/d(dB) [n*m] (NaN where the
 // value is unstable or failed). Returns the flags: CHOL_FAIL of any stage, EIG_NOCONV, UNSTABLE (J = +inf),
 // LYAP_NOCONV, NONFINITE. ws holds worst_ws_doubles<n, m>(N) doubles and is written only for the gradient.
-template <int n, int m>
+// SUP: J is gamma (x0 is not read); the factor ef of P_exp is an input, x* [n] and the eigengap go to xs and gap (NaN
+// where the loop is unstable or P_exp has no Cholesky factor), and the gradient is that of gamma.
+template <int n, int m, bool SUP = false>
 LQ_HD int worst_eval(const Problem<n, m>& pb, const double* dA, const double* dB, const double* x0, int N,
-                     const WsView& ws, double* J_out, double* rho_out, double* gA, double* gB) {
+                     const WsView& ws, double* J_out, double* rho_out, double* gA, double* gB,
+                     const ExpertFactor<n>* ef = nullptr, double* xs = nullptr, double* gap = nullptr) {
   constexpr int ps = n * (n + 1) / 2, rs = ps + m * n;
   const bool grad = gA != nullptr;
   double Ah[n * n], Bh[n * m], P[n * n], K0[m * n];
@@ -99,10 +165,20 @@ LQ_HD int worst_eval(const Problem<n, m>& pb, const double* dA, const double* dB
   }
   if (!(rho < 1.0)) {
     *J_out = HUGE_VAL;
+    if constexpr (SUP) {
+      *gap = NAN;
+      LQ_UNROLL for (int i = 0; i < n; ++i) xs[i] = NAN;
+    }
     return flags | FLAG_UNSTABLE;
   }
   if (!lyapunov_doubling<n>(Acl, W, S)) flags |= FLAG_LYAP_NOCONV;
-  const double J = quad<n>(x0, S, x0);
+  double J;
+  if constexpr (SUP) {
+    flags |= sup_ratio<n>(*ef, S, &J, xs, gap);
+    x0 = xs;                                     // the Gramian below is seeded with x* x*'
+  } else {
+    J = quad<n>(x0, S, x0);
+  }
   if (!(fabs(J) <= 1.79e308)) flags |= FLAG_NONFINITE;
   *J_out = J;
   if (!grad || (flags & kWorstFail)) return flags;
@@ -273,14 +349,16 @@ struct AscentSettings {
 //   * a trial with another failure flag is rejected; a start with one ends the ascent there;
 //   * the budget of max_iter accepted steps (or a line search that shrinks t by 4^60) ends it with ASCENT_MAXITER.
 // Returns the flags of the final point; J, rho and the accepted-step count go to the outputs.
-template <int n, int m>
+// SUP: the ascent of gamma (worst_eval's SUP mode; x0 is not read) with x* of the final point in xs [n].
+template <int n, int m, bool SUP = false>
 LQ_HD int worst_ascent(const Problem<n, m>& pb, double* dA, double* dB, const double* x0, int N,
-                       const AscentSettings& as, const WsView& ws, double* J_out, double* rho_out, int* iters) {
+                       const AscentSettings& as, const WsView& ws, double* J_out, double* rho_out, int* iters,
+                       const ExpertFactor<n>* ef = nullptr, double* xs = nullptr) {
   const double eA2 = as.eA * as.eA, eB2 = as.eB * as.eB;
   worst_project<n, n>(dA, as.eA, as.norm);
   worst_project<n, m>(dB, as.eB, as.norm);
-  double gA[n * n], gB[n * m], J, rho;
-  int flags = worst_eval<n, m>(pb, dA, dB, x0, N, ws, &J, &rho, gA, gB);
+  double gA[n * n], gB[n * m], J, rho, gap, xt[n];
+  int flags = worst_eval<n, m, SUP>(pb, dA, dB, x0, N, ws, &J, &rho, gA, gB, ef, xs, &gap);
   int it = 0;
   double t = 0.0;
   while (!(flags & (kWorstFail | FLAG_UNSTABLE))) {
@@ -301,7 +379,7 @@ LQ_HD int worst_ascent(const Problem<n, m>& pb, double* dA, double* dB, const do
       double dot = 0.0;
       LQ_UNROLL for (int i = 0; i < n * n; ++i) dot = fma(gA[i], tA[i] - dA[i], dot);
       LQ_UNROLL for (int i = 0; i < n * m; ++i) dot = fma(gB[i], tB[i] - dB[i], dot);
-      ft = worst_eval<n, m>(pb, tA, tB, x0, N, ws, &Jt, &rt, nullptr, nullptr);
+      ft = worst_eval<n, m, SUP>(pb, tA, tB, x0, N, ws, &Jt, &rt, nullptr, nullptr, ef, xt, &gap);
       if ((ft & FLAG_UNSTABLE) || (!(ft & kWorstFail) && Jt >= J + 1e-4 * dmax(dot, 0.0))) { accepted = true; break; }
       t *= 0.25;
     }
@@ -310,13 +388,14 @@ LQ_HD int worst_ascent(const Problem<n, m>& pb, double* dA, double* dB, const do
     if (ft & FLAG_UNSTABLE) {
       LQ_UNROLL for (int i = 0; i < n * n; ++i) dA[i] = tA[i];
       LQ_UNROLL for (int i = 0; i < n * m; ++i) dB[i] = tB[i];
+      if constexpr (SUP) { LQ_UNROLL for (int i = 0; i < n; ++i) xs[i] = xt[i]; }
       J = Jt; rho = rt; flags = ft;
       break;
     }
     // the gradient at the accepted point (its value repeats the trial's bit for bit). With s = u+ - u and
     // y = g^+ - g^, s'y = (dA+ - dA).(gA+ - gA) + (dB+ - dB).(gB+ - gB): the scales e cancel.
     double nA[n * n], nB[n * m], sy = 0.0;
-    flags = worst_eval<n, m>(pb, tA, tB, x0, N, ws, &J, &rho, nA, nB);
+    flags = worst_eval<n, m, SUP>(pb, tA, tB, x0, N, ws, &J, &rho, nA, nB, ef, xs, &gap);
     LQ_UNROLL for (int i = 0; i < n * n; ++i) {
       sy = fma(tA[i] - dA[i], nA[i] - gA[i], sy);
       dA[i] = tA[i]; gA[i] = nA[i];

@@ -28,7 +28,7 @@ FLAG_DOMAIN_ERROR = 512
 FLAG_TAIL_UNCERTIFIED = 1024
 FLAG_ASCENT_MAXITER = 2048
 
-WORST_NORMS = {"f": 0, "2": 1, "max": 2}   # norm_type of lqmpc_worst_case_batch
+WORST_NORMS = {"f": 0, "2": 1, "max": 2}   # norm_type of lqmpc_worst_case_batch / lqmpc_worst_case_sup_batch
 
 RADIX_MAX_SEL = 32          # LQMPC_RADIX_MAX_SEL: selectors per lqmpc_column_radix_histogram call
 
@@ -63,6 +63,9 @@ ABI = {
     "lqmpc_eval_grad_batch": (_int, [_vp, _i64, _vp, _vp, _vp, _int] + [_vp] * 6),
     "lqmpc_worst_case_batch": (_int, [_vp, _i64, _vp, _vp, _vp, _int, ctypes.c_double, ctypes.c_double, _int, _int,
                                       ctypes.c_double] + [_vp] * 7),
+    "lqmpc_ratio_sup_batch": (_int, [_vp, _i64, _vp, _vp, _int] + [_vp] * 7),
+    "lqmpc_worst_case_sup_batch": (_int, [_vp, _i64, _vp, _vp, _int, ctypes.c_double, ctypes.c_double, _int, _int,
+                                          ctypes.c_double] + [_vp] * 7),
     "lqmpc_bounds_fields": (_int, []),
     "lqmpc_bounds_batch": (_int, [_vp, _i64, _vp, _vp, _int, _vp, _vp, ctypes.c_double, ctypes.c_double, _vp,
                                   ctypes.c_double, _vp, _vp, _vp, _vp, _vp, ctypes.c_double, ctypes.c_double,
@@ -557,11 +560,12 @@ class Engine:
         return out
 
     # ------------------------------------------------------------------------------------------------ worst case
-    def _worst_operands(self, dA, dB, x0):
+    def _worst_operands(self, dA, dB, x0=None):
         n, m = self.n, self.m
-        dA, dB, x0 = self._dev(dA), self._dev(dB), self._dev(x0)
+        dA, dB = self._dev(dA), self._dev(dB)
+        x0 = None if x0 is None else self._dev(x0)
         S = dA.shape[-1]
-        if dA.numel() != n * n * S or dB.numel() != n * m * S or x0.numel() != n * S:
+        if dA.numel() != n * n * S or dB.numel() != n * m * S or (x0 is not None and x0.numel() != n * S):
             raise ValueError("operand shapes do not match (n, m, S)")
         return dA, dB, x0, S
 
@@ -605,6 +609,53 @@ class Engine:
                                              _ptr(out["dB"]), _ptr(out["J"]), _ptr(out["rho"]), _ptr(out["ratio"]),
                                              _ptr(out["iters"]), _ptr(out["flags"]))
         self._check(rc, "lqmpc_worst_case_batch")
+        return out
+
+    @_streamed
+    def ratio_sup_batch(self, dA, dB, N: int, grad: bool = False):
+        """The worst performance ratio over every initial state, gamma = sup_x0 J_inf(x0) / V_expert(x0) =
+        lambda_max(S, P_exp), at each model error (lqmpc_ratio_sup_batch). dA [n*n][S], dB [n*m][S]. Returns device
+        tensors gamma [S], x_worst [n][S] (the state attaining it, x_worst'P_exp x_worst = 1), gap [S] (relative
+        eigengap (lambda_1 - lambda_2) / lambda_1), rho [S] and flags [S]; with grad also gA [n*n][S] = dgamma/d(dA) and
+        gB [n*m][S] = dgamma/d(dB) (exact where gap > 0; NaN where unstable or failed)."""
+        torch = self.torch
+        n, m = self.n, self.m
+        dA, dB, _, S = self._worst_operands(dA, dB)
+        f64 = dict(dtype=torch.float64, device=self.device)
+        out = {k: torch.empty((S,), **f64) for k in ("gamma", "gap", "rho")}
+        out["x_worst"] = torch.empty((n, S), **f64)
+        out["flags"] = torch.empty((S,), dtype=torch.int32, device=self.device)
+        if grad:
+            out["gA"], out["gB"] = torch.empty((n * n, S), **f64), torch.empty((n * m, S), **f64)
+        rc = self.lib.lqmpc_ratio_sup_batch(self._h, S, _ptr(dA), _ptr(dB), int(N), _ptr(out["gamma"]),
+                                            _ptr(out["x_worst"]), _ptr(out["gap"]), _ptr(out["rho"]),
+                                            _ptr(out.get("gA")), _ptr(out.get("gB")), _ptr(out["flags"]))
+        self._check(rc, "lqmpc_ratio_sup_batch")
+        return out
+
+    @_streamed
+    def worst_case_sup_batch(self, dA, dB, N: int, e_A: float, e_B: float, norm: str = "f", max_iter: int = 200,
+                             tol: float = 1e-8):
+        """Projected ascent of gamma (ratio_sup_batch) from every sample over {||dA|| <= e_A, ||dB|| <= e_B}
+        (lqmpc_worst_case_sup_batch): the joint worst case over the model error and the initial state, to a stationary
+        point. Settings and flags as worst_case_batch. Returns device tensors dA [n*n][S], dB [n*m][S], gamma [S],
+        x_worst [n][S], rho [S], iters [S] and flags [S]."""
+        torch = self.torch
+        n, m = self.n, self.m
+        if norm not in WORST_NORMS:
+            raise ValueError("norm must be one of %s" % sorted(WORST_NORMS))
+        dA, dB, _, S = self._worst_operands(dA, dB)
+        f64 = dict(dtype=torch.float64, device=self.device)
+        out = {"dA": torch.empty((n * n, S), **f64), "dB": torch.empty((n * m, S), **f64),
+               "gamma": torch.empty((S,), **f64), "x_worst": torch.empty((n, S), **f64),
+               "rho": torch.empty((S,), **f64)}
+        out["iters"] = torch.empty((S,), dtype=torch.int32, device=self.device)
+        out["flags"] = torch.empty((S,), dtype=torch.int32, device=self.device)
+        rc = self.lib.lqmpc_worst_case_sup_batch(self._h, S, _ptr(dA), _ptr(dB), int(N), float(e_A), float(e_B),
+                                                 WORST_NORMS[norm], int(max_iter), float(tol), _ptr(out["dA"]),
+                                                 _ptr(out["dB"]), _ptr(out["gamma"]), _ptr(out["x_worst"]),
+                                                 _ptr(out["rho"]), _ptr(out["iters"]), _ptr(out["flags"]))
+        self._check(rc, "lqmpc_worst_case_sup_batch")
         return out
 
     # ------------------------------------------------------------------------------------------------ K3

@@ -5,6 +5,9 @@
 {||dA|| <= e_A, ||dB|| <= e_B}. Sampling alone rarely lands near the worst case of a many-dimensional error set; the
 ascent moves each start to a stationary point of J_inf on the set (or to an error that destabilises the loop).
 
+`worst_case_search_sup` does the same without an x0: its objective is the worst ratio over every initial state,
+gamma = lambda_max(S, P_exp), and its ascent is the joint one over the model error and the initial state.
+
 The operands are the engine's SoA layout: the grids `sampling.device_error_grids` returns (one error level, norm
 'f' or '2') or `sampling.synth_samples_soa` draws (norm 'max'). Every step runs on the device.
 """
@@ -41,6 +44,34 @@ def worst_case_search(engine, dA, dB, x0, N: int, e_A: float, e_B: float, norm: 
         "start_index": idx, "ratio_start": ratio[idx], "ratio": res["ratio"], "J": res["J"], "dA": res["dA"],
         "dB": res["dB"], "iters": res["iters"], "flags": res["flags"],
         "best_ratio": float(res["ratio"][best].item()) if k else float("nan"),
+        "best_index": int(idx[best].item()) if k else -1,
+        "n_unstable": int(((res["flags"] & FLAG_UNSTABLE) != 0).sum().item()),
+    }
+
+
+def worst_case_search_sup(engine, dA, dB, N: int, e_A: float, e_B: float, norm: str, top_k: int = 256,
+                          max_iter: int = 200, tol: float = 1e-8):
+    """worst_case_search over every initial state at once: ranks the S samples by gamma = sup_x0 J_inf / V_expert
+    (Engine.ratio_sup_batch, value only; +inf first, ties to the lowest index) and runs the ascent of gamma
+    (Engine.worst_case_sup_batch) from the `top_k` largest. dA [n*n][S], dB [n*m][S]. Returns the keys of
+    worst_case_search with `ratio` (and sampled_max_ratio, ratio_start, best_ratio) meaning gamma and `J` = gamma (the
+    cost J_inf(x_worst), since x_worst'P_exp x_worst = 1), plus x_worst [n][k]: the initial state attaining gamma."""
+    torch = engine.torch
+    dA, dB = engine._dev(dA), engine._dev(dB)
+    S = dA.shape[-1]
+    gamma = engine.ratio_sup_batch(dA, dB, N)["gamma"]
+    key = torch.nan_to_num(gamma, nan=-float("inf"), posinf=float("inf"))
+    order = torch.sort(key, descending=True, stable=True).indices
+    k = min(int(top_k), S)
+    idx = order[:k]
+    res = engine.worst_case_sup_batch(dA[:, idx], dB[:, idx], N, e_A, e_B, norm, max_iter, tol)
+    best = int(torch.argmax(torch.nan_to_num(res["gamma"], nan=-float("inf"))).item()) if k else -1
+    return {
+        "sampled_max_ratio": float(key[order[0]].item()) if S else float("nan"),
+        "sampled_argmax": int(order[0].item()) if S else -1,
+        "start_index": idx, "ratio_start": gamma[idx], "ratio": res["gamma"], "J": res["gamma"], "dA": res["dA"],
+        "dB": res["dB"], "iters": res["iters"], "flags": res["flags"], "x_worst": res["x_worst"],
+        "best_ratio": float(res["gamma"][best].item()) if k else float("nan"),
         "best_index": int(idx[best].item()) if k else -1,
         "n_unstable": int(((res["flags"] & FLAG_UNSTABLE) != 0).sum().item()),
     }
