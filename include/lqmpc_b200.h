@@ -236,6 +236,44 @@ int lqmpc_worst_case_sup_batch(lqmpc_ctx* ctx, int64_t S, const double* dA, cons
                                double e_B, int norm_type, int max_iter, double tol, double* dA_out, double* dB_out,
                                double* gamma, double* x_worst, double* rho, int32_t* iters, int32_t* flags);
 
+/* Worst-case model error of the input-constrained closed loop: K2c's certified J_inf (lqmpc_simulate_inf_batch, input
+ * box of lqmpc_set_problem, regulation) at one horizon N,
+ *   J_inf = sum_{t<tau} (x_t'Q x_t + u_t'R u_t) + x_tau'S x_tau,  u_t = QP_N(x_t; A+dA, B+dB)_0,  x_{t+1} = A x_t + B u_t,
+ * with S = W + A_cl'S A_cl, A_cl = A + B K0, K0 the unconstrained horizon-N gain of the model. J_inf is continuous in
+ * (dA, dB) and smooth wherever every pre-certificate QP is strictly complementary. One sample per thread, every compiled
+ * (n, m) pair. dA [n*n][S], dB [n*m][S] (device, SoA); the initial state as lqmpc_simulate_batch: x0_shared [n] or x0
+ * [n][S], exactly one. LQMPC_ESTATE without a problem; LQMPC_EINVAL with references or an input polytope installed, on
+ * the run-time-dimension route, on a tiled-only context, for N < 1, T_max < 0 and null dA / dB; S = 0 returns OK and
+ * launches nothing. Every output may be NULL. The per-thread workspace grows with T_max: the gradient and the ascent
+ * keep the closed-loop states x_0..x_tau, (T_max + 1) n doubles per resident thread, besides O(N (n^2 + n m)) for
+ * the solver, the Riccati stage records and the QP plans.
+ *
+ * lqmpc_simulate_inf_grad_batch: J_inf, T_cert, flags [S] as lqmpc_simulate_inf_batch (the same code computes them),
+ * rho [S] = rho(A + B K0), and with gA / gB non-NULL the gradient gA = dJ_inf/d(dA) [n*n][S], gB = dJ_inf/d(dB)
+ * [n*m][S] by one reverse pass over the steps t < tau. With lambda_tau = 2 S x_tau and c = 2 R u_t + B'lambda:
+ *   a step that took the unconstrained law adds c x_t' to Kbar = dJ/dK0 and sets lambda <- 2 Q x_t + A'lambda + K0'c;
+ *   a step with an active bound sets lambda <- 2 Q x_t + A'lambda + Kc0'c (Kc0 the stage-0 gain of the QP's final
+ *   working set) and adds the implicit-function vector-Jacobian product of c'u_t in (A+dA, B+dB), from the adjoint LQ
+ *   of that working set;
+ *   the tail adds 2 (R K0 + B'S A_cl) Lambda, Lambda = x_tau x_tau' + A_cl Lambda A_cl', to Kbar, which the adjoint of
+ *   the Riccati recursion (lqmpc_eval_grad_batch's) maps to (gA, gB).
+ * The gradient is exact where every pre-certificate solve is strictly complementary; elsewhere it is the gradient for
+ * the active sets the solver found. It is NaN where J_inf is +inf or NaN or any of LQMPC_FLAG_CHOL_FAIL, _LYAP_NOCONV,
+ * _EIG_NOCONV, _NONFINITE, _QP_MAXITER, _TAIL_UNCERTIFIED is set. A call without gA and gB computes the value only.
+ *
+ * lqmpc_worst_case_inf_batch: the projected ascent of lqmpc_worst_case_batch (same e_A, e_B, norm_type, max_iter, tol,
+ * checks and stopping rule) on this J_inf. A trial with any of the flags above is rejected and a start with one is
+ * returned as it is; an unstable trial is the result (J_inf = +inf, T_cert = -1, LQMPC_FLAG_UNSTABLE). Outputs dA_out /
+ * dB_out (may alias dA / dB), J_inf, T_cert, rho, iters, flags at the final point. The result is a stationary point of
+ * J_inf on the error set (or an error that destabilises the loop), not a certified global maximum. */
+int lqmpc_simulate_inf_grad_batch(lqmpc_ctx* ctx, int64_t S, const double* dA, const double* dB, int N, int T_max,
+                                  const double* x0_shared, const double* x0, double* J_inf, int32_t* T_cert,
+                                  double* rho, double* gA, double* gB, int32_t* flags);
+int lqmpc_worst_case_inf_batch(lqmpc_ctx* ctx, int64_t S, const double* dA, const double* dB, int N, int T_max,
+                               const double* x0_shared, const double* x0, double e_A, double e_B, int norm_type,
+                               int max_iter, double tol, double* dA_out, double* dB_out, double* J_inf,
+                               int32_t* T_cert, double* rho, int32_t* iters, int32_t* flags);
+
 /* K3 — batched bound coefficients: LQ_RDP_Calculator.energy_decreasing (utils_class.py:344-373) and
  * .energy_bound (utils_class.py:308-342) with every helper they call (utils.py: local_radius, ex_stability_lq,
  * ex_stability_bounds, fc_omega_eta, fc_ec_h, fc_ec_E, fc_ec_theta, fc_ec_g_*, geo_M, my_eigen, sl_syn_*,

@@ -15,7 +15,7 @@ LIBDIR = os.path.join(PKG, "_lib")
 OBJDIR = os.path.join(PKG, "_lib", "obj")
 LIB = os.path.join(LIBDIR, "liblqmpc_b200.so")
 SOURCES = ["c_api.cu", "k_eval.cu", "k_clqr.cu", "k_pclqr.cu", "k_bounds.cu", "k_stats.cu", "k_tiled.cu", "k_sampler.cu", "k_dyn.cu", "k_group.cu",
-           "k_worst.cu"]
+           "k_worst.cu", "k_worst_inf.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xptxas", "-v", "--expt-relaxed-constexpr"]
 NVCC_FLAGS += os.environ.get("LQMPC_NVCC_EXTRA", "").split()     # development switches, e.g. -DLQ_K4_PROFILE

@@ -106,7 +106,7 @@ int pipe_abort(lqmpc_ctx* ctx, int rc) {
 
 extern "C" {
 
-int lqmpc_abi_version(void) { return 5; }
+int lqmpc_abi_version(void) { return 6; }
 
 const char* lqmpc_supported_dims(void) { return LQ_DIMS_STRING; }
 
@@ -702,6 +702,54 @@ int lqmpc_worst_case_sup_batch(lqmpc_ctx* ctx, int64_t S, const double* dA, cons
   a.eA = e_A; a.eB = e_B; a.norm = norm_type; a.max_iter = max_iter; a.tol = tol;
   a.dA_out = dA_out; a.dB_out = dB_out; a.J = gamma; a.rho = rho; a.iters = iters; a.flags = flags;
   return lq_launch_worst_case_sup(ctx, a, x_worst);
+}
+
+namespace {
+
+// checks of the constrained worst-case entry points: those of lqmpc_simulate_inf_batch and of the worst-case calls
+int worst_inf_check(lqmpc_ctx* ctx, int64_t S, const double* dA, const double* dB, int N, int T_max,
+                    const double* x0_shared, const double* x0) {
+  int rc = worst_check(ctx, S, dA, dB, nullptr, N, false);
+  if (rc) return rc;
+  if (T_max < 0) return lq_set_error(ctx, LQMPC_EINVAL, "bad T_max");
+  if ((x0_shared == nullptr) == (x0 == nullptr))
+    return lq_set_error(ctx, LQMPC_EINVAL, "give exactly one of x0_shared / x0");
+  if (ctx->ref_ld > 0) return lq_set_error(ctx, LQMPC_EINVAL, "the infinite-horizon cost is for regulation (no references)");
+  if (ctx->poly_p > 0)
+    return lq_set_error(ctx, LQMPC_EINVAL, "the constrained worst-case entry points take the input box, not a polytope");
+  return LQMPC_OK;
+}
+
+}  // namespace
+
+int lqmpc_simulate_inf_grad_batch(lqmpc_ctx* ctx, int64_t S, const double* dA, const double* dB, int N, int T_max,
+                                  const double* x0_shared, const double* x0, double* J_inf, int32_t* T_cert,
+                                  double* rho, double* gA, double* gB, int32_t* flags) {
+  if (!ctx) return LQMPC_EINVAL;
+  int rc = worst_inf_check(ctx, S, dA, dB, N, T_max, x0_shared, x0);
+  if (rc || S == 0) return rc;
+  cudaSetDevice(ctx->device);
+  WorstInfArgs a{};
+  a.S = S; a.dA = dA; a.dB = dB; a.x0_shared = x0_shared; a.x0 = x0; a.N = N; a.T_max = T_max;
+  a.J = J_inf; a.T_cert = T_cert; a.rho = rho; a.gA = gA; a.gB = gB; a.flags = flags;
+  return lq_launch_simulate_inf_grad(ctx, a);
+}
+
+int lqmpc_worst_case_inf_batch(lqmpc_ctx* ctx, int64_t S, const double* dA, const double* dB, int N, int T_max,
+                               const double* x0_shared, const double* x0, double e_A, double e_B, int norm_type,
+                               int max_iter, double tol, double* dA_out, double* dB_out, double* J_inf,
+                               int32_t* T_cert, double* rho, int32_t* iters, int32_t* flags) {
+  if (!ctx) return LQMPC_EINVAL;
+  int rc = worst_inf_check(ctx, S, dA, dB, N, T_max, x0_shared, x0);
+  if (rc) return rc;
+  rc = ascent_check(ctx, e_A, e_B, norm_type, max_iter, tol);
+  if (rc || S == 0) return rc;
+  cudaSetDevice(ctx->device);
+  WorstInfArgs a{};
+  a.S = S; a.dA = dA; a.dB = dB; a.x0_shared = x0_shared; a.x0 = x0; a.N = N; a.T_max = T_max;
+  a.eA = e_A; a.eB = e_B; a.norm = norm_type; a.max_iter = max_iter; a.tol = tol;
+  a.dA_out = dA_out; a.dB_out = dB_out; a.J = J_inf; a.T_cert = T_cert; a.rho = rho; a.iters = iters; a.flags = flags;
+  return lq_launch_worst_case_inf(ctx, a);
 }
 
 int lqmpc_bounds_fields(void) { return (int)lq::BF_COUNT; }

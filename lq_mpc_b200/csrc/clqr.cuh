@@ -436,6 +436,15 @@ LQ_HD_NOINLINE_T bool clqr_backward_call(const Problem<n, m>& pb, const Plan<n, 
   return clqr_backward<n, m>(pb, pl, N, fixed, athi, ws, rf, klast, koff);
 }
 
+// Final working set of a solve that needed the active-set iterations (clqr_solve's optional output, written only when
+// the iterations converge): the clamped inputs, the bound each sits at, and klast, the last stage whose affine law
+// (ws.Kc / ws.kc; the rows of clamped inputs are zero in Kc) the final sweep stored. Beyond klast the law is the
+// unconstrained ws.Ku with zero offset.
+struct ClqrActiveSet {
+  Mask128 fixed, athi;
+  int klast;
+};
+
 // Exact constrained solve from state x0. Returns flags; writes u0[m] and V (= optimum + x0'Qx0).
 // Pass structure (every pass is a sequential N-stage chain on strided scratch, so passes are what the solve costs):
 //   one clipped rollout of the unconstrained law (feasible => optimal, done) doubles as the feasible start;
@@ -446,7 +455,7 @@ LQ_HD_NOINLINE_T bool clqr_backward_call(const Problem<n, m>& pb, const Plan<n, 
 // k + koff; which working sets restart from a stored S is decided by the stored-stage count of horizon N itself.
 template <int n, int m>
 LQ_HD int clqr_solve(const Problem<n, m>& pb, const Plan<n, m>& pl, int N, const double* x0, const WsView& ws,
-                     double* u0, double* V, const Refs& rf = Refs(), int koff = 0) {
+                     double* u0, double* V, const Refs& rf = Refs(), int koff = 0, ClqrActiveSet* aset = nullptr) {
   const ClqrLayout<n, m> L(N + koff);
   const int kp = (N < kStoredCostToGo) ? N : kStoredCostToGo;   // == ClqrLayout(N).kp
   const int64_t oKu = L.oKu + (int64_t)koff * (m * n);
@@ -539,11 +548,13 @@ LQ_HD int clqr_solve(const Problem<n, m>& pb, const Plan<n, m>& pl, int N, const
   const int maxit = 8 * N * m + 32;
   bool done = false;
   double cost = 0.0;
+  int klast_swept = -1;
   for (int it = 0; it < maxit && !done; ++it) {
     // regulation: stages beyond the last clamped one keep the unconstrained law — the sweep covers 0..klast only
     const int top = fixed.top_bit();
     int klast = trk ? N - 1 : (top < 0 ? -1 : top / m);
     if (klast + 1 >= kp) klast = N - 1;                    // S_{klast+1} is not stored that far out: full sweep
+    klast_swept = klast;
     if (!((n <= 4) ? clqr_backward<n, m>(pb, pl, N, fixed, athi, ws, rf, klast, koff)
                    : clqr_backward_call<n, m>(pb, pl, N, fixed, athi, ws, rf, klast, koff)))
       flags |= FLAG_CHOL_FAIL;
@@ -666,6 +677,7 @@ LQ_HD int clqr_solve(const Problem<n, m>& pb, const Plan<n, m>& pl, int N, const
   if (done) {                                              // `cost` is the objective of the last candidate = z
     LQ_UNROLL for (int j = 0; j < m; ++j) u0[j] = ws[oz + j];
     *V = cost;
+    if (aset) { aset->fixed = fixed; aset->athi = athi; aset->klast = klast_swept; }
     return flags;
   }
   flags |= FLAG_QP_MAXITER;

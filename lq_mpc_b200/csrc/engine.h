@@ -152,6 +152,29 @@ struct WorstArgs {
   double* ws = nullptr;         // filled by the launcher
 };
 
+// lqmpc_simulate_inf_grad_batch / lqmpc_worst_case_inf_batch (k_worst_inf.cu): the input-constrained closed loop's
+// J_inf (box, regulation). SoA operands [elements][S]; any output may be NULL
+struct WorstInfArgs {
+  int64_t S;
+  const double* dA;         // [n*n][S]
+  const double* dB;         // [n*m][S]
+  const double* x0_shared;  // [n] or NULL -> x0 [n][S]
+  const double* x0;
+  int N, T_max;
+  double eA = 0.0, eB = 0.0, tol = 0.0;   // ascent only
+  int norm = 0, max_iter = 0;
+  double* J = nullptr;          // [S]
+  int32_t* T_cert = nullptr;
+  double* rho = nullptr;
+  int32_t* flags = nullptr;
+  double* gA = nullptr;         // gradient pass: [n*n][S], [n*m][S]
+  double* gB = nullptr;
+  double* dA_out = nullptr;     // ascent: the final perturbation (may alias dA / dB)
+  double* dB_out = nullptr;
+  int32_t* iters = nullptr;     // ascent: accepted steps [S]
+  double* ws = nullptr;         // filled by the launcher
+};
+
 struct TiledEval {
   int64_t S;
   const double* dA;   // [S][n*n] array of matrices
@@ -184,12 +207,16 @@ int lq_launch_mpc_poly(lqmpc_ctx* ctx, const MpcArgs& a, bool simulate);
 int lq_launch_mpc_range(lqmpc_ctx* ctx, const MpcArgs& a);
 int lq_launch_simulate_inf(lqmpc_ctx* ctx, const MpcArgs& a);
 int lq_launch_simulate_inf_poly(lqmpc_ctx* ctx, const MpcArgs& a);
+// grid of the worst-case launches: one sample per thread, capped at one wave of resident CTAs (LQMPC_WORST_CTAS: lower)
+int64_t lq_worst_blocks(lqmpc_ctx* ctx, const void* kernel, int threads, int64_t S);
 int lq_launch_eval_grad(lqmpc_ctx* ctx, const WorstArgs& a);
 int lq_launch_worst_case(lqmpc_ctx* ctx, const WorstArgs& a);
 // sup over x0 (lqmpc_ratio_sup_batch / lqmpc_worst_case_sup_batch): a.x0 is not read, a.J receives gamma; x_worst
 // [n][S] and gap [S] may be NULL
 int lq_launch_ratio_sup(lqmpc_ctx* ctx, const WorstArgs& a, double* x_worst, double* gap);
 int lq_launch_worst_case_sup(lqmpc_ctx* ctx, const WorstArgs& a, double* x_worst);
+int lq_launch_simulate_inf_grad(lqmpc_ctx* ctx, const WorstInfArgs& a);
+int lq_launch_worst_case_inf(lqmpc_ctx* ctx, const WorstInfArgs& a);
 int lq_launch_bounds(lqmpc_ctx* ctx, const BoundsArgs& a);
 bool lq_bounds_range_fused(lqmpc_ctx* ctx, const BoundsArgs& a);
 int lq_launch_bounds_range(lqmpc_ctx* ctx, const BoundsArgs& a);

@@ -138,27 +138,12 @@ __global__ void __launch_bounds__(128) worst_case_sup_kernel(const __grid_consta
   }
 }
 
-// Grid of every worst-case launch: one sample per thread, capped at one wave of resident CTAs of `kernel`.
-int64_t worst_blocks(lqmpc_ctx* ctx, const void* kernel, int threads, int64_t S) {
-  int sms = 148;
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, ctx->device);
-  int occ = 0;
-  cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kernel, threads, 0);
-  if (occ < 1) occ = 1;
-  int64_t cap = (int64_t)sms * occ;
-  // LQMPC_WORST_CTAS: a smaller grid cap, so that tests can run several samples per thread at small batch sizes
-  if (const char* v = getenv("LQMPC_WORST_CTAS")) { if (atoi(v) > 0 && atoi(v) < cap) cap = atoi(v); }
-  int64_t blocks = (S + threads - 1) / threads;
-  if (blocks > cap) blocks = cap;
-  return blocks;
-}
-
 template <int n, int m, bool ASCENT>
 int launch_worst_t(lqmpc_ctx* ctx, WorstArgs a) {
   const lq::Problem<n, m>& pb = *reinterpret_cast<const lq::Problem<n, m>*>(ctx->pb);
   const int threads = 128;
-  const int64_t blocks = ASCENT ? worst_blocks(ctx, (const void*)worst_case_kernel<n, m>, threads, a.S)
-                                : worst_blocks(ctx, (const void*)eval_grad_kernel<n, m>, threads, a.S);
+  const int64_t blocks = ASCENT ? lq_worst_blocks(ctx, (const void*)worst_case_kernel<n, m>, threads, a.S)
+                                : lq_worst_blocks(ctx, (const void*)eval_grad_kernel<n, m>, threads, a.S);
   const int64_t nthreads = blocks * threads;
   const int64_t per = lq::worst_ws_doubles<n, m>(a.N);
   int rc = lq_reserve_ws(ctx, (size_t)(per * nthreads) * sizeof(double) + 64);
@@ -177,7 +162,7 @@ int launch_sup_t(lqmpc_ctx* ctx, WorstArgs a, double* x_worst, double* gap) {
   const lq::Problem<n, m>& pb = *reinterpret_cast<const lq::Problem<n, m>*>(ctx->pb);
   const int threads = 128;
   const auto kernel = ASCENT ? worst_case_sup_kernel<n, m> : ratio_sup_kernel<n, m>;
-  const int64_t blocks = worst_blocks(ctx, (const void*)kernel, threads, a.S);
+  const int64_t blocks = lq_worst_blocks(ctx, (const void*)kernel, threads, a.S);
   a.ws = nullptr;
   if (ASCENT || a.gA || a.gB) {
     const int64_t per = lq::worst_ws_doubles<n, m>(a.N);
@@ -191,6 +176,21 @@ int launch_sup_t(lqmpc_ctx* ctx, WorstArgs a, double* x_worst, double* gap) {
 }
 
 }  // namespace
+
+// Grid of every worst-case launch: one sample per thread, capped at one wave of resident CTAs of `kernel`.
+int64_t lq_worst_blocks(lqmpc_ctx* ctx, const void* kernel, int threads, int64_t S) {
+  int sms = 148;
+  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, ctx->device);
+  int occ = 0;
+  cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kernel, threads, 0);
+  if (occ < 1) occ = 1;
+  int64_t cap = (int64_t)sms * occ;
+  // LQMPC_WORST_CTAS: a smaller grid cap, so that tests can run several samples per thread at small batch sizes
+  if (const char* v = getenv("LQMPC_WORST_CTAS")) { if (atoi(v) > 0 && atoi(v) < cap) cap = atoi(v); }
+  int64_t blocks = (S + threads - 1) / threads;
+  if (blocks > cap) blocks = cap;
+  return blocks;
+}
 
 int lq_launch_eval_grad(lqmpc_ctx* ctx, const WorstArgs& a) {
 #define X(N_, M_) \

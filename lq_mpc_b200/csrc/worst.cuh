@@ -412,4 +412,177 @@ LQ_HD int worst_ascent(const Problem<n, m>& pb, double* dA, double* dB, const do
   return flags;
 }
 
+// ---- the same steps as shared functions, for the objectives of other headers (worst_inf.cuh). worst_eval and
+// worst_ascent above keep their own inline copies: routing them through these functions changes the generated code
+// of 21 of the 44 kernels of k_worst.cu (same operations, different register allocation and spills).
+
+// worst_eval's forward recursion on (Ah, Bh) from P = P(0) (set by the caller): K0 = K(N), P left at P(N-1) and st
+// holding the factor of G_N. With `grad` the pairs (P(k-1), K(k)), k = 1..N-1, go to ws. Returns CHOL_FAIL of any stage.
+template <int n, int m>
+LQ_HD int riccati_records(const Problem<n, m>& pb, const double* Ah, const double* Bh, int N, const WsView& ws,
+                          bool grad, double* P, RicStage<n, m>& st, double* K0) {
+  constexpr int ps = n * (n + 1) / 2, rs = ps + m * n;
+  int flags = 0;
+  for (int k = 1; k < N; ++k) {
+    riccati_factor<n, m>(P, Bh, pb.R, st);
+    if (!st.ok) flags |= FLAG_CHOL_FAIL;
+    if (grad) {
+      const int64_t o = (int64_t)(k - 1) * rs;
+      int e = 0;
+      LQ_UNROLL for (int i = 0; i < n; ++i)
+        LQ_UNROLL for (int j = i; j < n; ++j) ws[o + e++] = P[i * n + j];
+      riccati_gain<n, m>(st, Ah, K0);
+      LQ_UNROLL for (int i = 0; i < m * n; ++i) ws[o + ps + i] = K0[i];
+    }
+    riccati_update<n, m>(st, Ah, pb.Q, P);
+  }
+  riccati_factor<n, m>(P, Bh, pb.R, st);        // horizon N: P = P(N-1), st holds G_N = L L'
+  if (!st.ok) flags |= FLAG_CHOL_FAIL;
+  riccati_gain<n, m>(st, Ah, K0);
+  return flags;
+}
+
+// worst_eval's reverse sweep: from Kbar = dJ/dK0 (in Z, overwritten) to gA = dJ/d(dA), gB = dJ/d(dB) (written), with
+// K0, P = P(N-1) and the factor st of riccati_records and its stage records in ws.
+template <int n, int m>
+LQ_HD void riccati_adjoint(const double* Ah, const double* Bh, const double* K0, const double* P,
+                           const RicStage<n, m>& st, double* Z, int N, const WsView& ws, double* gA, double* gB) {
+  constexpr int ps = n * (n + 1) / 2, rs = ps + m * n;
+  solve_l_inv<m, n>(st.L, st.Li, Z);
+  solve_lt_inv<m, n>(st.L, st.Li, Z);
+  double F[n * n], PB[n * m], Pbar[n * n];
+  LQ_UNROLL for (int i = 0; i < n; ++i)
+    LQ_UNROLL for (int j = 0; j < n; ++j) {
+      double acc = Ah[i * n + j];
+      LQ_UNROLL for (int k = 0; k < m; ++k) acc = fma(Bh[i * m + k], K0[k * n + j], acc);
+      F[i * n + j] = acc;
+    }
+  mm<n, n, m>(P, Bh, PB);
+  {
+    double T[n * n], ZK[m * m], U[n * m];
+    mm<n, m, n>(PB, Z, T);
+    LQ_UNROLL for (int i = 0; i < n * n; ++i) gA[i] = -T[i];
+    mm<n, n, n>(P, F, T);                        // P F
+    mmt<n, n, m>(T, Z, U);                       // P F Z'
+    mmt<m, n, m>(Z, K0, ZK);                     // Z K0'
+    LQ_UNROLL for (int i = 0; i < n; ++i)
+      LQ_UNROLL for (int j = 0; j < m; ++j) {
+        double acc = U[i * m + j];
+        LQ_UNROLL for (int k = 0; k < m; ++k) acc = fma(PB[i * m + k], ZK[k * m + j], acc);
+        gB[i * m + j] = -acc;
+      }
+    mmt<n, n, m>(F, Z, U);                       // U = F Z'
+    LQ_UNROLL for (int i = 0; i < n; ++i)
+      LQ_UNROLL for (int j = i; j < n; ++j) {
+        double acc = 0.0;
+        LQ_UNROLL for (int k = 0; k < m; ++k) acc = fma(U[i * m + k], Bh[j * m + k], fma(Bh[i * m + k], U[j * m + k], acc));
+        Pbar[i * n + j] = Pbar[j * n + i] = -0.5 * acc;
+      }
+  }
+  for (int k = N - 1; k >= 1; --k) {
+    const int64_t o = (int64_t)(k - 1) * rs;
+    double Pk[n * n], Kk[m * n], Fk[n * n], T[n * n], X[n * n];
+    int e = 0;
+    LQ_UNROLL for (int i = 0; i < n; ++i)
+      LQ_UNROLL for (int j = i; j < n; ++j) { const double v = ws[o + e++]; Pk[i * n + j] = v; Pk[j * n + i] = v; }
+    LQ_UNROLL for (int i = 0; i < m * n; ++i) Kk[i] = ws[o + ps + i];
+    LQ_UNROLL for (int i = 0; i < n; ++i)
+      LQ_UNROLL for (int j = 0; j < n; ++j) {
+        double acc = Ah[i * n + j];
+        LQ_UNROLL for (int l = 0; l < m; ++l) acc = fma(Bh[i * m + l], Kk[l * n + j], acc);
+        Fk[i * n + j] = acc;
+      }
+    mm<n, n, n>(Pk, Fk, T);
+    mm<n, n, n>(T, Pbar, X);
+    LQ_UNROLL for (int i = 0; i < n * n; ++i) gA[i] = fma(2.0, X[i], gA[i]);
+    LQ_UNROLL for (int i = 0; i < n; ++i)
+      LQ_UNROLL for (int j = 0; j < m; ++j) {
+        double acc = 0.0;
+        LQ_UNROLL for (int l = 0; l < n; ++l) acc = fma(X[i * n + l], Kk[j * n + l], acc);
+        gB[i * m + j] = fma(2.0, acc, gB[i * m + j]);
+      }
+    mm<n, n, n>(Fk, Pbar, T);
+    LQ_UNROLL for (int i = 0; i < n; ++i)
+      LQ_UNROLL for (int j = i; j < n; ++j) {
+        double acc = 0.0;
+        LQ_UNROLL for (int l = 0; l < n; ++l) acc = fma(T[i * n + l], Fk[j * n + l], acc);
+        Pbar[i * n + j] = Pbar[j * n + i] = acc;
+      }
+  }
+}
+
+// worst_ascent for any objective: the projected ascent over the error set from (dA, dB), both overwritten with the
+// result, in the normalised coordinates u = (dA / e_A, dB / e_B) with gradient g^ = (e_A dJ/d(dA), e_B dJ/d(dB)):
+//   * project the start; at every accepted point the stationarity residual is r = ||Proj(u + g^/||g^||) - u||_2
+//     (0 when g^ = 0) and the ascent stops when r <= tol;
+//   * trial u+ = Proj(u + t g^), the first t = 0.5 / ||g^||, then Barzilai-Borwein t = s's / (-s'y) when s'y < 0 and
+//     10 t otherwise; accepted when J(u+) >= J(u) + 1e-4 g^.(u+ - u), else t <- t / 4;
+//   * trials take the value only, the gradient is computed at accepted points;
+//   * an unstable trial lies in the set and destabilises the loop: it is the result (J = +inf, UNSTABLE);
+//   * a trial with a flag of kFail is rejected; a start with one ends the ascent there;
+//   * the budget of max_iter accepted steps (or a line search that shrinks t by 4^60) ends it with ASCENT_MAXITER.
+// The objective is `eval(dA, dB, &J, &rho, gA, gB)` -> flags, a trial when gA is null; `keep_trial()` is called when
+// an unstable trial becomes the result, so that the objective can keep that trial's other outputs. Returns the flags of
+// the final point; J, rho and the accepted-step count go to the outputs.
+template <int n, int m, int kFail, class Eval, class KeepTrial>
+LQ_HD int ascent_run(double* dA, double* dB, const AscentSettings& as, Eval eval, KeepTrial keep_trial,
+                     double* J_out, double* rho_out, int* iters) {
+  const double eA2 = as.eA * as.eA, eB2 = as.eB * as.eB;
+  worst_project<n, n>(dA, as.eA, as.norm);
+  worst_project<n, m>(dB, as.eB, as.norm);
+  double gA[n * n], gB[n * m], J, rho;
+  int flags = eval(dA, dB, &J, &rho, gA, gB);
+  int it = 0;
+  double t = 0.0;
+  while (!(flags & (kFail | FLAG_UNSTABLE))) {
+    const double gn2 = eA2 * fro2<n * n>(gA) + eB2 * fro2<n * m>(gB);
+    if (!(gn2 > 0.0)) break;                              // g^ = 0: r = 0
+    const double gn = sqrt(gn2);
+    double tA[n * n], tB[n * m];
+    const double r2 = worst_step<n, n>(dA, gA, eA2 / gn, as.eA, as.norm, tA) +
+                      worst_step<n, m>(dB, gB, eB2 / gn, as.eB, as.norm, tB);
+    if (sqrt(r2) <= as.tol) break;
+    if (it >= as.max_iter) { flags |= FLAG_ASCENT_MAXITER; break; }
+    if (it == 0) t = 0.5 / gn;
+    double Jt = 0.0, rt = 0.0, ss = 0.0;
+    int ft = 0;
+    bool accepted = false;
+    for (int bt = 0; bt < kWorstMaxBacktrack; ++bt) {
+      ss = worst_step<n, n>(dA, gA, t * eA2, as.eA, as.norm, tA) + worst_step<n, m>(dB, gB, t * eB2, as.eB, as.norm, tB);
+      double dot = 0.0;
+      LQ_UNROLL for (int i = 0; i < n * n; ++i) dot = fma(gA[i], tA[i] - dA[i], dot);
+      LQ_UNROLL for (int i = 0; i < n * m; ++i) dot = fma(gB[i], tB[i] - dB[i], dot);
+      ft = eval(tA, tB, &Jt, &rt, nullptr, nullptr);
+      if ((ft & FLAG_UNSTABLE) || (!(ft & kFail) && Jt >= J + 1e-4 * dmax(dot, 0.0))) { accepted = true; break; }
+      t *= 0.25;
+    }
+    if (!accepted) { flags |= FLAG_ASCENT_MAXITER; break; }
+    ++it;
+    if (ft & FLAG_UNSTABLE) {
+      LQ_UNROLL for (int i = 0; i < n * n; ++i) dA[i] = tA[i];
+      LQ_UNROLL for (int i = 0; i < n * m; ++i) dB[i] = tB[i];
+      keep_trial();
+      J = Jt; rho = rt; flags = ft;
+      break;
+    }
+    // the gradient at the accepted point (its value repeats the trial's bit for bit). With s = u+ - u and
+    // y = g^+ - g^, s'y = (dA+ - dA).(gA+ - gA) + (dB+ - dB).(gB+ - gB): the scales e cancel.
+    double nA[n * n], nB[n * m], sy = 0.0;
+    flags = eval(tA, tB, &J, &rho, nA, nB);
+    LQ_UNROLL for (int i = 0; i < n * n; ++i) {
+      sy = fma(tA[i] - dA[i], nA[i] - gA[i], sy);
+      dA[i] = tA[i]; gA[i] = nA[i];
+    }
+    LQ_UNROLL for (int i = 0; i < n * m; ++i) {
+      sy = fma(tB[i] - dB[i], nB[i] - gB[i], sy);
+      dB[i] = tB[i]; gB[i] = nB[i];
+    }
+    t = (sy < 0.0) ? ss / -sy : 10.0 * t;
+  }
+  *J_out = J;
+  *rho_out = rho;
+  *iters = it;
+  return flags;
+}
+
 }  // namespace lq

@@ -66,6 +66,9 @@ ABI = {
     "lqmpc_ratio_sup_batch": (_int, [_vp, _i64, _vp, _vp, _int] + [_vp] * 7),
     "lqmpc_worst_case_sup_batch": (_int, [_vp, _i64, _vp, _vp, _int, ctypes.c_double, ctypes.c_double, _int, _int,
                                           ctypes.c_double] + [_vp] * 7),
+    "lqmpc_simulate_inf_grad_batch": (_int, [_vp, _i64, _vp, _vp, _int, _int] + [_vp] * 8),
+    "lqmpc_worst_case_inf_batch": (_int, [_vp, _i64, _vp, _vp, _int, _int, _vp, _vp, ctypes.c_double, ctypes.c_double,
+                                          _int, _int, ctypes.c_double] + [_vp] * 7),
     "lqmpc_bounds_fields": (_int, []),
     "lqmpc_bounds_batch": (_int, [_vp, _i64, _vp, _vp, _int, _vp, _vp, ctypes.c_double, ctypes.c_double, _vp,
                                   ctypes.c_double, _vp, _vp, _vp, _vp, _vp, ctypes.c_double, ctypes.c_double,
@@ -656,6 +659,65 @@ class Engine:
                                                  _ptr(out["dB"]), _ptr(out["gamma"]), _ptr(out["x_worst"]),
                                                  _ptr(out["rho"]), _ptr(out["iters"]), _ptr(out["flags"]))
         self._check(rc, "lqmpc_worst_case_sup_batch")
+        return out
+
+    def _inf_operands(self, dA, dB, x0_shared, x0):
+        n = self.n
+        dA, dB, _, S = self._worst_operands(dA, dB)
+        if (x0_shared is None) == (x0 is None):
+            raise ValueError("give exactly one of x0_shared / x0")
+        xs = None if x0_shared is None else self._dev(x0_shared).reshape(n)
+        x0 = None if x0 is None else self._dev(x0)
+        if x0 is not None and x0.numel() != n * S:
+            raise ValueError("operand shapes do not match (n, m, S)")
+        return dA, dB, xs, x0, S
+
+    @_streamed
+    def simulate_inf_grad_batch(self, dA, dB, N: int, T_max: int = 1000, x0_shared=None, x0=None, grad: bool = True):
+        """J_inf of the input-constrained closed loop (as simulate_inf_batch) and its exact gradient in the model error
+        (lqmpc_simulate_inf_grad_batch). dA [n*n][S], dB [n*m][S]; x0_shared: (n,) one state for all samples, or x0:
+        [n][S]. Returns device tensors J_inf [S] (+inf: unstable, NaN: not certified within T_max steps), T_cert [S],
+        rho [S] = rho(A + B K0), flags [S] and, with grad, gA [n*n][S] = dJ_inf/d(dA), gB [n*m][S] = dJ_inf/d(dB)
+        (NaN where J_inf is not finite or a failure flag is set). Box only, regulation only."""
+        torch = self.torch
+        n, m = self.n, self.m
+        dA, dB, xs, x0, S = self._inf_operands(dA, dB, x0_shared, x0)
+        f64 = dict(dtype=torch.float64, device=self.device)
+        out = {"J_inf": torch.empty((S,), **f64), "T_cert": torch.empty((S,), dtype=torch.int32, device=self.device),
+               "rho": torch.empty((S,), **f64), "flags": torch.empty((S,), dtype=torch.int32, device=self.device)}
+        if grad:
+            out["gA"], out["gB"] = torch.empty((n * n, S), **f64), torch.empty((n * m, S), **f64)
+        rc = self.lib.lqmpc_simulate_inf_grad_batch(self._h, S, _ptr(dA), _ptr(dB), int(N), int(T_max), _ptr(xs),
+                                                    _ptr(x0), _ptr(out["J_inf"]), _ptr(out["T_cert"]),
+                                                    _ptr(out["rho"]), _ptr(out.get("gA")), _ptr(out.get("gB")),
+                                                    _ptr(out["flags"]))
+        self._check(rc, "lqmpc_simulate_inf_grad_batch")
+        return out
+
+    @_streamed
+    def worst_case_inf_batch(self, dA, dB, N: int, e_A: float, e_B: float, norm: str = "f", max_iter: int = 200,
+                             tol: float = 1e-8, T_max: int = 1000, x0_shared=None, x0=None):
+        """Projected ascent of the input-constrained closed loop's J_inf (simulate_inf_grad_batch) from every sample
+        over {||dA|| <= e_A, ||dB|| <= e_B} (lqmpc_worst_case_inf_batch), to a stationary point. Settings as
+        worst_case_batch, operands as simulate_inf_grad_batch. Returns device tensors dA [n*n][S], dB [n*m][S] (the
+        final perturbation), J_inf, T_cert, rho, iters [S] and flags [S] (FLAG_UNSTABLE: a destabilising error, J_inf =
+        +inf; FLAG_ASCENT_MAXITER: budget exhausted; a start with another failure flag is returned as it is)."""
+        torch = self.torch
+        n, m = self.n, self.m
+        if norm not in WORST_NORMS:
+            raise ValueError("norm must be one of %s" % sorted(WORST_NORMS))
+        dA, dB, xs, x0, S = self._inf_operands(dA, dB, x0_shared, x0)
+        f64 = dict(dtype=torch.float64, device=self.device)
+        i32 = dict(dtype=torch.int32, device=self.device)
+        out = {"dA": torch.empty((n * n, S), **f64), "dB": torch.empty((n * m, S), **f64),
+               "J_inf": torch.empty((S,), **f64), "T_cert": torch.empty((S,), **i32), "rho": torch.empty((S,), **f64),
+               "iters": torch.empty((S,), **i32), "flags": torch.empty((S,), **i32)}
+        rc = self.lib.lqmpc_worst_case_inf_batch(self._h, S, _ptr(dA), _ptr(dB), int(N), int(T_max), _ptr(xs),
+                                                 _ptr(x0), float(e_A), float(e_B), WORST_NORMS[norm], int(max_iter),
+                                                 float(tol), _ptr(out["dA"]), _ptr(out["dB"]), _ptr(out["J_inf"]),
+                                                 _ptr(out["T_cert"]), _ptr(out["rho"]), _ptr(out["iters"]),
+                                                 _ptr(out["flags"]))
+        self._check(rc, "lqmpc_worst_case_inf_batch")
         return out
 
     # ------------------------------------------------------------------------------------------------ K3
